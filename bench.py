@@ -6,7 +6,7 @@ face_landmarks_model_rcr_22.bin on 640x480 synthetic 8UC1 frames, batched, one f
 (config 3, "configs[2]").  A "step" = one pass of the detect cascade (4 levels: HOG -> feature x weight
 GEMM -> IED-scaled update) over one batch of B frames.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference] [--dump-outputs DIR]
 
   value        whole-job faces/s with frames + initial landmarks already resident in HBM
   e2e          the same through the reference-facing call detection_model::detect(image, facebox)
@@ -18,6 +18,10 @@ GEMM -> IED-scaled update) over one batch of B frames.
   train        (N=1 only, extra) regressor-train seconds of a reduced RCR training config
 
 --impl reference times the CPU path alone (rank 0), same metric/config.
+
+--dump-outputs DIR writes what the last timed step returned (rank 0's share) as DIR/<name>.npy in float32: the landmarks
+of the detect workload; the weights of every level and the final landmarks of the train workloads.  The inputs depend on
+the arguments only, so two builds run with the same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -51,6 +55,23 @@ def measured_peaks():
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_BYTES = 60 * 10 ** 6      # data of all dumped arrays; leaves room for the .npy headers under 64 MB
+
+
+def dump_outputs(dirname, arrays):
+    """Writes each array as dirname/<name>.npy in float32.  When together they exceed DUMP_BYTES, every array larger than an
+    even share of it is cut to a fixed, seeded sample of its rows (in row order, the same rows on every run)."""
+    os.makedirs(dirname, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    over = sum(a.nbytes for a in arrays.values()) > DUMP_BYTES
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        if over and a.nbytes > share:
+            keep = max(1, share // (a.nbytes // a.shape[0]))
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def synth_boxes(count, seed):
@@ -135,7 +156,6 @@ class ClockSampler:
 def cpu_detect_rate(n_faces, threads, seed):
     """Reference CPU path: oracle glue + the reference's hog.c when oracle/_ref is built."""
     from oracle import oracle as O
-    O.build()
     om = O.Model(MODEL)
     use_ref = O.ref_available()
     frames = synth_frames_numpy(min(n_faces, 64), seed)
@@ -273,9 +293,10 @@ def syrk_executed_flops(n, D, M, passes=3):
 
 
 def run_train(sd, ctx, model, world, rank, dev, barrier, max_over_ranks, comm, cfg=None, steps=1, warmup=1, e2e=False, distributed_solve=None,
-              solver="cholesky"):
+              solver="cholesky", outputs=None):
     """Regressor-train seconds (all S levels: HOG + targets + Gram + exchange + solve + update), strong scaling: the SAME global
-    training set for every number of ranks (samples are generated by global index)."""
+    training set for every number of ranks (samples are generated by global index).  A dict passed as outputs receives what
+    the last timed step returned: the weights of every level and this rank's final landmarks."""
     import torch
     from superviseddescent_b200 import parallel
     cfg = cfg or TRAIN_CFG
@@ -311,6 +332,9 @@ def run_train(sd, ctx, model, world, rank, dev, barrier, max_over_ranks, comm, c
     barrier()
     secs = max_over_ranks(e0.elapsed_time(e1)) * 1e-3 / steps
     launches = int(ctx.launches() - l0) // steps
+    if outputs is not None:
+        outputs.update({f"weights_level{i}": r.x.cpu().numpy() for i, r in enumerate(sdo.regressors)})
+        outputs["landmarks"] = xf.cpu().numpy()
     solver_ms = ctx.solver_timings()
     g = torch.from_numpy(x_gt).to(dev)
     num = torch.stack([torch.sum((torch.from_numpy(x0).to(dev) - g) ** 2), torch.sum((xf - g) ** 2), torch.sum(g ** 2)]).double()
@@ -392,7 +416,6 @@ def cpu_train_level_seconds(n_samples, threads, cfg=None):
     BASELINE.md section 3.  n_samples may be a bounded sample of the config's N; total_extrapolated_s scales the parts."""
     import scipy.linalg
     from oracle import oracle as O
-    O.build()
     cfg = cfg or TRAIN_CFG
     om = O.Model(MODEL)
     use_ref = O.ref_available()
@@ -452,11 +475,14 @@ def run_train_workload(args, sd, ctx, model, world, rank, local, dev, barrier, m
     if rank == 0:
         sampler.start()
     ds = {"auto": None, "replicated": False, "distributed": True, "cg": "cg"}[args.solve]
+    outputs = {} if args.dump_outputs else None
     line = run_train(sd, ctx, model, world, rank, dev, barrier, max_over_ranks, comm, cfg, steps=args.steps, warmup=args.warmup, e2e=True,
-                     distributed_solve=ds, solver="cg" if args.solve == "cg" else "cholesky")
+                     distributed_solve=ds, solver="cg" if args.solve == "cg" else "cholesky", outputs=outputs)
     clocks = sampler.stop() if rank == 0 else None
     if rank != 0:
         return
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     line["clocks"] = clocks
     if world == 1 and not args.no_cpu:
         try:
@@ -543,6 +569,8 @@ def run_ours(args):
     ms = max_over_ranks(e0.elapsed_time(e1))
     launches = ctx.launches() - l0
     value = world * B * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"landmarks": out.cpu().numpy()})
 
     # ---------------- end to end through the host-buffer call ----------------
     for _ in range(min(args.warmup, 2)):
@@ -671,11 +699,17 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-train", action="store_true", help="skip the extra regressor-train measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (float32, at most 64 MB; a seeded sample of rows when larger)")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = {"detect": 10, "train": 3, "train5": 1}[args.workload]
     if args.warmup is None:
         args.warmup = {"detect": 3, "train": 1, "train5": 1}[args.workload]
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

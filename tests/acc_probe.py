@@ -1,7 +1,8 @@
 """Accuracy probe (test infrastructure: it uses the CPU oracle): weights of a few systems vs float64 truth, per gram mode.
    python tests/acc_probe.py   on a GPU box"""
 import sys, os, numpy as np
-sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/tests")
+HERE = os.path.dirname(os.path.abspath(__file__))
+sys.path.insert(0, os.path.dirname(HERE)); sys.path.insert(0, HERE)
 from oracle import oracle as O
 from superviseddescent_b200 import api as sd
 ctx = sd.default_context()

@@ -15,6 +15,9 @@ Outputs (all small, committed):
   hog_ref.npz                       outputs of the reference's own hog.c (oracle/_ref) on seeded inputs
                                     (pins oracle.hog_core when /root/reference is absent, i.e. on the GPU box)
   detect_ref.npz                    oracle detect() on the example frames with hog.c as the HOG core
+  hog_live_ref.npz                  the reference's hog.c on the inputs of tests/test_oracle.py's comparisons with
+                                    oracle/_ref (seeded images through the HOG core, and one frame through the
+                                    fixed-patch transform), stored with those inputs
 """
 import os
 import shutil
@@ -104,8 +107,39 @@ def main():
         feats = O.hog_transform(ex[f"gray{i}"], O.align_mean(m.mean, BOXES[i]), m.hog_params[0], m.right_idx, m.left_idx, use_ref=True)
         dt[f"features_l0_{i}"] = feats
     np.savez_compressed(f"{HERE}/detect_ref.npz", **dt)
+    live_reference_goldens()
     for f in sorted(os.listdir(HERE)):
         print(f, os.path.getsize(os.path.join(HERE, f)))
+
+
+def live_reference_goldens():
+    """hog_live_ref.npz: the inputs are built exactly as test_hog_core_matches_live_reference and
+    test_fixed_patch_transform_equals_adaptive_one_at_matching_size build them."""
+    sys.path.insert(0, os.path.dirname(HERE))
+    import synth
+    O.build()
+    assert O.ref_available(), "oracle/_ref is not built"
+    g = {}
+    rng = np.random.default_rng(7)
+    n = 0
+    for K in (4, 9, 6):
+        for fs, cs in ((55, 11), (30, 6), (48, 8)):
+            img = rng.integers(0, 256, (fs, fs)).astype(np.float32)
+            g[f"core_img{n}"] = img.astype(np.uint8)
+            g[f"core_out{n}"] = O.hog_core(img, cs, K, 1, use_ref=True)
+            g[f"core_cfg{n}"] = np.array([K, cs], dtype=np.int32)
+            n += 1
+    img = synth.smooth_images(1, 120, 160, seed=3)[0]
+    nc, cs, K, L = 3, 12, 4, 6
+    rng = np.random.default_rng(2)
+    x = np.concatenate([rng.uniform(10, 150, L), rng.uniform(10, 110, L)]).astype(np.float32)
+    x[0], x[L] = 40.0, 60.0
+    x[1], x[L + 1] = 40.0 + nc * cs, 60.0
+    x[2], x[L + 2] = 2.0, 118.0
+    g["fixed_img"], g["fixed_x"] = img, x
+    for variant in (0, 1):
+        g[f"fixed_out{variant}"] = O.hog_transform_fixed(img, x, O.HogParam(variant, nc, cs, K, 1.0), use_ref=True)
+    np.savez_compressed(f"{HERE}/hog_live_ref.npz", **g)
 
 
 if __name__ == "__main__":

@@ -1,7 +1,7 @@
 """Pins the CPU oracle (oracle/sd_oracle.c) against the reference's own golden data (no GPU needed).
 
   - cv2 4.13 resize / BGR2GRAY outputs                      (tests/golden/resize_cv2.npz, examples.npz)
-  - the reference's hog.c outputs                            (tests/golden/hog_ref.npz, and live vs oracle/_ref when built)
+  - the reference's hog.c outputs                            (tests/golden/hog_ref.npz, hog_live_ref.npz, and live vs oracle/_ref when built)
   - the shipped model file + the 5 annotated example frames  (byte round-trip, landmark error)
   - every literal of the reference's gtest suite             (tests/known_answers.py)
 """
@@ -37,14 +37,17 @@ def test_hog_core_matches_reference_goldens_bit_exact(oracle, golden):
         assert np.array_equal(got.view(np.uint32), golden.hog[f"out{i}"].view(np.uint32)), f"case {i} K={K_} cs={cs} v={variant}"
 
 
-def test_hog_core_matches_live_reference(oracle):
-    if not oracle.ref_available():
-        pytest.skip("oracle/_ref not built (no /root/reference on this box)")
-    rng = np.random.default_rng(7)
-    for K_ in (4, 9, 6):
-        for fs, cs in ((55, 11), (30, 6), (48, 8)):
-            img = rng.integers(0, 256, (fs, fs)).astype(np.float32)
-            a = oracle.hog_core(img, cs, K_, 1)
+def test_hog_core_matches_live_reference(oracle, golden):
+    """Against the reference's hog.c outputs stored in hog_live_ref.npz, and against oracle/_ref itself where it is built."""
+    ref = np.load(os.path.join(golden.dir, "hog_live_ref.npz"))
+    n = len([k for k in ref.files if k.startswith("core_img")])
+    assert n == 9
+    for i in range(n):
+        K_, cs = [int(v) for v in ref[f"core_cfg{i}"]]
+        img = ref[f"core_img{i}"].astype(np.float32)
+        a = oracle.hog_core(img, cs, K_, 1)
+        assert np.array_equal(a.view(np.uint32), ref[f"core_out{i}"].view(np.uint32)), f"case {i} K={K_} cs={cs}"
+        if oracle.ref_available():
             b = oracle.hog_core(img, cs, K_, 1, use_ref=True)
             assert np.array_equal(a.view(np.uint32), b.view(np.uint32))
 
@@ -252,7 +255,7 @@ def test_pose_estimation_example_config2(oracle):
     assert np.all(np.abs(pred[:3] - np.array([11.0, -25.0, -10.0])) < 6.0)      # example's ground truth (:334)
 
 
-def test_fixed_patch_transform_equals_adaptive_one_at_matching_size(oracle):
+def test_fixed_patch_transform_equals_adaptive_one_at_matching_size(oracle, golden):
     """examples/landmark_detection.cpp:195-261 (fixed patch, no resize, no bias) against adaptive_vlhog.hpp:109-185: when
     the inter-eye distance makes the adaptive patch exactly num_cells * cell_size wide, cv::resize is the identity and the
     two functors must agree value for value (the adaptive one appends its bias)."""
@@ -265,12 +268,14 @@ def test_fixed_patch_transform_equals_adaptive_one_at_matching_size(oracle):
     x[0], x[L] = 40.0, 60.0                       # right eye
     x[1], x[L + 1] = 40.0 + nc * cs, 60.0         # left eye: IED = 36 -> half = round(1.0 * 36 / 2) = 18 = nc * (cs / 2)
     x[2], x[L + 2] = 2.0, 118.0                   # near a corner: zero padding on two sides
+    ref = np.load(os.path.join(golden.dir, "hog_live_ref.npz"))   # the same frame and landmarks through the reference's hog.c
     for variant in (0, 1):
         hp = oracle.HogParam(variant, nc, cs, K, 1.0)
         adaptive = oracle.hog_transform(img, x, hp, [0], [1])
         fixed = oracle.hog_transform_fixed(img, x, hp)
         assert fixed.size == adaptive.size - 1 and adaptive[-1] == 1.0
         assert np.array_equal(fixed, adaptive[:-1])
+        assert np.array_equal(oracle.hog_transform_fixed(ref["fixed_img"], ref["fixed_x"], hp), ref[f"fixed_out{variant}"])
         if oracle.ref_available():
             assert np.array_equal(oracle.hog_transform_fixed(img, x, hp, use_ref=True), fixed)
 

@@ -1,6 +1,6 @@
 """Probes variants of the host-frame route of sd_detect_batch_host.  Development helper, not part of the product."""
 import os, sys, time, numpy as np, torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench
 from superviseddescent_b200 import api as sd
 ctx = sd.Context(0)

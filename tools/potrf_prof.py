@@ -1,9 +1,10 @@
 """Prints the clock64 phase timings of potrf_inv_kernel from the instrumented library (tools/build_prof.sh).
 Development helper, not part of the product."""
 import ctypes as C, os, sys, numpy as np, torch
-sys.path.insert(0, "/root/repo")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 from superviseddescent_b200 import _capi
-_capi.LIB_PATH = "/root/repo/superviseddescent_b200/lib_prof/libsd_b200.so"
+_capi.LIB_PATH = os.path.join(ROOT, "superviseddescent_b200", "lib_prof", "libsd_b200.so")
 from superviseddescent_b200 import api as sd
 rng = np.random.default_rng(0)
 n, d = 2000, 1500

@@ -1,7 +1,6 @@
 // Context, error handling and memory helpers of libsd_b200.so (C ABI: include/sd_b200.h).
 #include "sd_internal.cuh"
 
-#include <cstdlib>
 #include <cstring>
 
 int sd_fail(sd_ctx* ctx, int code, const char* fmt, ...)
@@ -127,10 +126,6 @@ int sd_ctx_create(int device, void* stream, sd_ctx** out)
     ok = ok && cudaMallocHost(&ctx->h_scratch, 4096) == cudaSuccess && cudaMalloc(&ctx->d_scratch, 4096) == cudaSuccess &&
          cudaMemset(ctx->d_scratch, 0, 4096) == cudaSuccess;
     if (!ok) { sd_ctx_destroy(ctx); return SD_ERR_CUDA; }
-    { const char* e = getenv("SD_B200_NO_ROI"); ctx->disable_roi = e && e[0] == '1'; }
-    { const char* e = getenv("SD_B200_HOST_ROUTE"); if (e) ctx->host_route = (e[0] == 'p') ? 1 : 0; }
-    { const char* e = getenv("SD_B200_PACK_THREADS"); if (e && atoi(e) >= 1 && atoi(e) <= 64) ctx->pack_threads = atoi(e); }
-    { const char* e = getenv("SD_B200_SOLVER"); if (e && e[0] == 'c' && e[1] == 'g') ctx->solver_mode = 1; }
     *out = ctx;
     return SD_OK;
 }
@@ -150,8 +145,6 @@ void sd_ctx_destroy(sd_ctx* ctx)
     }
     for (int i = 0; i < 6; ++i) if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
     for (int i = 0; i < 8; ++i) if (ctx->cg_ev[i]) cudaEventDestroy(ctx->cg_ev[i]);
-    if (ctx->pack_pool) sd_pack_pool_destroy(ctx->pack_pool);
-    for (int i = 0; i < 2; ++i) if (ctx->h_stage[i]) cudaFreeHost(ctx->h_stage[i]);
     if (ctx->h_scratch) cudaFreeHost(ctx->h_scratch);
     if (ctx->d_scratch) cudaFree(ctx->d_scratch);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
@@ -270,7 +263,6 @@ int sd_solver_timings(sd_ctx* ctx, float ms_out[4])
     for (int i = 0; i < 4; ++i) {
         float ms = 0.f;
         if (cudaEventElapsedTime(&ms, ctx->ev[i], ctx->ev[i + 1]) != cudaSuccess) { ms = 0.f; cudaGetLastError(); }
-        ctx->timings[i] = ms;
         ms_out[i] = ms;
     }
     return SD_OK;

@@ -16,7 +16,6 @@
 #include "sd_internal.cuh"
 
 #include <cmath>
-#include <cstdlib>
 
 namespace {
 
@@ -285,8 +284,8 @@ int sd_cg_solve(sd_ctx* ctx, sd_comm* comm, float* G, int64_t ldg, int n, int co
     cg_init_finish_kernel<<<1, 1024, 0, ctx->stream>>>(b, M);
     SD_LAUNCH_CHECK(ctx, "cg_init_finish_kernel");
 
-    static const float tol = getenv("SD_B200_CG_TOL") ? (float)atof(getenv("SD_B200_CG_TOL")) : 2e-6f;
-    static const int max_iter = getenv("SD_B200_CG_MAXIT") ? atoi(getenv("SD_B200_CG_MAXIT")) : 600;
+    constexpr float tol = 2e-6f;
+    constexpr int max_iter = 600;
     // The product is the same launch every iteration: Q[n x M] = S[k0:k1, :]^T P[k0:k1, :]  ( = S P summed over the ranks' slabs of
     // the contraction: S is symmetric ); prepared once (tensor maps, tile list).  S is the 128-row operand: n / 128 tiles keep the
     // SMs busy at any slab size, P is the narrow operand.  Pad columns of Q and the rows of a rank without slab stay zero.
@@ -305,7 +304,7 @@ int sd_cg_solve(sd_ctx* ctx, sd_comm* comm, float* G, int64_t ldg, int n, int co
     float* h_conv = reinterpret_cast<float*>(reinterpret_cast<char*>(ctx->h_scratch) + 2048);
     for (int i = 0; i < 8; ++i)
         if (!ctx->cg_ev[i]) SD_CUDA(ctx, cudaEventCreateWithFlags(&ctx->cg_ev[i], cudaEventDisableTiming));
-    int it = 0, prev_it = 0, done_at = -1;
+    int it = 0, prev_it = 0;
     float prev_conv = 0.f;
     bool converged = false, failed = false;
     for (; it < max_iter && !converged && !failed; ++it) {
@@ -338,7 +337,7 @@ int sd_cg_solve(sd_ctx* ctx, sd_comm* comm, float* G, int64_t ldg, int n, int co
             SD_CUDA(ctx, cudaEventSynchronize(ctx->cg_ev[look & 7]));
             const float cv = h_conv[2 * (look & 7)], bad = h_conv[2 * (look & 7) + 1];
             if (bad != 0.f || !(cv == cv)) { failed = true; break; }
-            if (cv <= tol) { converged = true; done_at = look + 1; }
+            if (cv <= tol) converged = true;
             else if (look >= 30 && prev_conv > 0.f && look > prev_it) {
                 // a system that would need more than max_iter iterations at the observed rate is the factorisation's job
                 const double rate = pow((double)cv / (double)prev_conv, 1.0 / (double)(look - prev_it));
@@ -356,7 +355,6 @@ int sd_cg_solve(sd_ctx* ctx, sd_comm* comm, float* G, int64_t ldg, int n, int co
             else if (cv <= tol) converged = true;
         }
     }
-    (void)done_at;
     if (iters) *iters = it;
     if (!converged) return SD_ERR_NUMERIC;
     *W_out = b.X;

@@ -617,7 +617,7 @@ int sd_gemm_tn_tc_prepare(sd_ctx* ctx, const float* d_SA, int64_t lda, const flo
     // C goes back through the TMA when it can be described by a tensor map (16-byte aligned base and pitch)
     plan->map_c = plan->map_b;
     a.tma_c = 0;
-    if ((beta == 0.f || beta == 1.f) && (ldc % 4) == 0 && (reinterpret_cast<uintptr_t>(d_C) & 15) == 0 && !getenv("SD_B200_NO_TMA_C")) {
+    if ((beta == 0.f || beta == 1.f) && (ldc % 4) == 0 && (reinterpret_cast<uintptr_t>(d_C) & 15) == 0) {
         rc = make_map_c(ctx, &plan->map_c, d_C, ldc, MI, NJ);
         if (rc) return rc;
         a.tma_c = beta == 1.f ? 2 : 1;
@@ -626,7 +626,7 @@ int sd_gemm_tn_tc_prepare(sd_ctx* ctx, const float* d_SA, int64_t lda, const flo
     SD_REQUIRE(ctx, a.ksplit == 1 || (a.tma_c == 2 && a.ksplit == 2), "split-K needs beta == 1, the TMA reduce-add write-back and two ranges");
     // a single tile column of at most 192 columns can run the narrow variants
     plan->nb = 8;
-    if (narrow && TJ == 1 && !getenv("SD_B200_NO_NARROW")) plan->nb = NJ <= 64 ? 2 : NJ <= 128 ? 4 : NJ <= 192 ? 6 : 8;
+    if (narrow && TJ == 1) plan->nb = NJ <= 64 ? 2 : NJ <= 128 ? 4 : NJ <= 192 ? 6 : 8;
     switch (plan->nb) {
     case 2: SD_CUDA(ctx, cudaFuncSetAttribute(syrk_tc2_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<2>::SMEM_BYTES)); break;
     case 4: SD_CUDA(ctx, cudaFuncSetAttribute(syrk_tc2_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<4>::SMEM_BYTES)); break;

@@ -735,7 +735,7 @@ int launch_hog(sd_ctx* ctx, const sd_image_batch* images, const int32_t* d_image
     memset(&maps, 0, sizeof(maps));
     a.tma_count = 0;
     if (!images->d_roi && !images->d_frames && (reinterpret_cast<uintptr_t>(images->d_data) & 15) == 0 && (images->row_stride % 16) == 0 &&
-        (images->image_stride % 16) == 0 && (images->count == 1 || images->image_stride > 0) && !getenv("SD_B200_HOG_NO_TMA")) {
+        (images->image_stride % 16) == 0 && (images->count == 1 || images->image_stride > 0)) {
         PFN_hogEncodeTiled enc = hog_encode_fn();
         if (enc) {
             bool ok = true;

@@ -44,9 +44,7 @@ struct sd_ctx {
     int solver_mode = 0;           // systems with D > 256: 0 = blocked Cholesky, 1 = conjugate gradients (Cholesky if they stall)
     int cg_iterations = 0;         // of the last solve (0: the factorisation ran)
     cudaEvent_t cg_ev[8] = {};     // convergence read-backs of the CG loop (the host runs a few iterations ahead of them)
-    bool disable_roi = false;      // sd_detect_batch_host: always upload whole frames
     int64_t roi_fallbacks = 0;     // faces repeated from the full frame because a patch left its ROI
-    float timings[4] = {0, 0, 0, 0};
     cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     void* hog_lut[SD_MAX_BINS + 1] = {};   // per K: (gx,gy) -> orientation bin table (sd_hog.cu)
     void* ws[SD_WS_COUNT] = {};
@@ -59,13 +57,7 @@ struct sd_ctx {
     size_t stage_bytes[2] = {0, 0};
     cudaEvent_t stage_ev[2] = {nullptr, nullptr};
     cudaEvent_t stage_done[2] = {nullptr, nullptr};
-    // "pack" staging route of sd_detect_batch_host: pinned buffers + host copy threads (sd_model.cu)
-    int host_route = 0;            // 0 = gather (zero-copy kernel), 1 = pack (host threads + one copy-engine transfer per chunk)
-    int pack_threads = 8;
-    void* h_stage[2] = {nullptr, nullptr};
-    struct sd_pack_pool* pack_pool = nullptr;
 };
-void sd_pack_pool_destroy(struct sd_pack_pool* p);
 
 int sd_fail(sd_ctx* ctx, int code, const char* fmt, ...);
 int sd_check_cuda(sd_ctx* ctx, cudaError_t e, const char* what);

@@ -322,8 +322,7 @@ int launch_gemm_nn(sd_ctx* ctx, const float* A, int64_t lda, int N, int D, const
     if (N <= 0 || M <= 0) return SD_OK;
     // the cascade's shape -- a long contraction, 2L output columns -- goes to the row-per-thread kernel for ANY number of rows: its
     // chunk boundaries are global multiples of 32, so a row's result does not depend on the batch it is computed in
-    if (D >= 1024 && M <= 4 * PR_COLS && (lda % 4) == 0 && (reinterpret_cast<uintptr_t>(A) & 15) == 0 &&
-        !getenv("SD_B200_OLD_PREDICT")) {
+    if (D >= 1024 && M <= 4 * PR_COLS && (lda % 4) == 0 && (reinterpret_cast<uintptr_t>(A) & 15) == 0) {
         const int row_blocks = sd_div_up(N, PR_ROWS), col_groups = sd_div_up(M, PR_COLS);
         int splits = (int)(2LL * ctx->sm_count / ((long long)row_blocks * col_groups));     // two CTAs' worth of work per SM, whole waves
         if (N < PR_ROWS) splits = splits * N / PR_ROWS + 1;                                 // few rows: few threads per CTA are live anyway
@@ -1227,8 +1226,7 @@ int launch_trsm_apply(sd_ctx* ctx, cudaStream_t stream, float* B, int64_t ldb, i
 
 bool sd_syrk_is_big(int K, int64_t MI, int64_t NJ)
 {
-    static const long long tc_min = getenv("SD_B200_TC_MIN") ? atoll(getenv("SD_B200_TC_MIN")) : 256LL * 256LL;
-    return MI * NJ >= tc_min && K >= 64;
+    return MI * NJ >= 256 * 256 && K >= 64;
 }
 
 // comm (optional, more than one rank): DISTRIBUTED factorisation.  Block-row-cyclic ownership in units of one 256-row panel
@@ -1258,8 +1256,7 @@ int cholesky_solve(sd_ctx* ctx, float* G, int64_t ldg, int D, int M, float* X, s
         SD_CUDA(ctx, cudaStreamCreateWithPriority(&ctx->chain_stream, cudaStreamNonBlocking, prio_hi));
         for (int i = 0; i < 2; ++i) SD_CUDA(ctx, cudaEventCreateWithFlags(&ctx->chain_ev[i], cudaEventDisableTiming));
     }
-    const bool lookahead = getenv("SD_B200_NO_LOOKAHEAD") == nullptr;      // debugging knob: run the chain in line
-    cudaStream_t main_s = ctx->stream, chain_s = lookahead ? ctx->chain_stream : ctx->stream;
+    cudaStream_t main_s = ctx->stream, chain_s = ctx->chain_stream;
     cudaEvent_t ev_head = ctx->chain_ev[0], ev_chain = ctx->chain_ev[1];
     GemmEpilogue ep;
     memset(&ep, 0, sizeof(ep));
@@ -1343,10 +1340,9 @@ int cholesky_solve(sd_ctx* ctx, float* G, int64_t ldg, int D, int M, float* X, s
         // one kernel family per rank-kp update, chosen from the size of the whole trailing matrix; the updates use the
         // unbiased hi/lo split: a truncated hi leaves a one-signed lo*lo term behind, which is harmless in the Gram (it
         // scales [AtA|Atb] almost uniformly) but is amplified by the cancellation inside Schur complements
-        static const bool upd_unbiased = getenv("SD_B200_UPDATE_BIASED") == nullptr;
         const int path = sd_syrk_is_big(kp, rest, cols3) ? 1 : 2;
         if (me == next_owner) {
-            rc = sd_syrk_update(ctx, row1, ldg, kp, head, cols3, C3, ldg, -1.0f, 1.0f, path, upd_unbiased);
+            rc = sd_syrk_update(ctx, row1, ldg, kp, head, cols3, C3, ldg, -1.0f, 1.0f, path, true);
             if (rc) return rc;
             SD_CUDA(ctx, cudaEventRecord(ev_head, main_s));
             SD_CUDA(ctx, cudaStreamWaitEvent(chain_s, ev_head, 0));
@@ -1357,9 +1353,9 @@ int cholesky_solve(sd_ctx* ctx, float* G, int64_t ldg, int D, int M, float* X, s
         if (rest > head) {
             sd_row_filter own;
             own.block = 2 * kCholNb; own.nranks = nranks; own.rank = me; own.first_row = j3 + head;
-            ctx->syrk_sm_reserve = (lookahead && me == next_owner) ? 1 : 0;   // leave one SM to the chain running beside it
+            ctx->syrk_sm_reserve = (me == next_owner) ? 1 : 0;   // leave one SM to the chain running beside it
             rc = sd_syrk_update(ctx, row1 + head, ldg, kp, rest - head, cols3 - head, C3 + (int64_t)head * ldg + head, ldg, -1.0f, 1.0f, path,
-                                upd_unbiased, dist ? &own : nullptr);
+                                true, dist ? &own : nullptr);
             ctx->syrk_sm_reserve = 0;
             if (rc) return rc;
         }

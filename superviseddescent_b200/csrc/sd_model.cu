@@ -10,12 +10,7 @@
 #include <cstring>
 #include <exception>
 #include <fstream>
-#include <atomic>
-#include <condition_variable>
-#include <functional>
-#include <mutex>
 #include <string>
-#include <thread>
 #include <vector>
 
 struct sd_model {
@@ -541,59 +536,6 @@ static int detect_host_full(sd_ctx* ctx, const sd_model* m, const uint8_t* h_ima
     return sd_check_hog_status(ctx, "detect");                // synchronises
 }
 
-// Host-side staging of the ROI route ("pack"): a few host threads copy the ROI rows of a chunk of faces into a contiguous
-// pinned buffer, which then crosses PCIe as ONE copy-engine transfer (copy engines move ~50 GB/s over Gen5 x16; the SMs'
-// zero-copy loads of the "gather" route are limited to ~20 GB/s by the outstanding-read budget of the link).  Pure data
-// movement: no arithmetic happens on the host.
-extern "C++" {
-struct sd_pack_pool {
-    std::vector<std::thread> workers;
-    std::mutex mu;
-    std::condition_variable cv_work, cv_done;
-    std::function<void(int)> fn;
-    int n_items = 0, generation = 0, pending = 0;
-    std::atomic<int> next{0};
-    bool stop = false;
-
-    explicit sd_pack_pool(int threads)
-    {
-        for (int t = 0; t < threads; ++t)
-            workers.emplace_back([this] {
-                int seen = 0;
-                for (;;) {
-                    std::unique_lock<std::mutex> lk(mu);
-                    cv_work.wait(lk, [&] { return stop || generation != seen; });
-                    if (stop) return;
-                    seen = generation;
-                    lk.unlock();
-                    for (int i = next.fetch_add(1); i < n_items; i = next.fetch_add(1)) fn(i);
-                    lk.lock();
-                    if (--pending == 0) cv_done.notify_all();
-                }
-            });
-    }
-    ~sd_pack_pool()
-    {
-        { std::lock_guard<std::mutex> lk(mu); stop = true; }
-        cv_work.notify_all();
-        for (auto& w : workers) w.join();
-    }
-    void run(int n, std::function<void(int)> f)
-    {
-        std::unique_lock<std::mutex> lk(mu);
-        fn = std::move(f);
-        n_items = n;
-        next = 0;
-        pending = (int)workers.size();
-        ++generation;
-        cv_work.notify_all();
-        cv_done.wait(lk, [&] { return pending == 0; });
-    }
-};
-
-void sd_pack_pool_destroy(sd_pack_pool* p) { delete p; }
-}  // extern "C++"
-
 // ROI route: needs the caller's frames in pinned (device-mapped) host memory
 static int detect_host_roi(sd_ctx* ctx, const sd_model* m, const uint8_t* h_images, const uint8_t* d_alias, int count, int width,
                            int height, int row_stride, const int32_t* h_boxes, float* h_landmarks)
@@ -625,13 +567,6 @@ static int detect_host_roi(sd_ctx* ctx, const sd_model* m, const uint8_t* h_imag
             ctx->stage_bytes[b] = chunk_cap + (1u << 20);
         }
     }
-    // staging route: "pack" (host threads + one DMA per chunk) or "gather" (zero-copy reads by a kernel)
-    const bool pack = ctx->host_route == 1;
-    if (pack) {
-        if (!ctx->pack_pool) ctx->pack_pool = new sd_pack_pool(ctx->pack_threads);
-        for (int b = 0; b < 2; ++b)
-            if (!ctx->h_stage[b]) SD_CUDA(ctx, cudaMallocHost(&ctx->h_stage[b], chunk_cap + (1u << 20)));
-    }
     // device tables: landmarks (in, out), ROI records, miss flags
     const size_t xbytes = (size_t)count * P * sizeof(float);
     const size_t rbytes = (size_t)count * sizeof(sd_roi);
@@ -650,25 +585,9 @@ static int detect_host_roi(sd_ctx* ctx, const sd_model* m, const uint8_t* h_imag
     for (size_t c = 0; c + 1 < chunk_first.size(); ++c, buf ^= 1) {
         const int first = chunk_first[c], n = chunk_first[c + 1] - first;
         SD_CUDA(ctx, cudaStreamWaitEvent(ctx->copy_stream, ctx->stage_done[buf], 0));   // also orders the table uploads before the first gather
-        if (pack) {
-            // host threads pack the chunk's ROI rows, one copy-engine transfer moves them
-            if (c >= 2) SD_CUDA(ctx, cudaEventSynchronize(ctx->stage_ev[buf]));       // the transfer that last read this pinned buffer
-            uint8_t* hs = (uint8_t*)ctx->h_stage[buf];
-            const sd_roi* rr = rois.data();
-            ctx->pack_pool->run(n, [=](int f) {
-                const sd_roi& r = rr[first + f];
-                const uint8_t* src = h_images + (size_t)(first + f) * frame_bytes + (size_t)r.y * row_stride + r.x;
-                uint8_t* dst = hs + r.offset;
-                for (int y = 0; y < r.h; ++y) memcpy(dst + (size_t)y * r.row_stride, src + (size_t)y * row_stride, (size_t)r.row_stride);
-            });
-            const sd_roi& last = rois[first + n - 1];
-            const size_t bytes = (size_t)last.offset + (size_t)last.row_stride * last.h;
-            SD_CUDA(ctx, cudaMemcpyAsync(ctx->d_stage[buf], hs, bytes, cudaMemcpyHostToDevice, ctx->copy_stream));
-        } else {
-            const int blocks = n < 8 * ctx->sm_count ? n : 8 * ctx->sm_count;
-            roi_gather_kernel<<<blocks, 256, 0, ctx->copy_stream>>>(d_alias, (long long)frame_bytes, row_stride, d_roi, first, n, (uint8_t*)ctx->d_stage[buf]);
-            SD_LAUNCH_CHECK(ctx, "roi_gather_kernel");
-        }
+        const int blocks = n < 8 * ctx->sm_count ? n : 8 * ctx->sm_count;
+        roi_gather_kernel<<<blocks, 256, 0, ctx->copy_stream>>>(d_alias, (long long)frame_bytes, row_stride, d_roi, first, n, (uint8_t*)ctx->d_stage[buf]);
+        SD_LAUNCH_CHECK(ctx, "roi_gather_kernel");
         SD_CUDA(ctx, cudaEventRecord(ctx->stage_ev[buf], ctx->copy_stream));
         SD_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->stage_ev[buf], 0));
         sd_image_batch ib{};
@@ -709,7 +628,7 @@ int sd_detect_batch_host(sd_ctx* ctx, const sd_model* m, const uint8_t* h_images
     const bool pinned = cudaPointerGetAttributes(&attr, h_images) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer;
     if (!pinned) cudaGetLastError();
     const bool aligned = pinned && ((reinterpret_cast<uintptr_t>(attr.devicePointer) | (uintptr_t)row_stride | (uintptr_t)frame_bytes) & 15) == 0;
-    if (aligned && !ctx->disable_roi)
+    if (aligned)
         return detect_host_roi(ctx, m, h_images, (const uint8_t*)attr.devicePointer, count, width, height, row_stride, h_boxes, h_landmarks);
     return detect_host_full(ctx, m, h_images, count, width, height, row_stride, h_boxes, h_landmarks);
 }

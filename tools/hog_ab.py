@@ -1,5 +1,5 @@
-"""Times the level-0 HOG launch and the whole device-resident detect step (development helper for A/B experiments with
-SD_B200_HOG_FLAGS / other switches): python tools/hog_ab.py [batch]"""
+"""Times the HOG launch of every cascade level and the whole device-resident detect step (development helper for comparing
+two builds of the library): python tools/hog_ab.py [batch]"""
 import ctypes as C, os, sys
 import numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -35,4 +35,4 @@ for _ in range(3): model.detect_batch_device(frames, x0)
 torch.cuda.synchronize(); e0.record()
 for _ in range(5): model.detect_batch_device(frames, x0)
 e1.record(); torch.cuda.synchronize()
-print(f"FLAGS={os.environ.get('SD_B200_HOG_FLAGS', '0')} NO_TMA={os.environ.get('SD_B200_HOG_NO_TMA', '0')} hog ms per level {out} sum {sum(out):.3f}; detect step {e0.elapsed_time(e1) / 5:.3f} ms ({B * 5 / e0.elapsed_time(e1) * 1e3:.0f} faces/s)", flush=True)
+print(f"hog ms per level {out} sum {sum(out):.3f}; detect step {e0.elapsed_time(e1) / 5:.3f} ms ({B * 5 / e0.elapsed_time(e1) * 1e3:.0f} faces/s)", flush=True)

@@ -109,9 +109,18 @@ typedef struct {
     const sd_roi* d_roi;
     uint8_t* d_roi_miss;
     /* Optional (NULL = equally sized frames): per-frame size / pitch / position; width, height, row_stride and image_stride
-     * above are then ignored.  Not combinable with d_roi. */
+     * above are then ignored.  With d_roi, d_frames[i] gives only the size of the frame that d_roi[i] was cut from (its
+     * row_stride and offset are unused). */
     const sd_frame* d_frames;
 } sd_image_batch;
+
+/* One 8UC1 frame in host memory for sd_detect_faces_host; frames need not be contiguous or equally sized.  The frame is
+ * `height` rows of `row_stride` bytes from h_data; its last row needs only `width` readable bytes. */
+typedef struct {
+    const uint8_t* h_data;
+    int32_t width, height, row_stride;
+    int32_t reserved;
+} sd_host_frame;
 
 /* ---- context --------------------------------------------------------------------------- */
 /* stream: a cudaStream_t owned by the caller (e.g. torch's current stream); NULL is the CUDA default
@@ -125,7 +134,7 @@ SD_API int sd_sync(sd_ctx* ctx);
 SD_API const char* sd_version(void);
 /* number of kernels of THIS library launched on ctx since creation (bench.py's gpu_launches) */
 SD_API int64_t sd_launch_count(const sd_ctx* ctx);
-/* faces that sd_detect_batch_host had to repeat from their full frame (a patch left the uploaded ROI) */
+/* faces that sd_detect_batch_host / sd_detect_faces_host had to repeat from their full frame (a patch left the uploaded ROI) */
 SD_API int64_t sd_roi_fallback_count(const sd_ctx* ctx);
 
 /* device / pinned-host memory for hosts that do not bring their own allocator */
@@ -346,6 +355,28 @@ SD_API int sd_detect_batch_device(sd_ctx* ctx, const sd_model* m, const sd_image
 SD_API int sd_detect_batch_host(sd_ctx* ctx, const sd_model* m, const uint8_t* h_images, int count,
                                 int width, int height, int row_stride, const int32_t* h_boxes,
                                 float* h_landmarks);
+
+/* ---- several faces per frame, frames of any size ---------------------------------------------------------------------
+ * A face detector returns a list of boxes per frame (cv::CascadeClassifier::detectMultiScale); these calls take every face of
+ * a batch of frames in one call, each face carrying the index of its frame.  Results are bit-identical to detecting each face
+ * on its own frame with the calls above. */
+/* align_mean(mean, box) (model.hpp:64-76) for count boxes on the device: d_boxes is count x 4 (x, y, w, h) int32, row i of
+ * d_x0 (row stride ldx floats) receives the 2L initial landmarks, bit-identical to sd_align_mean(.., 1, 1, 0, 0).  Async. */
+SD_API int sd_model_align_boxes(sd_ctx* ctx, const sd_model* m, const int32_t* d_boxes, int count,
+                                float* d_x0, int64_t ldx);
+/* detect(image, initialisation) for count faces, everything on the device: face i starts from d_x0[i*2L ..] and reads frame
+ * d_frame_index[i] of `frames` (equally sized frames, or one d_frames descriptor each; d_roi is not accepted).  An index out
+ * of range is reported as SD_ERR_INVALID through the projection's status flag (the call synchronises). */
+SD_API int sd_detect_faces_device(sd_ctx* ctx, const sd_model* m, const sd_image_batch* frames,
+                                  const int32_t* d_frame_index, const float* d_x0, int count, float* d_landmarks);
+/* detect(image, facebox) for count faces in num_frames host frames: face i has box h_boxes[4i ..] in frame
+ * h_frames[h_frame_index[i]]; h_landmarks receives count x 2L.  Every index is checked before any work is queued (out of
+ * range: SD_ERR_INVALID); frames without faces are never read.  count == 0 returns SD_OK.
+ * Route: when every referenced frame is pinned and device-mapped with 16-byte aligned base and pitch, the neighbourhoods of
+ * the faces are gathered from host memory (ROIs of one frame that intersect are gathered once, as one region); otherwise
+ * every referenced frame is copied to the device once, whatever its number of faces. */
+SD_API int sd_detect_faces_host(sd_ctx* ctx, const sd_model* m, const sd_host_frame* h_frames, int num_frames,
+                                const int32_t* h_frame_index, const int32_t* h_boxes, int count, float* h_landmarks);
 
 #ifdef __cplusplus
 }

@@ -326,6 +326,40 @@ def bgr2gray(images, ctx: Optional["Context"] = None) -> torch.Tensor:
     return out
 
 
+_FRAME_DTYPE = np.dtype([("w", "<i4"), ("h", "<i4"), ("s", "<i4"), ("r", "<i4"), ("o", "<i8")])   # sd_frame
+
+
+def _gray_frame(im, ctx: "Context"):
+    """One frame as a 2-D uint8 array / tensor; (H, W, 3) B,G,R frames are converted on the device (sd_bgr2gray)."""
+    t = im if isinstance(im, torch.Tensor) else np.ascontiguousarray(im, dtype=np.uint8)
+    if t.ndim == 3 and t.shape[2] == 3:
+        t = bgr2gray(t[None], ctx)[0]
+    if t.ndim != 2 or t.dtype not in (np.uint8, torch.uint8):
+        raise ValueError("every frame must be (H, W) uint8 or (H, W, 3) uint8")
+    return t
+
+
+def pack_frames(images, ctx: Optional["Context"] = None):
+    """Frames of any sizes ((H, W) uint8 or (H, W, 3) uint8 B,G,R; host arrays or tensors) packed back to back on the device,
+    each row padded with zeros to a multiple of 16 bytes.  Returns (data, table): the uint8 device buffer and one sd_frame
+    record per frame (as a uint8 device tensor), the d_data / d_frames pair of an sd_image_batch."""
+    ctx = ctx or default_context()
+    dev = f"cuda:{ctx.device}"
+    grays = [_gray_frame(im, ctx) for im in images]
+    recs, off = [], 0
+    for g in grays:
+        h, w = g.shape
+        stride = (w + 15) // 16 * 16
+        recs.append((w, h, stride, 0, off))
+        off += h * stride
+    data = torch.zeros(max(off, 1), dtype=torch.uint8, device=dev)
+    for g, (w, h, stride, _, o) in zip(grays, recs):
+        src = g if isinstance(g, torch.Tensor) else torch.from_numpy(g)
+        data[o:o + h * stride].view(h, stride)[:, :w].copy_(src)
+    table = np.array(recs, dtype=_FRAME_DTYPE)
+    return data, torch.from_numpy(table.view(np.uint8).copy()).to(dev)
+
+
 class HogTransform:
     """Projection functor h.  images: (count, H, W) uint8 (8UC1) or (count, H, W, 3) uint8 (8UC3, B G R: converted
     once on the device as adaptive_vlhog.hpp:114-120 does per call), on host or device.
@@ -341,26 +375,9 @@ class HogTransform:
         self.ctx = ctx or default_context()
         self.frames = None
         if isinstance(images, (list, tuple)) and len({np.asarray(im).shape for im in images}) > 1:
-            # frames of different sizes (the reference takes a std::vector<cv::Mat>): packed back to back, rows 16-byte aligned,
-            # with one sd_frame descriptor each
-            recs, chunks, off = [], [], 0
-            for im in images:
-                a = np.ascontiguousarray(im, dtype=np.uint8)
-                if a.ndim == 3 and a.shape[2] == 3:
-                    a = bgr2gray(a[None], self.ctx)[0].cpu().numpy()
-                if a.ndim != 2:
-                    raise ValueError("every image must be (H, W) uint8 or (H, W, 3) uint8")
-                h, w = a.shape
-                stride = (w + 15) // 16 * 16
-                buf = np.zeros((h, stride), dtype=np.uint8)
-                buf[:, :w] = a
-                recs.append((w, h, stride, 0, off))
-                chunks.append(buf.reshape(-1))
-                off += h * stride
-            self.images = torch.from_numpy(np.concatenate(chunks)).to(f"cuda:{self.ctx.device}")
-            table = np.array(recs, dtype=[("w", "<i4"), ("h", "<i4"), ("s", "<i4"), ("r", "<i4"), ("o", "<i8")])
-            self.frames = torch.from_numpy(table.view(np.uint8).copy()).to(f"cuda:{self.ctx.device}")
-            self.frame_count = len(recs)
+            # frames of different sizes (the reference takes a std::vector<cv::Mat>)
+            self.images, self.frames = pack_frames(images, self.ctx)
+            self.frame_count = len(images)
         else:
             if isinstance(images, (list, tuple)):
                 images = np.stack([np.asarray(im) for im in images])
@@ -603,6 +620,43 @@ def calculate_normalised_landmark_errors(predictions, groundtruth, model_landmar
     return out
 
 
+_HOST_FRAME_DTYPE = np.dtype([("p", "<u8"), ("w", "<i4"), ("h", "<i4"), ("s", "<i4"), ("r", "<i4")])   # sd_host_frame
+
+
+def _host_frame_table(frames):
+    """sd_host_frame records of gray host frames read in place: an (n, H, W) uint8 array / CPU tensor, or a list of (H, W) ones.
+    Returns (table, objects that must stay alive during the call)."""
+    def plain(f):
+        if isinstance(f, torch.Tensor):
+            if f.is_cuda or f.dtype != torch.uint8:
+                raise ValueError("host frames must be uint8 CPU tensors or arrays")
+            return f if f.stride(-1) == 1 else f.contiguous()
+        f = np.asarray(f)
+        return f if f.dtype == np.uint8 and f.strides[-1] == 1 else np.ascontiguousarray(f, dtype=np.uint8)
+
+    def geometry(f):   # base address, (H, W), row pitch
+        if isinstance(f, torch.Tensor):
+            return f.data_ptr(), tuple(f.shape[-2:]), f.stride(-2)
+        return f.ctypes.data, f.shape[-2:], f.strides[-2]
+
+    if isinstance(frames, (np.ndarray, torch.Tensor)):            # one batch: records computed, not looped over
+        f = plain(frames)
+        base, (h, w), pitch = geometry(f)
+        step = f.stride(0) if isinstance(f, torch.Tensor) else f.strides[0]
+        table = np.zeros(f.shape[0], dtype=_HOST_FRAME_DTYPE)
+        table["p"] = base + step * np.arange(f.shape[0], dtype=np.uint64)
+        table["w"], table["h"], table["s"] = w, h, pitch
+        return table, f
+    keep = [plain(f) for f in frames]
+    table = np.zeros(len(keep), dtype=_HOST_FRAME_DTYPE)
+    for k, f in enumerate(keep):
+        if f.ndim != 2:
+            raise ValueError("every host frame must be (H, W) uint8")
+        base, (h, w), pitch = geometry(f)
+        table[k] = (base, w, h, pitch, 0)
+    return table, keep
+
+
 class detection_model:
     """rcr::detection_model (model.hpp:122-183) resident on the GPU."""
 
@@ -687,6 +741,79 @@ class detection_model:
         ib = ImageBatchC(C.c_void_p(images.data_ptr()), w, h, images.stride(1), images.stride(0), n)
         out = torch.empty((n, 2 * self.num_landmarks), dtype=torch.float32, device=images.device)
         _check(self.ctx.h, _capi.lib().sd_detect_batch_device(self.ctx.h, self._m, C.byref(ib), ptr(x0), n, ptr(out)))
+        return out
+
+    def align_boxes(self, boxes) -> torch.Tensor:
+        """align_mean(mean, box) (model.hpp:64-76) for every (x, y, w, h) row of `boxes`, on the device: (count, 2L) float32,
+        bit-identical to align_mean() on the host."""
+        b = _dev(np.asarray(boxes, dtype=np.int32).reshape(-1, 4) if not isinstance(boxes, torch.Tensor) else boxes.reshape(-1, 4),
+                 self.ctx, dtype=torch.int32)
+        out = torch.empty((b.shape[0], 2 * self.num_landmarks), dtype=torch.float32, device=b.device)
+        _check(self.ctx.h, _capi.lib().sd_model_align_boxes(self.ctx.h, self._m, ptr(b), b.shape[0], ptr(out), C.c_int64(out.stride(0))))
+        return out
+
+    def _device_frames(self, frames):
+        """(sd_image_batch, tensors to keep alive) for frames on the device: an (n, H, W) / (n, H, W, 3) uint8 tensor or array,
+        or a list of frames of any sizes (packed with pack_frames)."""
+        if isinstance(frames, (list, tuple)):
+            data, table = pack_frames(frames, self.ctx)
+            return ImageBatchC(C.c_void_p(data.data_ptr()), 0, 0, 0, 0, len(frames), None, None, C.c_void_p(table.data_ptr())), (data, table)
+        t = frames if isinstance(frames, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(frames, dtype=np.uint8))
+        if t.dim() == 2:
+            t = t.unsqueeze(0)
+        if t.dim() == 4 and t.shape[3] == 3:
+            t = bgr2gray(t, self.ctx)
+        if t.dtype != torch.uint8 or t.dim() != 3:
+            raise ValueError("frames must be (n, H, W) uint8, (n, H, W, 3) uint8 or a list of frames")
+        t = t.to(f"cuda:{self.ctx.device}").contiguous()
+        n, h, w = t.shape
+        return ImageBatchC(C.c_void_p(t.data_ptr()), w, h, t.stride(1), t.stride(0), n), (t,)
+
+    def detect_faces_device(self, frames, frame_index, x0) -> torch.Tensor:
+        """detect(image, initialisation) for several faces per frame on the device: face i starts from x0[i] (count, 2L) and
+        reads frames[frame_index[i]].  frames: an (n, H, W) uint8 tensor, or a list of frames of any sizes.  An index out of
+        range raises SdError with code 1 (SD_ERR_INVALID)."""
+        ib, keep = self._device_frames(frames)
+        idx = _dev(np.asarray(frame_index, dtype=np.int32).ravel() if not isinstance(frame_index, torch.Tensor) else frame_index.reshape(-1),
+                   self.ctx, dtype=torch.int32)
+        x = _dev(x0, self.ctx).reshape(-1, 2 * self.num_landmarks)
+        if x.shape[0] != idx.shape[0]:
+            raise ValueError("one frame index per initialisation")
+        out = torch.empty((x.shape[0], 2 * self.num_landmarks), dtype=torch.float32, device=x.device)
+        _check(self.ctx.h, _capi.lib().sd_detect_faces_device(self.ctx.h, self._m, C.byref(ib), ptr(idx), ptr(x), x.shape[0], ptr(out)))
+        del keep
+        return out
+
+    def detect_faces(self, frames, boxes, frame_index) -> np.ndarray:
+        """detect(image, facebox) for every face of a batch of frames of any sizes: face i has box boxes[i] = (x, y, w, h) in
+        frames[frame_index[i]]; returns (count, 2L).  frames: a list of (H, W) / (H, W, 3) uint8 frames, or an (n, H, W) array.
+        Gray host frames are read in place (each referenced frame is uploaded once; pinned torch tensors take the
+        region-of-interest route); colour frames are converted on the device and take the device route.  A frame index out of
+        range raises SdError with code 1 before any work is queued."""
+        b = np.ascontiguousarray(boxes, dtype=np.int32).reshape(-1, 4)
+        idx = np.ascontiguousarray(frame_index, dtype=np.int32).ravel()
+        if idx.shape[0] != b.shape[0]:
+            raise ValueError("one frame index per box")
+        count, P = b.shape[0], 2 * self.num_landmarks
+        out = np.empty((count, P), dtype=np.float32)
+        batch = isinstance(frames, (np.ndarray, torch.Tensor))
+        if batch and frames.ndim != 3 and frames.ndim != 4:
+            raise ValueError("frames must be an (n, H, W) / (n, H, W, 3) array or a list of frames")
+        if not batch:
+            frames = [f if isinstance(f, (np.ndarray, torch.Tensor)) else np.asarray(f) for f in frames]
+        if count == 0:
+            return out
+        bad = (idx < 0) | (idx >= len(frames))
+        if bad.any():
+            i = int(np.argmax(bad))
+            raise SdError(1, f"detect_faces: face {i}: frame index {int(idx[i])} is not in [0, {len(frames)})")
+        if (batch and frames.ndim == 4) or (not batch and any(f.ndim == 3 for f in frames)):
+            return self.detect_faces_device(frames, idx, self.align_boxes(b)).cpu().numpy()
+        table, keep = _host_frame_table(frames)
+        _check(self.ctx.h, _capi.lib().sd_detect_faces_host(self.ctx.h, self._m, table.ctypes.data_as(C.c_void_p), len(table),
+                                                            idx.ctypes.data_as(C.c_void_p), b.ctypes.data_as(C.c_void_p), count,
+                                                            out.ctypes.data_as(C.c_void_p)))
+        del keep
         return out
 
     def save(self, filename: str) -> None:

@@ -679,7 +679,6 @@ int launch_hog(sd_ctx* ctx, const sd_image_batch* images, const int32_t* d_image
     a.roi = images->d_roi;
     a.roi_miss = images->d_roi_miss;
     a.frames = images->d_frames;
-    SD_REQUIRE(ctx, !(images->d_roi && images->d_frames), "d_roi and d_frames cannot be combined");
     if (!d_image_index) SD_REQUIRE(ctx, images->count >= N, "fewer images than samples and no image index");
     a.x = d_x; a.ldx = ldx; a.N = N; a.L = L;
     a.variant = p->variant; a.nc = p->num_cells; a.cs = p->cell_size; a.K = p->num_bins; a.fs = fs;

@@ -23,6 +23,7 @@ struct sd_model {
     std::vector<sd_regulariser> regs;
     std::vector<sd_hog_param> hog;
     std::vector<float> mean;
+    float* d_mean = nullptr;                      // device copy for sd_model_align_boxes
     std::vector<std::string> ids, right_ids, left_ids;
     sd_normalisation norm{};
 };
@@ -136,12 +137,15 @@ int validate_and_upload(sd_ctx* ctx, sd_model* m)
         SD_CUDA(ctx, cudaMalloc(&m->d_weights[s], bytes));
         SD_CUDA(ctx, cudaMemcpyAsync(m->d_weights[s], m->weights[s].data(), bytes, cudaMemcpyHostToDevice, ctx->stream));
     }
+    SD_CUDA(ctx, cudaMalloc(&m->d_mean, m->mean.size() * sizeof(float)));
+    SD_CUDA(ctx, cudaMemcpyAsync(m->d_mean, m->mean.data(), m->mean.size() * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
     SD_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return SD_OK;
 }
 
-int detect_device(sd_ctx* ctx, const sd_model* m, const sd_image_batch* images, const float* d_x0, int count,
-                  float* d_landmarks)
+// d_image_index: frame of each face (NULL: face i reads frame i)
+int detect_device(sd_ctx* ctx, const sd_model* m, const sd_image_batch* images, const int32_t* d_image_index, const float* d_x0,
+                  int count, float* d_landmarks)
 {
     const int L = m->num_landmarks, P = 2 * L;
     if (count <= 0) return SD_OK;
@@ -158,7 +162,7 @@ int detect_device(sd_ctx* ctx, const sd_model* m, const sd_image_batch* images, 
     float* cur = xa;
     float* nxt = xb;
     for (int s = 0; s < m->num_levels; ++s) {               // superviseddescent.hpp:326-342
-        int rc = sd_hog_batch(ctx, images, nullptr, cur, P, count, L, &m->norm, &m->hog[s], A, ld);
+        int rc = sd_hog_batch(ctx, images, d_image_index, cur, P, count, L, &m->norm, &m->hog[s], A, ld);
         if (rc) return rc;
         rc = sd_cascade_update(ctx, A, ld, count, m->rows[s], m->d_weights[s], P, cur, &m->norm, nxt);
         if (rc) return rc;
@@ -169,18 +173,27 @@ int detect_device(sd_ctx* ctx, const sd_model* m, const sd_image_batch* images, 
 }
 
 
-// ---- region-of-interest upload (sd_detect_batch_host) ------------------------------------------------
-// The cascade only ever reads a neighbourhood of the face, so instead of copying whole 640x480 frames over
-// PCIe a small kernel pulls the ROI rows of every face straight out of the caller's PINNED host buffer
-// (zero-copy loads through the unified address space, 16-byte vectors) into a packed device buffer.  If a
-// patch later needs a frame pixel outside its ROI the HOG kernel raises d_roi_miss[face] and that face is
-// repeated from its full frame, so the result never depends on the ROI heuristic.
-__global__ void __launch_bounds__(256) roi_gather_kernel(const uint8_t* __restrict__ h_frames, long long frame_bytes, int row_stride,
-                                                         const sd_roi* __restrict__ roi, int first, int n, uint8_t* __restrict__ dst)
+// ---- region-of-interest upload (sd_detect_batch_host, sd_detect_faces_host) --------------------------------
+// The cascade only ever reads a neighbourhood of the face, so instead of copying whole frames over PCIe a small kernel pulls
+// the rows of every ROI straight out of the caller's PINNED host frames (zero-copy loads through the unified address space,
+// 16-byte vectors) into a packed device buffer.  If a patch later needs a frame pixel outside its ROI the HOG kernel raises
+// d_roi_miss[roi] and the faces of that ROI are repeated from their full frame, so the result never depends on the ROI
+// heuristic.
+
+// where ROI i is read from: the device-mapped address of its frame's first pixel and the frame's pitch
+struct RoiSource {
+    const uint8_t* frame;
+    long long row_stride;
+};
+
+__global__ void __launch_bounds__(256) roi_gather_kernel(const RoiSource* __restrict__ srcs, const sd_roi* __restrict__ roi, int first,
+                                                         int n, uint8_t* __restrict__ dst)
 {
     for (int f = blockIdx.x; f < n; f += gridDim.x) {
         const sd_roi r = roi[first + f];
-        const uint8_t* src = h_frames + (long long)(first + f) * frame_bytes + (long long)r.y * row_stride + r.x;
+        const RoiSource s = srcs[first + f];
+        const long long row_stride = s.row_stride;
+        const uint8_t* src = s.frame + (long long)r.y * row_stride + r.x;
         uint8_t* d = dst + r.offset;
         const int vec_per_row = r.row_stride >> 4;
         const int total = vec_per_row * r.h;
@@ -200,6 +213,22 @@ __global__ void __launch_bounds__(256) roi_gather_kernel(const uint8_t* __restri
                 if (i0 + u * blockDim.x < total) reinterpret_cast<uint4*>(d + (long long)row[u] * r.row_stride)[col[u]] = v[u];
         }
     }
+}
+
+// sd_align_mean(mean, box, 1, 1, 0, 0) for every coordinate of every box, bit for bit: the scale and offset are formed in
+// double and rounded to float as the host does, and the product and sum are separately rounded (no FMA contraction)
+__global__ void align_boxes_kernel(const float* __restrict__ mean, int L, const int32_t* __restrict__ boxes, int count,
+                                   float* __restrict__ x0, long long ldx)
+{
+    const long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    const int P = 2 * L;
+    if (t >= (long long)count * P) return;
+    const int i = (int)(t / P), j = (int)(t - (long long)i * P);
+    const bool is_y = j >= L;
+    const int origin = boxes[4 * i + (is_y ? 1 : 0)], size = boxes[4 * i + (is_y ? 3 : 2)];
+    const float a = __double2float_rn(__dmul_rn(1.0, (double)size));
+    const float b = __double2float_rn(__dadd_rn(__dmul_rn(__dadd_rn(0.5, 0.0), (double)size), (double)origin));
+    x0[(long long)i * ldx + j] = __fadd_rn(__fmul_rn(mean[j], a), b);
 }
 
 // conservative ROI of one face: landmark bounding box of the initialisation, grown by the largest patch
@@ -434,6 +463,7 @@ void sd_model_destroy(sd_model* m)
     if (!m) return;
     cudaSetDevice(m->device);
     for (float* p : m->d_weights) if (p) cudaFree(p);
+    if (m->d_mean) cudaFree(m->d_mean);
     delete m;
 }
 
@@ -483,138 +513,344 @@ int sd_detect_batch_device(sd_ctx* ctx, const sd_model* m, const sd_image_batch*
     if (!ctx) return SD_ERR_INVALID;
     SD_REQUIRE(ctx, m && images && d_x0 && d_landmarks && count >= 0, "bad argument");
     SD_REQUIRE(ctx, images->count >= count, "fewer images than faces");
-    const int rc = detect_device(ctx, m, images, d_x0, count, d_landmarks);
+    const int rc = detect_device(ctx, m, images, nullptr, d_x0, count, d_landmarks);
     if (rc) return rc;
     // a degenerate face (inter-eye distance too small for a patch) or a bad frame index is an error here, as it is in the
     // reference (cv::resize on an empty ROI throws); reading the flag synchronises the stream
     return sd_check_hog_status(ctx, "detect");
 }
 
-static int detect_host_full(sd_ctx* ctx, const sd_model* m, const uint8_t* h_images, int count, int width, int height,
-                            int row_stride, const int32_t* h_boxes, float* h_landmarks)
+}  // extern "C"
+
+namespace {
+
+// one 8UC1 frame in host memory; d_alias: its device-mapped address when it is pinned with 16-byte aligned base and pitch
+struct HostFrame {
+    const uint8_t* h;
+    const uint8_t* d_alias;
+    int width, height, row_stride;
+};
+
+int ensure_staging(sd_ctx* ctx, size_t bytes)
 {
-    const int L = m->num_landmarks, P = 2 * L;
-    const size_t frame_bytes = (size_t)height * row_stride;
-    // chunking: ~128 MB of frames per staging buffer, at least 1 face
-    int chunk = (int)((size_t)(128u << 20) / frame_bytes);
-    if (chunk < 1) chunk = 1;
-    if (chunk > count) chunk = count;
     for (int b = 0; b < 2; ++b) {
-        if (ctx->stage_bytes[b] < (size_t)chunk * frame_bytes) {
+        if (ctx->stage_bytes[b] < bytes) {
             if (ctx->d_stage[b]) { SD_CUDA(ctx, cudaStreamSynchronize(ctx->stream)); SD_CUDA(ctx, cudaStreamSynchronize(ctx->copy_stream)); SD_CUDA(ctx, cudaFree(ctx->d_stage[b])); ctx->d_stage[b] = nullptr; }
-            SD_CUDA(ctx, cudaMalloc(&ctx->d_stage[b], (size_t)chunk * frame_bytes));
-            ctx->stage_bytes[b] = (size_t)chunk * frame_bytes;
+            SD_CUDA(ctx, cudaMalloc(&ctx->d_stage[b], bytes));
+            ctx->stage_bytes[b] = bytes;
         }
     }
-    // initial landmarks for every face: align_mean on the host (model.hpp:135), one small upload
-    std::vector<float> x0((size_t)count * P);
-    for (int i = 0; i < count; ++i)
-        sd_align_mean(m->mean.data(), L, h_boxes[4 * i], h_boxes[4 * i + 1], h_boxes[4 * i + 2], h_boxes[4 * i + 3], 1.f, 1.f, 0.f, 0.f, &x0[(size_t)i * P]);
-    float* d_x = (float*)sd_workspace(ctx, SD_WS_PARTIAL, (size_t)2 * count * P * sizeof(float));
-    if (!d_x) return SD_ERR_CUDA;
-    float* d_out = d_x + (size_t)count * P;
-    SD_CUDA(ctx, cudaMemcpyAsync(d_x, x0.data(), x0.size() * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+    return SD_OK;
+}
+
+// Whole-frame route.  Faces [0, count) with frame[k] = frames[fidx[k]], fidx non-decreasing; h_x0 / h_out in that order.
+// Every referenced frame is uploaded once into the double-buffered staging, in chunks of whole frames (~128 MB, or a single
+// frame larger than that) together with all of their faces.  A chunk of equally sized frames is staged as a uniform batch (the
+// HOG kernel's TMA route applies), any other chunk is described by sd_frame records.
+int detect_host_full(sd_ctx* ctx, const sd_model* m, const HostFrame* frames, const int* fidx, const float* h_x0, int count, float* h_out)
+{
+    const int P = 2 * m->num_landmarks;
+    const size_t cap = (size_t)128 << 20;
+    // distinct referenced frames (in face order) and the chunks they are staged in
+    std::vector<int> uf;                       // unique frame -> frames[]
+    std::vector<int> face_u(count);            // face -> unique frame
+    for (int k = 0; k < count; ++k) {
+        if (k == 0 || fidx[k] != fidx[k - 1]) uf.push_back(fidx[k]);
+        face_u[k] = (int)uf.size() - 1;
+    }
+    struct Chunk { int u0, u1, f0, f1; bool uniform; };
+    std::vector<Chunk> chunks;
+    std::vector<sd_frame> rec(uf.size());
+    size_t used = 0, stage_need = 0;
+    for (int u = 0; u < (int)uf.size(); ++u) {
+        const HostFrame& f = frames[uf[u]];
+        const size_t padded = ((size_t)f.height * f.row_stride + 15) & ~(size_t)15;
+        if (chunks.empty() || used + padded > cap) { chunks.push_back({u, u, 0, 0, true}); used = 0; }
+        rec[u] = sd_frame{f.width, f.height, f.row_stride, 0, (int64_t)used};
+        used += padded;
+        chunks.back().u1 = u + 1;
+    }
+    for (Chunk& c : chunks) {
+        const HostFrame& f0 = frames[uf[c.u0]];
+        for (int u = c.u0; u < c.u1; ++u) {
+            const HostFrame& f = frames[uf[u]];
+            c.uniform = c.uniform && f.width == f0.width && f.height == f0.height && f.row_stride == f0.row_stride;
+        }
+        const size_t fb = (size_t)f0.height * f0.row_stride;
+        if (c.uniform)                          // packed back to back, like one (n, height, row_stride) array
+            for (int u = c.u0; u < c.u1; ++u) rec[u].offset = (int64_t)((u - c.u0) * fb);
+        const size_t bytes = (size_t)(rec[c.u1 - 1].offset) + (size_t)frames[uf[c.u1 - 1]].height * frames[uf[c.u1 - 1]].row_stride;
+        stage_need = bytes > stage_need ? bytes : stage_need;
+    }
+    for (size_t c = 0, k = 0; c < chunks.size(); ++c) {
+        chunks[c].f0 = (int)k;
+        while (k < (size_t)count && face_u[k] < chunks[c].u1) ++k;
+        chunks[c].f1 = (int)k;
+    }
+    int rc = ensure_staging(ctx, stage_need);
+    if (rc) return rc;
+    // device tables: landmarks (in, out), frame of every face relative to its chunk, frame records
+    std::vector<int32_t> local(count);
+    bool identity = true;                       // one face per frame: no index needed
+    for (const Chunk& c : chunks)
+        for (int k = c.f0; k < c.f1; ++k) { local[k] = face_u[k] - c.u0; identity = identity && local[k] == k - c.f0; }
+    const size_t xbytes = (size_t)count * P * sizeof(float);
+    const size_t ibytes = ((size_t)count * sizeof(int32_t) + 15) & ~(size_t)15;
+    unsigned char* tab = (unsigned char*)sd_workspace(ctx, SD_WS_PARTIAL, 2 * xbytes + ibytes + rec.size() * sizeof(sd_frame));
+    if (!tab) return SD_ERR_CUDA;
+    float* d_x = (float*)tab;
+    float* d_out = (float*)(tab + xbytes);
+    int32_t* d_idx = (int32_t*)(tab + 2 * xbytes);
+    sd_frame* d_rec = (sd_frame*)(tab + 2 * xbytes + ibytes);
+    SD_CUDA(ctx, cudaMemcpyAsync(d_x, h_x0, xbytes, cudaMemcpyHostToDevice, ctx->stream));
+    if (!identity) SD_CUDA(ctx, cudaMemcpyAsync(d_idx, local.data(), (size_t)count * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+    bool any_mixed = false;
+    for (const Chunk& c : chunks) any_mixed = any_mixed || !c.uniform;
+    if (any_mixed) SD_CUDA(ctx, cudaMemcpyAsync(d_rec, rec.data(), rec.size() * sizeof(sd_frame), cudaMemcpyHostToDevice, ctx->stream));
     // the copy stream must not run ahead of work already queued on the compute stream that still reads the staging buffers
     SD_CUDA(ctx, cudaEventRecord(ctx->stage_done[0], ctx->stream));
     SD_CUDA(ctx, cudaEventRecord(ctx->stage_done[1], ctx->stream));
     int buf = 0;
-    for (int first = 0; first < count; first += chunk, buf ^= 1) {
-        const int n = (count - first < chunk) ? count - first : chunk;
+    for (size_t c = 0; c < chunks.size(); ++c, buf ^= 1) {
+        const Chunk& ch = chunks[c];
+        uint8_t* stage = (uint8_t*)ctx->d_stage[buf];
         SD_CUDA(ctx, cudaStreamWaitEvent(ctx->copy_stream, ctx->stage_done[buf], 0));
-        SD_CUDA(ctx, cudaMemcpyAsync(ctx->d_stage[buf], h_images + (size_t)first * frame_bytes, (size_t)n * frame_bytes,
-                                     cudaMemcpyHostToDevice, ctx->copy_stream));
+        // one copy per run of frames that lie back to back both in host memory and in the staging buffer; the last row of a run
+        // is copied up to its width only (the caller's buffer may end there)
+        for (int u = ch.u0; u < ch.u1;) {
+            const HostFrame& f = frames[uf[u]];
+            const size_t fb = (size_t)f.height * f.row_stride;
+            int v = u + 1;
+            while (v < ch.u1 && frames[uf[v]].h == f.h + (v - u) * fb && rec[v].offset == rec[u].offset + (int64_t)((v - u) * fb) &&
+                   frames[uf[v]].row_stride == f.row_stride && frames[uf[v]].height == f.height && frames[uf[v]].width == f.width)
+                ++v;
+            const size_t bytes = (size_t)(v - u - 1) * fb + (size_t)(f.height - 1) * f.row_stride + f.width;
+            SD_CUDA(ctx, cudaMemcpyAsync(stage + rec[u].offset, f.h, bytes, cudaMemcpyHostToDevice, ctx->copy_stream));
+            u = v;
+        }
         SD_CUDA(ctx, cudaEventRecord(ctx->stage_ev[buf], ctx->copy_stream));
         SD_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->stage_ev[buf], 0));
         sd_image_batch ib{};
-        ib.d_data = (const uint8_t*)ctx->d_stage[buf];
-        ib.width = width; ib.height = height; ib.row_stride = row_stride; ib.image_stride = (int64_t)frame_bytes; ib.count = n;
-        int rc = detect_device(ctx, m, &ib, d_x + (size_t)first * P, n, d_out + (size_t)first * P);
+        ib.d_data = stage;
+        ib.count = ch.u1 - ch.u0;
+        if (ch.uniform) {
+            const HostFrame& f = frames[uf[ch.u0]];
+            ib.width = f.width; ib.height = f.height; ib.row_stride = f.row_stride; ib.image_stride = (int64_t)f.height * f.row_stride;
+        } else {
+            ib.d_frames = d_rec + ch.u0;
+        }
+        const int n = ch.f1 - ch.f0;
+        rc = detect_device(ctx, m, &ib, identity ? nullptr : d_idx + ch.f0, d_x + (size_t)ch.f0 * P, n, d_out + (size_t)ch.f0 * P);
         if (rc) return rc;
         SD_CUDA(ctx, cudaEventRecord(ctx->stage_done[buf], ctx->stream));
     }
-    SD_CUDA(ctx, cudaMemcpyAsync(h_landmarks, d_out, (size_t)count * P * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    SD_CUDA(ctx, cudaMemcpyAsync(h_out, d_out, xbytes, cudaMemcpyDeviceToHost, ctx->stream));
     return sd_check_hog_status(ctx, "detect");                // synchronises
 }
 
-// ROI route: needs the caller's frames in pinned (device-mapped) host memory
-static int detect_host_roi(sd_ctx* ctx, const sd_model* m, const uint8_t* h_images, const uint8_t* d_alias, int count, int width,
-                           int height, int row_stride, const int32_t* h_boxes, float* h_landmarks)
+bool roi_intersect(const sd_roi& a, const sd_roi& b)
 {
-    const int L = m->num_landmarks, P = 2 * L;
-    const size_t frame_bytes = (size_t)height * row_stride;
+    return a.x < b.x + b.w && b.x < a.x + a.w && a.y < b.y + b.h && b.y < a.y + a.h;
+}
+
+// ROI route: every referenced frame pinned and device-mapped (HostFrame::d_alias).  Same face order and arguments as
+// detect_host_full.  The ROIs of the faces of one frame that intersect are merged into one ROI group, gathered once; face ->
+// group is the image index of the HOG launch, and d_roi / d_roi_miss / the gather's source table are indexed by group.
+int detect_host_roi(sd_ctx* ctx, const sd_model* m, const HostFrame* frames, const int* fidx, const float* h_x0, int count, float* h_out)
+{
+    const int P = 2 * m->num_landmarks;
     const size_t chunk_cap = (size_t)48 << 20;            // packed ROI bytes per staging buffer
-    // initial landmarks and the ROI of every face; faces are grouped into chunks that fit one staging buffer
-    std::vector<float> x0((size_t)count * P);
-    std::vector<sd_roi> rois(count);
-    std::vector<int> chunk_first;
-    size_t used = 0;
-    for (int i = 0; i < count; ++i) {
-        sd_align_mean(m->mean.data(), L, h_boxes[4 * i], h_boxes[4 * i + 1], h_boxes[4 * i + 2], h_boxes[4 * i + 3], 1.f, 1.f, 0.f, 0.f, &x0[(size_t)i * P]);
-        sd_roi r = face_roi(m, &x0[(size_t)i * P], width, height, row_stride);
-        const size_t bytes = (size_t)r.row_stride * r.h;
-        if (bytes > chunk_cap)                                // a face window larger than a staging buffer: whole-frame route
-            return detect_host_full(ctx, m, h_images, count, width, height, row_stride, h_boxes, h_landmarks);
-        if (chunk_first.empty() || used + bytes > chunk_cap) { chunk_first.push_back(i); used = 0; }
-        r.offset = (int64_t)used;
-        used += bytes;
-        rois[i] = r;
-    }
-    chunk_first.push_back(count);
-    for (int b = 0; b < 2; ++b) {
-        if (ctx->stage_bytes[b] < chunk_cap + (1u << 20)) {
-            if (ctx->d_stage[b]) { SD_CUDA(ctx, cudaStreamSynchronize(ctx->stream)); SD_CUDA(ctx, cudaStreamSynchronize(ctx->copy_stream)); SD_CUDA(ctx, cudaFree(ctx->d_stage[b])); ctx->d_stage[b] = nullptr; }
-            SD_CUDA(ctx, cudaMalloc(&ctx->d_stage[b], chunk_cap + (1u << 20)));
-            ctx->stage_bytes[b] = chunk_cap + (1u << 20);
+    // ROI groups, frame by frame: merge until no two groups of the frame intersect
+    std::vector<sd_roi> groups;
+    std::vector<int> group_frame;
+    std::vector<int> face_group(count);
+    for (int k0 = 0; k0 < count;) {
+        int k1 = k0;
+        while (k1 < count && fidx[k1] == fidx[k0]) ++k1;
+        const HostFrame& f = frames[fidx[k0]];
+        const int g0 = (int)groups.size();
+        for (int k = k0; k < k1; ++k) {
+            sd_roi r = face_roi(m, h_x0 + (size_t)k * P, f.width, f.height, f.row_stride);
+            int g = -1;
+            for (int j = g0; j < (int)groups.size() && g < 0; ++j) if (roi_intersect(groups[j], r)) g = j;
+            if (g < 0) { groups.push_back(r); group_frame.push_back(fidx[k0]); face_group[k] = (int)groups.size() - 1; continue; }
+            face_group[k] = g;
+            for (bool grown = true; grown;) {              // the union may now reach other groups of this frame: absorb them
+                sd_roi& u = groups[g];
+                const int xa = u.x < r.x ? u.x : r.x, ya = u.y < r.y ? u.y : r.y;
+                const int xb = u.x + u.w > r.x + r.w ? u.x + u.w : r.x + r.w, yb = u.y + u.h > r.y + r.h ? u.y + u.h : r.y + r.h;
+                u.x = xa; u.y = ya; u.w = xb - xa; u.h = yb - ya; u.row_stride = u.w;   // x and w stay multiples of 16
+                grown = false;
+                for (int j = g0; j < (int)groups.size(); ++j) {
+                    if (j == g || !roi_intersect(groups[j], groups[g])) continue;
+                    r = groups[j];
+                    const int ng = j < g ? g - 1 : g;      // index of group g once j is erased
+                    for (int q = k0; q < k; ++q) face_group[q] = face_group[q] == j ? ng : (face_group[q] > j ? face_group[q] - 1 : face_group[q]);
+                    groups.erase(groups.begin() + j);
+                    group_frame.erase(group_frame.begin() + j);
+                    g = ng;
+                    face_group[k] = g;
+                    grown = true;
+                    break;
+                }
+            }
         }
+        k0 = k1;
     }
-    // device tables: landmarks (in, out), ROI records, miss flags
+    const int G = (int)groups.size();
+    // faces ordered by group (stable): the faces of a group are contiguous, so chunks of whole groups are ranges of faces
+    std::vector<int> pos(count);                           // group order -> position in the caller's order
+    {
+        std::vector<int> start(G + 1, 0);
+        for (int k = 0; k < count; ++k) start[face_group[k] + 1]++;
+        for (int g = 0; g < G; ++g) start[g + 1] += start[g];
+        for (int k = 0; k < count; ++k) pos[start[face_group[k]]++] = k;
+    }
+    bool identity = G == count;                            // one face per group, groups in face order
+    for (int k = 0; k < count && identity; ++k) identity = pos[k] == k && face_group[k] == k;
+    std::vector<float> gx0, gout;
+    const float* x0 = h_x0;
+    float* out = h_out;
+    if (!identity) {
+        gx0.resize((size_t)count * P); gout.resize((size_t)count * P);
+        for (int k = 0; k < count; ++k) memcpy(&gx0[(size_t)k * P], h_x0 + (size_t)pos[k] * P, P * sizeof(float));
+        x0 = gx0.data(); out = gout.data();
+    }
+    std::vector<int> gface0(G + 1, 0);                     // first face (group order) of every group
+    for (int k = 0; k < count; ++k) gface0[face_group[pos[k]] + 1]++;
+    for (int g = 0; g < G; ++g) gface0[g + 1] += gface0[g];
+    std::vector<int32_t> local(count);                     // face -> group, relative to the chunk's first group
+    std::vector<int> chunk_first;                          // groups
+    std::vector<RoiSource> srcs(G);
+    bool same_size = true;
+    size_t used = 0;
+    for (int g = 0; g < G; ++g) {
+        const HostFrame& f = frames[group_frame[g]];
+        same_size = same_size && f.width == frames[group_frame[0]].width && f.height == frames[group_frame[0]].height;
+        const size_t bytes = (size_t)groups[g].row_stride * groups[g].h;
+        if (bytes > chunk_cap)                                // a face window larger than a staging buffer: whole-frame route
+            return detect_host_full(ctx, m, frames, fidx, h_x0, count, h_out);
+        if (chunk_first.empty() || used + bytes > chunk_cap) { chunk_first.push_back(g); used = 0; }
+        groups[g].offset = (int64_t)used;
+        used += bytes;
+        srcs[g] = RoiSource{f.d_alias, (long long)f.row_stride};
+        for (int k = gface0[g]; k < gface0[g + 1]; ++k) local[k] = g - chunk_first.back();
+    }
+    chunk_first.push_back(G);
+    int rc = ensure_staging(ctx, chunk_cap + (1u << 20));
+    if (rc) return rc;
+    // frames of different sizes: the size of every group's frame (where the zero padding of a patch starts)
+    std::vector<sd_frame> gframes;
+    if (!same_size)
+        for (int g = 0; g < G; ++g) gframes.push_back(sd_frame{frames[group_frame[g]].width, frames[group_frame[g]].height, 0, 0, 0});
+    // device tables: landmarks (in, out), ROI records, gather sources, face -> group, frame sizes, miss flags
     const size_t xbytes = (size_t)count * P * sizeof(float);
-    const size_t rbytes = (size_t)count * sizeof(sd_roi);
-    unsigned char* tab = (unsigned char*)sd_workspace(ctx, SD_WS_PARTIAL, 2 * xbytes + rbytes + count + 64);
+    const size_t rbytes = (size_t)G * sizeof(sd_roi);
+    const size_t sbytes = (size_t)G * sizeof(RoiSource);
+    const size_t ibytes = ((size_t)count * sizeof(int32_t) + 15) & ~(size_t)15;
+    const size_t fbytes = gframes.size() * sizeof(sd_frame);
+    unsigned char* tab = (unsigned char*)sd_workspace(ctx, SD_WS_PARTIAL, 2 * xbytes + rbytes + sbytes + ibytes + fbytes + G + 64);
     if (!tab) return SD_ERR_CUDA;
     float* d_x = (float*)tab;
     float* d_out = (float*)(tab + xbytes);
     sd_roi* d_roi = (sd_roi*)(tab + 2 * xbytes);
-    uint8_t* d_miss = tab + 2 * xbytes + rbytes;
-    SD_CUDA(ctx, cudaMemcpyAsync(d_x, x0.data(), xbytes, cudaMemcpyHostToDevice, ctx->stream));
-    SD_CUDA(ctx, cudaMemcpyAsync(d_roi, rois.data(), rbytes, cudaMemcpyHostToDevice, ctx->stream));
-    SD_CUDA(ctx, cudaMemsetAsync(d_miss, 0, count, ctx->stream));
+    RoiSource* d_src = (RoiSource*)(tab + 2 * xbytes + rbytes);
+    int32_t* d_idx = (int32_t*)(tab + 2 * xbytes + rbytes + sbytes);
+    sd_frame* d_gframes = (sd_frame*)(tab + 2 * xbytes + rbytes + sbytes + ibytes);
+    uint8_t* d_miss = tab + 2 * xbytes + rbytes + sbytes + ibytes + fbytes;
+    SD_CUDA(ctx, cudaMemcpyAsync(d_x, x0, xbytes, cudaMemcpyHostToDevice, ctx->stream));
+    SD_CUDA(ctx, cudaMemcpyAsync(d_roi, groups.data(), rbytes, cudaMemcpyHostToDevice, ctx->stream));
+    SD_CUDA(ctx, cudaMemcpyAsync(d_src, srcs.data(), sbytes, cudaMemcpyHostToDevice, ctx->stream));
+    if (!identity) SD_CUDA(ctx, cudaMemcpyAsync(d_idx, local.data(), (size_t)count * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+    if (fbytes) SD_CUDA(ctx, cudaMemcpyAsync(d_gframes, gframes.data(), fbytes, cudaMemcpyHostToDevice, ctx->stream));
+    SD_CUDA(ctx, cudaMemsetAsync(d_miss, 0, G, ctx->stream));
     SD_CUDA(ctx, cudaEventRecord(ctx->stage_done[0], ctx->stream));
     SD_CUDA(ctx, cudaEventRecord(ctx->stage_done[1], ctx->stream));
+    const HostFrame& f0 = frames[group_frame[0]];
     int buf = 0;
     for (size_t c = 0; c + 1 < chunk_first.size(); ++c, buf ^= 1) {
         const int first = chunk_first[c], n = chunk_first[c + 1] - first;
         SD_CUDA(ctx, cudaStreamWaitEvent(ctx->copy_stream, ctx->stage_done[buf], 0));   // also orders the table uploads before the first gather
         const int blocks = n < 8 * ctx->sm_count ? n : 8 * ctx->sm_count;
-        roi_gather_kernel<<<blocks, 256, 0, ctx->copy_stream>>>(d_alias, (long long)frame_bytes, row_stride, d_roi, first, n, (uint8_t*)ctx->d_stage[buf]);
+        roi_gather_kernel<<<blocks, 256, 0, ctx->copy_stream>>>(d_src, d_roi, first, n, (uint8_t*)ctx->d_stage[buf]);
         SD_LAUNCH_CHECK(ctx, "roi_gather_kernel");
         SD_CUDA(ctx, cudaEventRecord(ctx->stage_ev[buf], ctx->copy_stream));
         SD_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->stage_ev[buf], 0));
         sd_image_batch ib{};
         ib.d_data = (const uint8_t*)ctx->d_stage[buf];
-        ib.width = width; ib.height = height; ib.row_stride = row_stride; ib.image_stride = 0; ib.count = n;
+        ib.width = f0.width; ib.height = f0.height; ib.row_stride = f0.row_stride; ib.image_stride = 0; ib.count = n;
         ib.d_roi = d_roi + first;
         ib.d_roi_miss = d_miss + first;
-        int rc = detect_device(ctx, m, &ib, d_x + (size_t)first * P, n, d_out + (size_t)first * P);
+        if (fbytes) ib.d_frames = d_gframes + first;
+        const int k0 = gface0[first], nf = gface0[first + n] - k0;
+        rc = detect_device(ctx, m, &ib, identity ? nullptr : d_idx + k0, d_x + (size_t)k0 * P, nf, d_out + (size_t)k0 * P);
         if (rc) return rc;
         SD_CUDA(ctx, cudaEventRecord(ctx->stage_done[buf], ctx->stream));
     }
-    std::vector<uint8_t> miss(count);
-    SD_CUDA(ctx, cudaMemcpyAsync(h_landmarks, d_out, xbytes, cudaMemcpyDeviceToHost, ctx->stream));
-    SD_CUDA(ctx, cudaMemcpyAsync(miss.data(), d_miss, count, cudaMemcpyDeviceToHost, ctx->stream));
-    {
-        const int rc = sd_check_hog_status(ctx, "detect");    // synchronises
+    std::vector<uint8_t> miss(G);
+    SD_CUDA(ctx, cudaMemcpyAsync(out, d_out, xbytes, cudaMemcpyDeviceToHost, ctx->stream));
+    SD_CUDA(ctx, cudaMemcpyAsync(miss.data(), d_miss, G, cudaMemcpyDeviceToHost, ctx->stream));
+    rc = sd_check_hog_status(ctx, "detect");             // synchronises
+    if (rc) return rc;
+    // groups whose cascade wandered outside the uploaded region: repeat their faces from the full frame, uploaded once
+    for (int g = 0; g < G; ++g) {
+        if (!miss[g]) continue;
+        const int k0 = gface0[g], nf = gface0[g + 1] - k0;
+        ctx->roi_fallbacks += nf;
+        const std::vector<int> zero(nf, 0);
+        rc = detect_host_full(ctx, m, &frames[group_frame[g]], zero.data(), x0 + (size_t)k0 * P, nf, out + (size_t)k0 * P);
         if (rc) return rc;
     }
-    // faces whose cascade wandered outside the uploaded region: repeat them from their full frames
-    for (int i = 0; i < count; ++i) {
-        if (!miss[i]) continue;
-        ctx->roi_fallbacks++;
-        int rc = detect_host_full(ctx, m, h_images + (size_t)i * frame_bytes, 1, width, height, row_stride, h_boxes + 4 * i, h_landmarks + (size_t)i * P);
-        if (rc) return rc;
-    }
+    if (!identity)
+        for (int k = 0; k < count; ++k) memcpy(h_out + (size_t)pos[k] * P, &gout[(size_t)k * P], P * sizeof(float));
     return SD_OK;
 }
+
+// detect(image, facebox) for count faces; face i in frames[frame_index ? frame_index[i] : i] (indices already validated).
+// Faces are taken frame by frame (stable), their initial landmarks aligned on the host (model.hpp:135).
+int detect_host(sd_ctx* ctx, const sd_model* m, const std::vector<HostFrame>& frames, const int32_t* frame_index, const int32_t* h_boxes,
+                int count, float* h_landmarks, bool roi)
+{
+    const int L = m->num_landmarks, P = 2 * L;
+    const int F = (int)frames.size();
+    std::vector<int> order(count), fidx(count);
+    if (frame_index) {
+        std::vector<int> start(F + 1, 0);
+        for (int i = 0; i < count; ++i) start[frame_index[i] + 1]++;
+        for (int f = 0; f < F; ++f) start[f + 1] += start[f];
+        for (int i = 0; i < count; ++i) order[start[frame_index[i]]++] = i;
+        for (int k = 0; k < count; ++k) fidx[k] = frame_index[order[k]];
+    } else {
+        for (int i = 0; i < count; ++i) order[i] = fidx[i] = i;
+    }
+    bool identity = true;
+    for (int k = 0; k < count && identity; ++k) identity = order[k] == k;
+    std::vector<float> x0((size_t)count * P), sorted_out;
+    for (int k = 0; k < count; ++k) {
+        const int32_t* b = h_boxes + 4 * (size_t)order[k];
+        sd_align_mean(m->mean.data(), L, b[0], b[1], b[2], b[3], 1.f, 1.f, 0.f, 0.f, &x0[(size_t)k * P]);
+    }
+    float* out = h_landmarks;
+    if (!identity) { sorted_out.resize((size_t)count * P); out = sorted_out.data(); }
+    const int rc = roi ? detect_host_roi(ctx, m, frames.data(), fidx.data(), x0.data(), count, out)
+                       : detect_host_full(ctx, m, frames.data(), fidx.data(), x0.data(), count, out);
+    if (rc) return rc;
+    if (!identity)
+        for (int k = 0; k < count; ++k) memcpy(h_landmarks + (size_t)order[k] * P, &sorted_out[(size_t)k * P], P * sizeof(float));
+    return SD_OK;
+}
+
+// device-mapped address of a pinned host buffer, or null (pageable memory: not an error)
+const uint8_t* mapped_alias(const void* h)
+{
+    cudaPointerAttributes attr;
+    if (cudaPointerGetAttributes(&attr, h) != cudaSuccess) { cudaGetLastError(); return nullptr; }
+    return attr.type == cudaMemoryTypeHost ? (const uint8_t*)attr.devicePointer : nullptr;
+}
+
+}  // namespace
+
+extern "C" {
 
 int sd_detect_batch_host(sd_ctx* ctx, const sd_model* m, const uint8_t* h_images, int count, int width, int height,
                          int row_stride, const int32_t* h_boxes, float* h_landmarks)
@@ -624,13 +860,66 @@ int sd_detect_batch_host(sd_ctx* ctx, const sd_model* m, const uint8_t* h_images
     if (count == 0) return SD_OK;
     // ROI route when the frames are in pinned, device-mapped host memory with 16-byte aligned rows
     const size_t frame_bytes = (size_t)height * row_stride;
-    cudaPointerAttributes attr;
-    const bool pinned = cudaPointerGetAttributes(&attr, h_images) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer;
-    if (!pinned) cudaGetLastError();
-    const bool aligned = pinned && ((reinterpret_cast<uintptr_t>(attr.devicePointer) | (uintptr_t)row_stride | (uintptr_t)frame_bytes) & 15) == 0;
-    if (aligned)
-        return detect_host_roi(ctx, m, h_images, (const uint8_t*)attr.devicePointer, count, width, height, row_stride, h_boxes, h_landmarks);
-    return detect_host_full(ctx, m, h_images, count, width, height, row_stride, h_boxes, h_landmarks);
+    const uint8_t* alias = mapped_alias(h_images);
+    const bool aligned = alias && ((reinterpret_cast<uintptr_t>(alias) | (uintptr_t)row_stride | (uintptr_t)frame_bytes) & 15) == 0;
+    std::vector<HostFrame> frames(count);
+    for (int i = 0; i < count; ++i)
+        frames[i] = HostFrame{h_images + i * frame_bytes, aligned ? alias + i * frame_bytes : nullptr, width, height, row_stride};
+    return detect_host(ctx, m, frames, nullptr, h_boxes, count, h_landmarks, aligned);
+}
+
+int sd_model_align_boxes(sd_ctx* ctx, const sd_model* m, const int32_t* d_boxes, int count, float* d_x0, int64_t ldx)
+{
+    if (!ctx) return SD_ERR_INVALID;
+    SD_REQUIRE(ctx, m && count >= 0 && ldx >= 2 * (int64_t)m->num_landmarks, "bad argument");
+    if (count == 0) return SD_OK;
+    SD_REQUIRE(ctx, d_boxes && d_x0, "null argument");
+    const int L = m->num_landmarks;
+    const long long total = (long long)count * 2 * L;
+    align_boxes_kernel<<<sd_div_up(total, 256), 256, 0, ctx->stream>>>(m->d_mean, L, d_boxes, count, d_x0, ldx);
+    SD_LAUNCH_CHECK(ctx, "align_boxes_kernel");
+    return SD_OK;
+}
+
+int sd_detect_faces_device(sd_ctx* ctx, const sd_model* m, const sd_image_batch* frames, const int32_t* d_frame_index, const float* d_x0,
+                           int count, float* d_landmarks)
+{
+    if (!ctx) return SD_ERR_INVALID;
+    SD_REQUIRE(ctx, m && frames && count >= 0, "bad argument");
+    if (count == 0) return SD_OK;
+    SD_REQUIRE(ctx, d_frame_index && d_x0 && d_landmarks && frames->count >= 1, "bad argument");
+    SD_REQUIRE(ctx, !frames->d_roi, "d_roi is not supported here");
+    const int rc = detect_device(ctx, m, frames, d_frame_index, d_x0, count, d_landmarks);
+    if (rc) return rc;
+    return sd_check_hog_status(ctx, "detect");               // a frame index out of range is reported here
+}
+
+int sd_detect_faces_host(sd_ctx* ctx, const sd_model* m, const sd_host_frame* h_frames, int num_frames, const int32_t* h_frame_index,
+                         const int32_t* h_boxes, int count, float* h_landmarks)
+{
+    if (!ctx) return SD_ERR_INVALID;
+    SD_REQUIRE(ctx, m && count >= 0 && num_frames >= 0, "bad argument");
+    if (count == 0) return SD_OK;
+    SD_REQUIRE(ctx, h_frames && h_frame_index && h_boxes && h_landmarks && num_frames >= 1, "bad argument");
+    std::vector<char> used(num_frames, 0);
+    for (int i = 0; i < count; ++i) {
+        if (h_frame_index[i] < 0 || h_frame_index[i] >= num_frames)
+            return sd_fail(ctx, SD_ERR_INVALID, "%s: face %d: frame index %d is not in [0, %d)", __func__, i, h_frame_index[i], num_frames);
+        used[h_frame_index[i]] = 1;
+    }
+    // frames without faces are never read, so only the referenced ones are checked
+    std::vector<HostFrame> frames(num_frames, HostFrame{nullptr, nullptr, 0, 0, 0});
+    bool roi = true;
+    for (int f = 0; f < num_frames; ++f) {
+        if (!used[f]) continue;
+        const sd_host_frame& hf = h_frames[f];
+        if (!hf.h_data || hf.width <= 0 || hf.height <= 0 || hf.row_stride < hf.width)
+            return sd_fail(ctx, SD_ERR_INVALID, "%s: frame %d: bad data pointer or size", __func__, f);
+        const uint8_t* alias = roi ? mapped_alias(hf.h_data) : nullptr;
+        roi = alias && ((reinterpret_cast<uintptr_t>(alias) | (uintptr_t)hf.row_stride) & 15) == 0;
+        frames[f] = HostFrame{hf.h_data, alias, hf.width, hf.height, hf.row_stride};
+    }
+    return detect_host(ctx, m, frames, h_frame_index, h_boxes, count, h_landmarks, roi);
 }
 
 }  // extern "C"

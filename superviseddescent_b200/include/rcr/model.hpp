@@ -163,6 +163,74 @@ public:
         return out;
     }
 
+    // Several faces per frame, frames of any sizes (the box list a face detector such as detectMultiScale returns for each
+    // frame): result[i][j] holds the landmarks of faceboxes[i][j] in images[i].  Gray frames are read in place through their
+    // own row pointers (sd_detect_faces_host); if any frame with faces is colour, the frames go to the device, are converted
+    // there (sd_bgr2gray) and the boxes are aligned there (sd_model_align_boxes, sd_detect_faces_device).
+    std::vector<std::vector<LandmarkCollection<cv::Vec2f>>> detect(const std::vector<cv::Mat>& images, const std::vector<std::vector<cv::Rect>>& faceboxes)
+    {
+        if (images.size() != faceboxes.size()) throw std::runtime_error("detect: images / faceboxes size mismatch");
+        sd_ctx* ctx = sd_b200::context();
+        const int P = 2 * sd_model_num_landmarks(handle.get());
+        std::vector<int32_t> index, boxes;
+        bool colour = false;
+        for (size_t i = 0; i < images.size(); ++i) {
+            if (faceboxes[i].empty()) continue;
+            if (images[i].empty()) throw std::runtime_error("detect: empty image with face boxes");
+            colour = colour || images[i].channels() == 3;
+            for (const cv::Rect& b : faceboxes[i]) {
+                index.push_back(static_cast<int32_t>(i));
+                boxes.push_back(b.x); boxes.push_back(b.y); boxes.push_back(b.width); boxes.push_back(b.height);
+            }
+        }
+        const int count = static_cast<int>(index.size());
+        std::vector<float> lms(static_cast<size_t>(count) * P);
+        if (count > 0 && !colour) {
+            std::vector<sd_host_frame> frames(images.size());
+            for (size_t i = 0; i < images.size(); ++i)
+                if (!faceboxes[i].empty())
+                    frames[i] = sd_host_frame{images[i].ptr<unsigned char>(0), images[i].cols, images[i].rows, static_cast<int32_t>(images[i].step()), 0};
+            sd_b200::check(ctx, sd_detect_faces_host(ctx, handle.get(), frames.data(), static_cast<int>(frames.size()), index.data(), boxes.data(), count,
+                                                     lms.data()), "sd_detect_faces_host");
+        } else if (count > 0) {
+            // the frames with faces, packed on the device as 8UC1 with 16-byte aligned rows, one sd_frame record each
+            std::vector<sd_frame> rec;
+            std::vector<int32_t> local(images.size(), -1);
+            int64_t off = 0;
+            for (size_t i = 0; i < images.size(); ++i) {
+                if (faceboxes[i].empty()) continue;
+                const int w = images[i].cols, h = images[i].rows, stride = (w + 15) / 16 * 16;
+                local[i] = static_cast<int32_t>(rec.size());
+                rec.push_back(sd_frame{w, h, stride, 0, off});
+                off += static_cast<int64_t>(h) * stride;
+            }
+            for (int32_t& f : index) f = local[f];
+            sd_b200::DeviceBuffer dimg(static_cast<size_t>(off)), drec(rec.size() * sizeof(sd_frame)), didx(index.size() * sizeof(int32_t)),
+                dboxes(boxes.size() * sizeof(int32_t)), dx(lms.size() * sizeof(float)), dout(lms.size() * sizeof(float)), bgr;
+            for (size_t i = 0; i < images.size(); ++i)
+                if (local[i] >= 0) upload_gray(ctx, images[i], dimg.as<unsigned char>() + rec[local[i]].offset, bgr, rec[local[i]].row_stride);
+            sd_b200::check(ctx, sd_memcpy_h2d(ctx, drec.as<sd_frame>(), rec.data(), rec.size() * sizeof(sd_frame)), "detect");
+            sd_b200::check(ctx, sd_memcpy_h2d(ctx, didx.as<int32_t>(), index.data(), index.size() * sizeof(int32_t)), "detect");
+            sd_b200::check(ctx, sd_memcpy_h2d(ctx, dboxes.as<int32_t>(), boxes.data(), boxes.size() * sizeof(int32_t)), "detect");
+            sd_b200::check(ctx, sd_model_align_boxes(ctx, handle.get(), dboxes.as<int32_t>(), count, dx.as<float>(), P), "sd_model_align_boxes");
+            sd_image_batch ib{};
+            ib.d_data = dimg.as<unsigned char>(); ib.count = static_cast<int32_t>(rec.size()); ib.d_frames = drec.as<sd_frame>();
+            sd_b200::check(ctx, sd_detect_faces_device(ctx, handle.get(), &ib, didx.as<int32_t>(), dx.as<float>(), count, dout.as<float>()),
+                           "sd_detect_faces_device");
+            const cv::Mat all = sd_b200::download(dout.as<float>(), count, P, P);
+            std::memcpy(lms.data(), all.ptr<float>(0), lms.size() * sizeof(float));
+        }
+        std::vector<std::vector<LandmarkCollection<cv::Vec2f>>> out(images.size());
+        size_t k = 0;
+        for (size_t i = 0; i < images.size(); ++i)
+            for (size_t j = 0; j < faceboxes[i].size(); ++j, ++k) {
+                cv::Mat row(1, P, CV_32FC1);
+                std::memcpy(row.ptr<float>(0), &lms[k * P], sizeof(float) * P);
+                out[i].push_back(to_landmark_collection(row, landmark_ids));
+            }
+        return out;
+    }
+
     cv::Mat get_mean()
     {
         cv::Mat mean(1, 2 * sd_model_num_landmarks(handle.get()), CV_32FC1);
@@ -174,21 +242,22 @@ public:
 
 private:
     friend detection_model load_detection_model(std::string filename);
-    // frame -> device as 8UC1; colour frames go up as B,G,R and are converted there
-    // (cv::cvtColor BGR2GRAY of adaptive_vlhog.hpp:115-117 == sd_bgr2gray)
-    static void upload_gray(sd_ctx* ctx, const cv::Mat& image, unsigned char* d_dst, sd_b200::DeviceBuffer& bgr)
+    // frame -> device as 8UC1 with rows dst_stride bytes apart (0: packed); colour frames go up as B,G,R and are converted
+    // there (cv::cvtColor BGR2GRAY of adaptive_vlhog.hpp:115-117 == sd_bgr2gray)
+    static void upload_gray(sd_ctx* ctx, const cv::Mat& image, unsigned char* d_dst, sd_b200::DeviceBuffer& bgr, int dst_stride = 0)
     {
         const int w = image.cols, h = image.rows;
         const size_t frame = static_cast<size_t>(w) * h;
+        const size_t ds = dst_stride > 0 ? static_cast<size_t>(dst_stride) : static_cast<size_t>(w);
         if (image.channels() == 3) {
             bgr.allocate(3 * frame);
             for (int y = 0; y < h; ++y)
                 sd_b200::check(ctx, sd_memcpy_h2d(ctx, bgr.as<unsigned char>() + static_cast<size_t>(y) * 3 * w, image.ptr<unsigned char>(y), 3 * static_cast<size_t>(w)), "detect upload");
-            sd_b200::check(ctx, sd_bgr2gray(ctx, bgr.as<unsigned char>(), w, h, 3 * static_cast<int64_t>(w), 3 * static_cast<int64_t>(frame), 1, d_dst, w,
-                                            static_cast<int64_t>(frame)), "sd_bgr2gray");
+            sd_b200::check(ctx, sd_bgr2gray(ctx, bgr.as<unsigned char>(), w, h, 3 * static_cast<int64_t>(w), 3 * static_cast<int64_t>(frame), 1, d_dst,
+                                            static_cast<int64_t>(ds), static_cast<int64_t>(ds * h)), "sd_bgr2gray");
         } else {
             for (int y = 0; y < h; ++y)
-                sd_b200::check(ctx, sd_memcpy_h2d(ctx, d_dst + static_cast<size_t>(y) * w, image.ptr<unsigned char>(y), w), "detect upload");
+                sd_b200::check(ctx, sd_memcpy_h2d(ctx, d_dst + static_cast<size_t>(y) * ds, image.ptr<unsigned char>(y), w), "detect upload");
         }
     }
 

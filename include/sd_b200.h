@@ -12,7 +12,8 @@
  *   - matrices are row-major float32, one sample per row (cv::Mat CV_32FC1 as the
  *     reference uses it, regressors.hpp:202-206); `ld` = row stride in floats.
  *   - landmark rows are [x_0..x_{L-1}, y_0..y_{L-1}] (adaptive_vlhog.hpp:96-97).
- *   - images are 8-bit single channel (adaptive_vlhog.hpp:115-120 grey path).
+ *   - images are 8-bit single channel (adaptive_vlhog.hpp:115-120 grey path); the host-frame detect calls also take
+ *     8-bit B,G,R frames and convert them as cv::cvtColor(BGR2GRAY) does.
  *   - pointers named d_* are DEVICE pointers, h_* are HOST pointers.
  *   - every call is asynchronous on the context's stream unless it returns host
  *     data; sd_sync() waits.  Functions are re-entrant on distinct contexts.
@@ -114,12 +115,14 @@ typedef struct {
     const sd_frame* d_frames;
 } sd_image_batch;
 
-/* One 8UC1 frame in host memory for sd_detect_faces_host; frames need not be contiguous or equally sized.  The frame is
- * `height` rows of `row_stride` bytes from h_data; its last row needs only `width` readable bytes. */
+/* One frame in host memory for sd_detect_faces_host / sd_detect_faces_host_init; frames need not be contiguous or equally
+ * sized.  channels: 0 or 1 = 8UC1, 3 = 8UC3 interleaved B,G,R (cv::imread / cv::VideoCapture output; converted as
+ * cv::cvtColor(BGR2GRAY), adaptive_vlhog.hpp:114-120, bit for bit like sd_bgr2gray).  The frame is `height` rows of
+ * `row_stride` bytes (at least channels x width) from h_data; its last row needs only channels x width readable bytes. */
 typedef struct {
     const uint8_t* h_data;
     int32_t width, height, row_stride;
-    int32_t reserved;
+    int32_t channels;
 } sd_host_frame;
 
 /* ---- context --------------------------------------------------------------------------- */
@@ -370,13 +373,21 @@ SD_API int sd_model_align_boxes(sd_ctx* ctx, const sd_model* m, const int32_t* d
 SD_API int sd_detect_faces_device(sd_ctx* ctx, const sd_model* m, const sd_image_batch* frames,
                                   const int32_t* d_frame_index, const float* d_x0, int count, float* d_landmarks);
 /* detect(image, facebox) for count faces in num_frames host frames: face i has box h_boxes[4i ..] in frame
- * h_frames[h_frame_index[i]]; h_landmarks receives count x 2L.  Every index is checked before any work is queued (out of
- * range: SD_ERR_INVALID); frames without faces are never read.  count == 0 returns SD_OK.
+ * h_frames[h_frame_index[i]]; h_landmarks receives count x 2L.  Every index and every referenced frame (size, pitch,
+ * channels) is checked before any work is queued (SD_ERR_INVALID); frames without faces are never read.  count == 0
+ * returns SD_OK.  Gray and colour frames may be mixed.
  * Route: when every referenced frame is pinned and device-mapped with 16-byte aligned base and pitch, the neighbourhoods of
- * the faces are gathered from host memory (ROIs of one frame that intersect are gathered once, as one region); otherwise
- * every referenced frame is copied to the device once, whatever its number of faces. */
+ * the faces are gathered from host memory (ROIs of one frame that intersect are gathered once, as one region; a colour ROI
+ * is converted to gray as it is gathered, so only the neighbourhood is read and converted); otherwise every referenced frame
+ * is copied to the device once, whatever its number of faces (colour frames as B,G,R, converted there). */
 SD_API int sd_detect_faces_host(sd_ctx* ctx, const sd_model* m, const sd_host_frame* h_frames, int num_frames,
                                 const int32_t* h_frame_index, const int32_t* h_boxes, int count, float* h_landmarks);
+/* detect(image, initialisation) (model.hpp:147-157, e.g. the landmarks of the previous frame of a video) for count faces in
+ * host frames: face i starts from h_x0[i * ldx .. + 2L] (ldx >= 2L floats).  Checks, routes and results as
+ * sd_detect_faces_host, which is this call with the mean aligned to each box. */
+SD_API int sd_detect_faces_host_init(sd_ctx* ctx, const sd_model* m, const sd_host_frame* h_frames, int num_frames,
+                                     const int32_t* h_frame_index, const float* h_x0, int64_t ldx, int count,
+                                     float* h_landmarks);
 
 #ifdef __cplusplus
 }

@@ -45,8 +45,9 @@ class FrameC(C.Structure):
 
 
 class HostFrameC(C.Structure):
-    """sd_host_frame: one 8UC1 frame in host memory for sd_detect_faces_host."""
-    _fields_ = [("h_data", C.c_void_p), ("width", C.c_int32), ("height", C.c_int32), ("row_stride", C.c_int32), ("reserved", C.c_int32)]
+    """sd_host_frame: one frame in host memory for sd_detect_faces_host / sd_detect_faces_host_init; channels 0 or 1 = 8UC1,
+    3 = 8UC3 B,G,R."""
+    _fields_ = [("h_data", C.c_void_p), ("width", C.c_int32), ("height", C.c_int32), ("row_stride", C.c_int32), ("channels", C.c_int32)]
 
 
 # every symbol declared in include/sd_b200.h (tests/test_abi.py checks the list against the header)
@@ -64,7 +65,7 @@ EXPORTS = [
     "sd_model_get_mean", "sd_model_get_weights", "sd_model_landmark_id", "sd_align_mean",
     "sd_perturb_box", "sd_normalised_landmark_errors",
     "sd_detect_batch_device", "sd_detect_batch_host",
-    "sd_model_align_boxes", "sd_detect_faces_device", "sd_detect_faces_host",
+    "sd_model_align_boxes", "sd_detect_faces_device", "sd_detect_faces_host", "sd_detect_faces_host_init",
 ]
 
 _lib = None

@@ -620,41 +620,54 @@ def calculate_normalised_landmark_errors(predictions, groundtruth, model_landmar
     return out
 
 
-_HOST_FRAME_DTYPE = np.dtype([("p", "<u8"), ("w", "<i4"), ("h", "<i4"), ("s", "<i4"), ("r", "<i4")])   # sd_host_frame
+_HOST_FRAME_DTYPE = np.dtype([("p", "<u8"), ("w", "<i4"), ("h", "<i4"), ("s", "<i4"), ("channels", "<i4")])   # sd_host_frame
 
 
 def _host_frame_table(frames):
-    """sd_host_frame records of gray host frames read in place: an (n, H, W) uint8 array / CPU tensor, or a list of (H, W) ones.
-    Returns (table, objects that must stay alive during the call)."""
-    def plain(f):
+    """sd_host_frame records of host frames read in place: an (n, H, W) or (n, H, W, 3) uint8 array / CPU tensor, or a list of
+    (H, W) / (H, W, 3) ones (3 channels: interleaved B, G, R).  Returns (table, objects that must stay alive during the call)."""
+    def plain(f, colour):   # rows of contiguous pixels: in place where they already are
         if isinstance(f, torch.Tensor):
             if f.is_cuda or f.dtype != torch.uint8:
                 raise ValueError("host frames must be uint8 CPU tensors or arrays")
-            return f if f.stride(-1) == 1 else f.contiguous()
-        f = np.asarray(f)
-        return f if f.dtype == np.uint8 and f.strides[-1] == 1 else np.ascontiguousarray(f, dtype=np.uint8)
+            return f if f.stride(-1) == 1 and (not colour or f.stride(-2) == 3) else f.contiguous()
+        ok = f.dtype == np.uint8 and f.strides[-1] == 1 and (not colour or f.strides[-2] == 3)
+        return f if ok else np.ascontiguousarray(f, dtype=np.uint8)
 
-    def geometry(f):   # base address, (H, W), row pitch
+    def geometry(f, colour):   # base address, (H, W), row pitch in bytes
+        r = -3 if colour else -2
         if isinstance(f, torch.Tensor):
-            return f.data_ptr(), tuple(f.shape[-2:]), f.stride(-2)
-        return f.ctypes.data, f.shape[-2:], f.strides[-2]
+            return f.data_ptr(), (f.shape[r], f.shape[r + 1]), f.stride(r)
+        return f.ctypes.data, (f.shape[r], f.shape[r + 1]), f.strides[r]
 
     if isinstance(frames, (np.ndarray, torch.Tensor)):            # one batch: records computed, not looped over
-        f = plain(frames)
-        base, (h, w), pitch = geometry(f)
+        colour = frames.ndim == 4
+        if frames.ndim not in (3, 4) or (colour and frames.shape[3] != 3):
+            raise ValueError("a batch of host frames must be (n, H, W) uint8 or (n, H, W, 3) uint8")
+        f = plain(frames, colour)
+        base, (h, w), pitch = geometry(f, colour)
         step = f.stride(0) if isinstance(f, torch.Tensor) else f.strides[0]
         table = np.zeros(f.shape[0], dtype=_HOST_FRAME_DTYPE)
         table["p"] = base + step * np.arange(f.shape[0], dtype=np.uint64)
-        table["w"], table["h"], table["s"] = w, h, pitch
+        table["w"], table["h"], table["s"], table["channels"] = w, h, pitch, 3 if colour else 1
         return table, f
-    keep = [plain(f) for f in frames]
-    table = np.zeros(len(keep), dtype=_HOST_FRAME_DTYPE)
-    for k, f in enumerate(keep):
-        if f.ndim != 2:
-            raise ValueError("every host frame must be (H, W) uint8")
-        base, (h, w), pitch = geometry(f)
-        table[k] = (base, w, h, pitch, 0)
+    keep = []
+    table = np.zeros(len(frames), dtype=_HOST_FRAME_DTYPE)
+    for k, f in enumerate(frames):
+        f = f if isinstance(f, torch.Tensor) else np.asarray(f)
+        colour = f.ndim == 3 and f.shape[2] == 3
+        if f.ndim != 2 and not colour:
+            raise ValueError("every host frame must be (H, W) uint8 or (H, W, 3) uint8")
+        keep.append(plain(f, colour))
+        base, (h, w), pitch = geometry(keep[-1], colour)
+        table[k] = (base, w, h, pitch, 3 if colour else 1)
     return table, keep
+
+
+def _on_device(frames) -> bool:
+    if isinstance(frames, torch.Tensor):
+        return frames.is_cuda
+    return isinstance(frames, (list, tuple)) and any(isinstance(f, torch.Tensor) and f.is_cuda for f in frames)
 
 
 class detection_model:
@@ -705,28 +718,26 @@ class detection_model:
         return out
 
     def detect(self, image, facebox_or_initialisation) -> np.ndarray:
-        """detect(image, facebox) / detect(image, initialisation) (model.hpp:132-157): one frame, returns the 2L row."""
-        image = np.ascontiguousarray(image, dtype=np.uint8)
+        """detect(image, facebox) / detect(image, initialisation) (model.hpp:132-157): one frame, (H, W) or (H, W, 3) B,G,R
+        uint8, returns the 2L row."""
         arg = np.asarray(facebox_or_initialisation)
+        if not isinstance(image, torch.Tensor):
+            image = np.ascontiguousarray(image, dtype=np.uint8)
         if arg.size == 4:
             return self.detect_batch(image[None], np.asarray(arg, dtype=np.int32)[None])[0]
-        x0 = _dev(np.asarray(arg, dtype=np.float32).reshape(1, -1), self.ctx)
-        imgs = _dev(image[None], self.ctx, dtype=torch.uint8)
-        return self.detect_batch_device(imgs, x0).cpu().numpy()[0]
+        return self.detect_faces_from([image], arg.reshape(1, -1), np.zeros(1, dtype=np.int32))[0]
 
     def detect_batch(self, images: np.ndarray, boxes: np.ndarray) -> np.ndarray:
-        """Batched detect(image, facebox) with HOST buffers (copies are part of the call).  Colour frames
-        (count, H, W, 3) are converted on the device first (model.hpp:134-145 calls cvtColor through HogTransform)."""
+        """Batched detect(image, facebox) with HOST buffers (copies are part of the call), one face per frame.  Colour frames
+        (count, H, W, 3), B,G,R as cv::imread gives them, are converted to gray on the device as they are read
+        (model.hpp:134-145 calls cvtColor through HogTransform)."""
         if isinstance(images, torch.Tensor):
             images_np = images.numpy()
         else:
             images_np = np.ascontiguousarray(images, dtype=np.uint8)
         if images_np.ndim == 4:
-            gray = bgr2gray(images_np, self.ctx)
-            n = gray.shape[0]
-            b = np.ascontiguousarray(boxes, dtype=np.int32).reshape(n, 4)
-            x0 = torch.from_numpy(np.stack([align_mean(self.get_mean(), tuple(int(v) for v in b[i])) for i in range(n)]).astype(np.float32))
-            return self.detect_batch_device(gray, x0.to(gray.device)).cpu().numpy()
+            n = images_np.shape[0]
+            return self.detect_faces(images_np, np.asarray(boxes, dtype=np.int32).reshape(n, 4), np.arange(n, dtype=np.int32))
         n, h, w = images_np.shape
         boxes = np.ascontiguousarray(boxes, dtype=np.int32).reshape(n, 4)
         out = np.empty((n, 2 * self.num_landmarks), dtype=np.float32)
@@ -784,35 +795,62 @@ class detection_model:
         del keep
         return out
 
-    def detect_faces(self, frames, boxes, frame_index) -> np.ndarray:
-        """detect(image, facebox) for every face of a batch of frames of any sizes: face i has box boxes[i] = (x, y, w, h) in
-        frames[frame_index[i]]; returns (count, 2L).  frames: a list of (H, W) / (H, W, 3) uint8 frames, or an (n, H, W) array.
-        Gray host frames are read in place (each referenced frame is uploaded once; pinned torch tensors take the
-        region-of-interest route); colour frames are converted on the device and take the device route.  A frame index out of
-        range raises SdError with code 1 before any work is queued."""
-        b = np.ascontiguousarray(boxes, dtype=np.int32).reshape(-1, 4)
+    def _frames_and_index(self, frames, frame_index, count: int, what: str):
+        """(frames, int32 index, batch?) of a detect_faces / detect_faces_from call; an index out of range raises SdError 1."""
         idx = np.ascontiguousarray(frame_index, dtype=np.int32).ravel()
-        if idx.shape[0] != b.shape[0]:
-            raise ValueError("one frame index per box")
-        count, P = b.shape[0], 2 * self.num_landmarks
-        out = np.empty((count, P), dtype=np.float32)
+        if idx.shape[0] != count:
+            raise ValueError(f"one frame index per {what}")
         batch = isinstance(frames, (np.ndarray, torch.Tensor))
         if batch and frames.ndim != 3 and frames.ndim != 4:
             raise ValueError("frames must be an (n, H, W) / (n, H, W, 3) array or a list of frames")
         if not batch:
             frames = [f if isinstance(f, (np.ndarray, torch.Tensor)) else np.asarray(f) for f in frames]
-        if count == 0:
-            return out
         bad = (idx < 0) | (idx >= len(frames))
-        if bad.any():
+        if count and bad.any():
             i = int(np.argmax(bad))
             raise SdError(1, f"detect_faces: face {i}: frame index {int(idx[i])} is not in [0, {len(frames)})")
-        if (batch and frames.ndim == 4) or (not batch and any(f.ndim == 3 for f in frames)):
+        return frames, idx
+
+    def detect_faces(self, frames, boxes, frame_index) -> np.ndarray:
+        """detect(image, facebox) for every face of a batch of frames of any sizes: face i has box boxes[i] = (x, y, w, h) in
+        frames[frame_index[i]]; returns (count, 2L).  frames: a list of (H, W) / (H, W, 3) uint8 frames (3 channels: B,G,R),
+        or an (n, H, W) / (n, H, W, 3) array.  Host frames, gray or colour, are read in place (each referenced frame is uploaded
+        once; pinned torch tensors take the region-of-interest route, which converts colour neighbourhoods to gray as it
+        gathers them); frames already on the device take the device route.  A frame index out of range raises SdError with
+        code 1 before any work is queued."""
+        b = np.ascontiguousarray(boxes, dtype=np.int32).reshape(-1, 4)
+        count, P = b.shape[0], 2 * self.num_landmarks
+        frames, idx = self._frames_and_index(frames, frame_index, count, "box")
+        out = np.empty((count, P), dtype=np.float32)
+        if count == 0:
+            return out
+        if _on_device(frames):
             return self.detect_faces_device(frames, idx, self.align_boxes(b)).cpu().numpy()
         table, keep = _host_frame_table(frames)
         _check(self.ctx.h, _capi.lib().sd_detect_faces_host(self.ctx.h, self._m, table.ctypes.data_as(C.c_void_p), len(table),
                                                             idx.ctypes.data_as(C.c_void_p), b.ctypes.data_as(C.c_void_p), count,
                                                             out.ctypes.data_as(C.c_void_p)))
+        del keep
+        return out
+
+    def detect_faces_from(self, frames, initialisations, frame_index) -> np.ndarray:
+        """detect(image, initialisation) (model.hpp:147-157, e.g. the landmarks of the previous video frame) for every face of a
+        batch of frames: face i starts from initialisations[i] (count, 2L) in frames[frame_index[i]]; returns (count, 2L).
+        Frames and routes as in detect_faces."""
+        P = 2 * self.num_landmarks
+        x0 = np.ascontiguousarray(initialisations.cpu().numpy() if isinstance(initialisations, torch.Tensor) else initialisations,
+                                  dtype=np.float32).reshape(-1, P)
+        count = x0.shape[0]
+        frames, idx = self._frames_and_index(frames, frame_index, count, "initialisation")
+        out = np.empty((count, P), dtype=np.float32)
+        if count == 0:
+            return out
+        if _on_device(frames):
+            return self.detect_faces_device(frames, idx, x0).cpu().numpy()
+        table, keep = _host_frame_table(frames)
+        _check(self.ctx.h, _capi.lib().sd_detect_faces_host_init(self.ctx.h, self._m, table.ctypes.data_as(C.c_void_p), len(table),
+                                                                 idx.ctypes.data_as(C.c_void_p), x0.ctypes.data_as(C.c_void_p),
+                                                                 C.c_int64(P), count, out.ctypes.data_as(C.c_void_p)))
         del keep
         return out
 

@@ -779,39 +779,59 @@ int launch_hog(sd_ctx* ctx, const sd_image_batch* images, const int32_t* d_image
 namespace {
 // cv::cvtColor(BGR2GRAY), 8-bit, OpenCV >= 3 fixed point (15-bit coefficients): HBM-bound, 3 bytes read + 1 written per
 // pixel.  A thread converts four pixels: three aligned 32-bit loads, one 32-bit store (scalar path for the row tail or
-// unaligned rows).
-__global__ void bgr2gray_kernel(const uint8_t* __restrict__ bgr, int width, int height, long long srow, long long simg, int count,
-                                uint8_t* __restrict__ gray, long long drow, long long dimg, int vec_ok)
+// unaligned rows).  Frame j of the launch is jobs[j] (frames of any sizes, e.g. the colour frames of one staging chunk), or
+// with jobs == NULL `uniform` shifted by j image strides.  blockIdx.y strides over the frames, blockIdx.x over one frame.
+__global__ void bgr2gray_kernel(const uint8_t* __restrict__ bgr, uint8_t* __restrict__ gray, sd_bgr2gray_job uniform,
+                                long long simg, long long dimg, const sd_bgr2gray_job* __restrict__ jobs, int count)
 {
-    const int groups = (width + 3) >> 2;
-    const long long total = (long long)count * height * groups;
-    for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < total; t += (long long)gridDim.x * blockDim.x) {
-        const int g = (int)(t % groups);
-        const long long ry = t / groups;
-        const int y = (int)(ry % height);
-        const long long im = ry / height;
-        const uint8_t* s = bgr + im * simg + (long long)y * srow + 12 * g;
-        uint8_t* d = gray + im * dimg + (long long)y * drow + 4 * g;
-        const int x0 = 4 * g;
-        if (vec_ok && x0 + 4 <= width) {
-            const uint32_t w0 = *reinterpret_cast<const uint32_t*>(s), w1 = *reinterpret_cast<const uint32_t*>(s + 4),
-                           w2 = *reinterpret_cast<const uint32_t*>(s + 8);
-            // bytes: w0 = B0 G0 R0 B1 | w1 = G1 R1 B2 G2 | w2 = R2 B3 G3 R3   (little endian)
-            const uint32_t b0 = w0 & 255, g0 = (w0 >> 8) & 255, r0 = (w0 >> 16) & 255, b1 = w0 >> 24;
-            const uint32_t g1 = w1 & 255, r1 = (w1 >> 8) & 255, b2 = (w1 >> 16) & 255, g2 = w1 >> 24;
-            const uint32_t r2 = w2 & 255, b3 = (w2 >> 8) & 255, g3 = (w2 >> 16) & 255, r3 = w2 >> 24;
-            const uint32_t y0 = (3735u * b0 + 19235u * g0 + 9798u * r0 + (1u << 14)) >> 15;
-            const uint32_t y1 = (3735u * b1 + 19235u * g1 + 9798u * r1 + (1u << 14)) >> 15;
-            const uint32_t y2 = (3735u * b2 + 19235u * g2 + 9798u * r2 + (1u << 14)) >> 15;
-            const uint32_t y3 = (3735u * b3 + 19235u * g3 + 9798u * r3 + (1u << 14)) >> 15;
-            *reinterpret_cast<uint32_t*>(d) = y0 | (y1 << 8) | (y2 << 16) | (y3 << 24);
-        } else {
-            for (int k = 0; k < 4 && x0 + k < width; ++k)
-                d[k] = (uint8_t)((3735u * s[3 * k] + 19235u * s[3 * k + 1] + 9798u * s[3 * k + 2] + (1u << 14)) >> 15);
+    for (int j = blockIdx.y; j < count; j += gridDim.y) {
+        const sd_bgr2gray_job job = jobs ? jobs[j] : uniform;
+        const uint8_t* sbase = bgr + job.src_offset + (jobs ? 0 : j * simg);
+        uint8_t* dbase = gray + job.dst_offset + (jobs ? 0 : j * dimg);
+        const int width = job.width;
+        const long long srow = job.src_row_stride, drow = job.dst_row_stride;
+        const bool vec_ok = ((reinterpret_cast<uintptr_t>(sbase) | reinterpret_cast<uintptr_t>(dbase) | (uintptr_t)srow | (uintptr_t)drow) & 3) == 0;
+        const int groups = (width + 3) >> 2;
+        const long long total = (long long)job.height * groups;
+        for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < total; t += (long long)gridDim.x * blockDim.x) {
+            const int g = (int)(t % groups);
+            const int y = (int)(t / groups);
+            const uint8_t* s = sbase + (long long)y * srow + 12 * g;
+            uint8_t* d = dbase + (long long)y * drow + 4 * g;
+            const int x0 = 4 * g;
+            if (vec_ok && x0 + 4 <= width) {
+                const uint32_t w0 = *reinterpret_cast<const uint32_t*>(s), w1 = *reinterpret_cast<const uint32_t*>(s + 4),
+                               w2 = *reinterpret_cast<const uint32_t*>(s + 8);
+                // bytes: w0 = B0 G0 R0 B1 | w1 = G1 R1 B2 G2 | w2 = R2 B3 G3 R3   (little endian)
+                *reinterpret_cast<uint32_t*>(d) = sd_bgr2gray_px(w0 & 255, (w0 >> 8) & 255, (w0 >> 16) & 255) |
+                                                  (sd_bgr2gray_px(w0 >> 24, w1 & 255, (w1 >> 8) & 255) << 8) |
+                                                  (sd_bgr2gray_px((w1 >> 16) & 255, w1 >> 24, w2 & 255) << 16) |
+                                                  (sd_bgr2gray_px((w2 >> 8) & 255, (w2 >> 16) & 255, w2 >> 24) << 24);
+            } else {
+                for (int k = 0; k < 4 && x0 + k < width; ++k) d[k] = (uint8_t)sd_bgr2gray_px(s[3 * k], s[3 * k + 1], s[3 * k + 2]);
+            }
         }
     }
 }
 }  // namespace
+
+int sd_bgr2gray_launch(sd_ctx* ctx, cudaStream_t stream, const uint8_t* d_bgr, uint8_t* d_gray, const sd_bgr2gray_job& uniform,
+                       int64_t bgr_image_stride, int64_t gray_image_stride, const sd_bgr2gray_job* d_jobs, int count,
+                       int64_t max_groups)
+{
+    if (count <= 0) return SD_OK;
+    // about 16 CTAs per SM in all: one row of the grid per frame while there are fewer frames than that
+    const int64_t want = 16LL * ctx->sm_count;
+    const int gy = (int)(count < 65535 ? count : 65535);
+    int64_t gx = sd_div_up(max_groups, 256);
+    const int64_t share = sd_div_up(want, gy);
+    gx = gx < share ? gx : share;
+    gx = gx < 1 ? 1 : gx;
+    bgr2gray_kernel<<<dim3((unsigned)gx, (unsigned)gy), 256, 0, stream>>>(d_bgr, d_gray, uniform, bgr_image_stride, gray_image_stride,
+                                                                          d_jobs, count);
+    SD_LAUNCH_CHECK(ctx, "bgr2gray_kernel");
+    return SD_OK;
+}
 
 extern "C" {
 
@@ -849,14 +869,9 @@ int sd_bgr2gray(sd_ctx* ctx, const uint8_t* d_bgr, int width, int height, int64_
     SD_REQUIRE(ctx, count >= 0 && width > 0 && height > 0, "bad argument");
     if (count == 0) return SD_OK;
     SD_REQUIRE(ctx, d_bgr && d_gray && bgr_row_stride >= 3LL * width && gray_row_stride >= width, "bad argument");
-    const int vec_ok = ((reinterpret_cast<uintptr_t>(d_bgr) | reinterpret_cast<uintptr_t>(d_gray) | (uintptr_t)bgr_row_stride |
-                         (uintptr_t)bgr_image_stride | (uintptr_t)gray_row_stride | (uintptr_t)gray_image_stride) & 3) == 0;
-    const long long total = (long long)count * height * ((width + 3) >> 2);
-    const int blocks = (int)(sd_div_up(total, 256) < 16LL * ctx->sm_count ? sd_div_up(total, 256) : 16LL * ctx->sm_count);
-    bgr2gray_kernel<<<blocks, 256, 0, ctx->stream>>>(d_bgr, width, height, bgr_row_stride, bgr_image_stride, count, d_gray,
-                                                     gray_row_stride, gray_image_stride, vec_ok);
-    SD_LAUNCH_CHECK(ctx, "bgr2gray_kernel");
-    return SD_OK;
+    const sd_bgr2gray_job uniform{0, 0, width, height, bgr_row_stride, gray_row_stride};
+    return sd_bgr2gray_launch(ctx, ctx->stream, d_bgr, d_gray, uniform, bgr_image_stride, gray_image_stride, nullptr, count,
+                              (int64_t)height * ((width + 3) >> 2));
 }
 
 }  // extern "C"

@@ -108,6 +108,18 @@ bool sd_syrk_tc_supported(const float* d_S, int64_t lds, int K, int MI, int NJ, 
 
 int sd_check_hog_status(sd_ctx* ctx, const char* what);   // sd_api.cu: synchronises, reports and clears the projection's flags
 
+// one B,G,R frame -> 8UC1 conversion of a bgr2gray_kernel launch (sd_hog.cu); offsets in bytes from the launch's base pointers
+struct sd_bgr2gray_job {
+    int64_t src_offset, dst_offset;
+    int32_t width, height;
+    int64_t src_row_stride, dst_row_stride;
+};
+// cv::cvtColor(BGR2GRAY) of `count` frames in one launch on `stream`: jobs[j] (d_jobs, device) or, with d_jobs == NULL, `uniform`
+// moved by j image strides.  max_groups: the most 4-pixel groups (height x ceil(width / 4)) of any one frame.
+int sd_bgr2gray_launch(sd_ctx* ctx, cudaStream_t stream, const uint8_t* d_bgr, uint8_t* d_gray, const sd_bgr2gray_job& uniform,
+                       int64_t bgr_image_stride, int64_t gray_image_stride, const sd_bgr2gray_job* d_jobs, int count,
+                       int64_t max_groups);
+
 // numerical rank of the symmetric matrix whose upper triangle is in d_G (pivoted Cholesky, sd_rank.cu); rank -1: not computed
 int sd_gram_rank(sd_ctx* ctx, const float* d_G, int64_t ldg, int D, int* rank_out, float* first_pivot, float* last_pivot);
 
@@ -153,6 +165,12 @@ struct sd_eyes_dev {
 int sd_eyes_to_dev(sd_ctx* ctx, const sd_normalisation* n, int num_landmarks, sd_eyes_dev* out);
 
 #ifdef __CUDACC__
+// cv::cvtColor(BGR2GRAY) of one 8-bit pixel, OpenCV >= 3 fixed point (15-bit coefficients; SURVEY.md 8c, pinned against cv2)
+__device__ __forceinline__ uint32_t sd_bgr2gray_px(uint32_t b, uint32_t g, uint32_t r)
+{
+    return (3735u * b + 19235u * g + 9798u * r + (1u << 14)) >> 15;
+}
+
 // Inter-eye distance exactly as helpers.hpp:136-160 evaluates it: eye centres are float sums
 // scaled by the float reciprocal of the count (cv::Vec /= float), the difference is taken in float,
 // squares are accumulated in double (cv::norm NORM_L2) and the root is a double sqrt.

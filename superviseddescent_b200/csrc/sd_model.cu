@@ -180,23 +180,77 @@ int detect_device(sd_ctx* ctx, const sd_model* m, const sd_image_batch* images, 
 // d_roi_miss[roi] and the faces of that ROI are repeated from their full frame, so the result never depends on the ROI
 // heuristic.
 
-// where ROI i is read from: the device-mapped address of its frame's first pixel and the frame's pitch
+// where ROI i is read from: the device-mapped address of its frame's first pixel, the frame's pitch in bytes and its channel
+// count (1: 8UC1, 3: 8UC3 B,G,R)
 struct RoiSource {
     const uint8_t* frame;
     long long row_stride;
+    int channels;
 };
 
+// one 16-byte vector of gray pixels from 48 bytes of interleaved B,G,R (16 pixels), cv::cvtColor(BGR2GRAY) bit for bit
+__device__ __forceinline__ uint4 bgr48_to_gray16(const uint4& a, const uint4& b, const uint4& c)
+{
+    const uint32_t w[12] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w, c.x, c.y, c.z, c.w};
+    uint32_t g[4];
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+        uint32_t v = 0;
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const int p = 3 * (4 * q + k);                // byte of the pixel's B in the 48 bytes
+            const uint32_t bb = (w[p >> 2] >> (8 * (p & 3))) & 255;
+            const uint32_t gg = (w[(p + 1) >> 2] >> (8 * ((p + 1) & 3))) & 255;
+            const uint32_t rr = (w[(p + 2) >> 2] >> (8 * ((p + 2) & 3))) & 255;
+            v |= sd_bgr2gray_px(bb, gg, rr) << (8 * k);
+        }
+        g[q] = v;
+    }
+    return make_uint4(g[0], g[1], g[2], g[3]);
+}
+
+// One CTA per ROI (grid-stride over the ROIs); the instance for CH channels gathers the ROIs of CH-channel frames and skips the
+// others.  A colour ROI is converted to gray as it is gathered: three 16-byte loads (16 B,G,R pixels) per stored 16-byte gray
+// vector, so the packed buffer holds gray ROIs only.  Two instances rather than a branch on the channel count: the colour loop
+// keeps twelve 16-byte loads and their conversion live (80 registers a thread, the gray loop 48), and one kernel holding both
+// loops took 116, a footprint the gray gather would then carry beside the HOG kernels it overlaps.
+template <int CH>
 __global__ void __launch_bounds__(256) roi_gather_kernel(const RoiSource* __restrict__ srcs, const sd_roi* __restrict__ roi, int first,
                                                          int n, uint8_t* __restrict__ dst)
 {
     for (int f = blockIdx.x; f < n; f += gridDim.x) {
-        const sd_roi r = roi[first + f];
         const RoiSource s = srcs[first + f];
+        if (s.channels != CH) continue;
+        const sd_roi r = roi[first + f];
         const long long row_stride = s.row_stride;
-        const uint8_t* src = s.frame + (long long)r.y * row_stride + r.x;
         uint8_t* d = dst + r.offset;
         const int vec_per_row = r.row_stride >> 4;
         const int total = vec_per_row * r.h;
+        if (CH == 3) {
+            // x is a multiple of 16 pixels = 48 bytes: with a 16-byte aligned base and pitch every load is aligned
+            const uint8_t* src = s.frame + (long long)r.y * row_stride + 3LL * r.x;
+            // four vectors (twelve 16-byte reads) in flight per thread before the stores: PCIe read latency is ~1 us
+            for (int i0 = threadIdx.x; i0 < total; i0 += 4 * blockDim.x) {
+                uint4 v[4][3];
+                int row[4], col[4];
+#pragma unroll
+                for (int u = 0; u < 4; ++u) {
+                    const int i = i0 + u * blockDim.x;
+                    row[u] = i / vec_per_row;
+                    col[u] = i - row[u] * vec_per_row;
+                    if (i < total) {
+                        const uint4* p = reinterpret_cast<const uint4*>(src + (long long)row[u] * row_stride) + 3 * col[u];
+                        v[u][0] = p[0]; v[u][1] = p[1]; v[u][2] = p[2];
+                    }
+                }
+#pragma unroll
+                for (int u = 0; u < 4; ++u)
+                    if (i0 + u * blockDim.x < total)
+                        reinterpret_cast<uint4*>(d + (long long)row[u] * r.row_stride)[col[u]] = bgr48_to_gray16(v[u][0], v[u][1], v[u][2]);
+            }
+            continue;
+        }
+        const uint8_t* src = s.frame + (long long)r.y * row_stride + r.x;
         // four independent 16-byte reads in flight per thread before the stores: PCIe read latency is ~1 us
         for (int i0 = threadIdx.x; i0 < total; i0 += 4 * blockDim.x) {
             uint4 v[4];
@@ -232,8 +286,9 @@ __global__ void align_boxes_kernel(const float* __restrict__ mean, int L, const 
 }
 
 // conservative ROI of one face: landmark bounding box of the initialisation, grown by the largest patch
-// half size of the schedule plus a drift allowance, clipped to the frame, x aligned to 16 bytes
-sd_roi face_roi(const sd_model* m, const float* x0, int width, int height, int row_stride)
+// half size of the schedule plus a drift allowance, clipped to the frame, x aligned to 16 pixels; row_pixels = the frame's pitch
+// in pixels (row_stride / channels): rows are never read past it
+sd_roi face_roi(const sd_model* m, const float* x0, int width, int height, int row_pixels)
 {
     const int L = m->num_landmarks;
     float minx = x0[0], maxx = x0[0], miny = x0[L], maxy = x0[L];
@@ -261,7 +316,7 @@ sd_roi face_roi(const sd_model* m, const float* x0, int width, int height, int r
     if (xb <= xa || yb <= ya) { xa = 0; ya = 0; xb = 16 < width ? 16 : width; yb = 1; }   // face entirely outside the frame
     r.x = xa & ~15;
     int w = ((xb - r.x) + 15) & ~15;
-    const int maxw = (row_stride - r.x) & ~15;
+    const int maxw = (row_pixels - r.x) & ~15;
     if (w > maxw) w = maxw;
     r.w = w; r.y = ya; r.h = yb - ya; r.row_stride = w; r.reserved = 0; r.offset = 0;
     return r;
@@ -524,11 +579,13 @@ int sd_detect_batch_device(sd_ctx* ctx, const sd_model* m, const sd_image_batch*
 
 namespace {
 
-// one 8UC1 frame in host memory; d_alias: its device-mapped address when it is pinned with 16-byte aligned base and pitch
+// one frame in host memory (channels 1: 8UC1, 3: 8UC3 B,G,R); d_alias: its device-mapped address when it is pinned with 16-byte
+// aligned base and pitch
 struct HostFrame {
     const uint8_t* h;
     const uint8_t* d_alias;
     int width, height, row_stride;
+    int channels;
 };
 
 int ensure_staging(sd_ctx* ctx, size_t bytes)
@@ -546,7 +603,9 @@ int ensure_staging(sd_ctx* ctx, size_t bytes)
 // Whole-frame route.  Faces [0, count) with frame[k] = frames[fidx[k]], fidx non-decreasing; h_x0 / h_out in that order.
 // Every referenced frame is uploaded once into the double-buffered staging, in chunks of whole frames (~128 MB, or a single
 // frame larger than that) together with all of their faces.  A chunk of equally sized frames is staged as a uniform batch (the
-// HOG kernel's TMA route applies), any other chunk is described by sd_frame records.
+// HOG kernel's TMA route applies), any other chunk is described by sd_frame records.  A colour frame goes up as B,G,R into the
+// chunk's buffer behind its gray frames (the 128 MB count both) and one conversion launch per chunk, on the copy stream before
+// the chunk's stage event, writes its gray frame with a 16-byte aligned pitch.
 int detect_host_full(sd_ctx* ctx, const sd_model* m, const HostFrame* frames, const int* fidx, const float* h_x0, int count, float* h_out)
 {
     const int P = 2 * m->num_landmarks;
@@ -558,30 +617,50 @@ int detect_host_full(sd_ctx* ctx, const sd_model* m, const HostFrame* frames, co
         if (k == 0 || fidx[k] != fidx[k - 1]) uf.push_back(fidx[k]);
         face_u[k] = (int)uf.size() - 1;
     }
-    struct Chunk { int u0, u1, f0, f1; bool uniform; };
+    // gray pitch in the staging buffer: a gray frame keeps its own, a colour frame is converted into 16-byte aligned rows
+    auto gray_pitch = [](const HostFrame& f) { return f.channels == 3 ? (f.width + 15) & ~15 : f.row_stride; };
+    struct Chunk { int u0, u1, f0, f1; bool uniform; size_t bgr_bytes; };
     std::vector<Chunk> chunks;
     std::vector<sd_frame> rec(uf.size());
-    size_t used = 0, stage_need = 0;
+    std::vector<size_t> src_off(uf.size());    // where the frame's host bytes go in the staging buffer (gray: rec offset)
+    size_t used = 0, bgr_used = 0, stage_need = 0;
     for (int u = 0; u < (int)uf.size(); ++u) {
         const HostFrame& f = frames[uf[u]];
-        const size_t padded = ((size_t)f.height * f.row_stride + 15) & ~(size_t)15;
-        if (chunks.empty() || used + padded > cap) { chunks.push_back({u, u, 0, 0, true}); used = 0; }
-        rec[u] = sd_frame{f.width, f.height, f.row_stride, 0, (int64_t)used};
+        const size_t padded = ((size_t)f.height * gray_pitch(f) + 15) & ~(size_t)15;
+        const size_t bgr = f.channels == 3 ? (size_t)f.height * f.row_stride : 0;
+        if (chunks.empty() || used + bgr_used + padded + bgr > cap) { chunks.push_back({u, u, 0, 0, true, 0}); used = 0; bgr_used = 0; }
+        rec[u] = sd_frame{f.width, f.height, gray_pitch(f), 0, (int64_t)used};
+        src_off[u] = bgr_used;                 // relative to the chunk's B,G,R region until the chunk is complete
         used += padded;
+        bgr_used += bgr;
         chunks.back().u1 = u + 1;
+        chunks.back().bgr_bytes = bgr_used;
     }
+    std::vector<sd_bgr2gray_job> jobs;
+    std::vector<int> chunk_job0;               // first conversion job of every chunk
     for (Chunk& c : chunks) {
         const HostFrame& f0 = frames[uf[c.u0]];
         for (int u = c.u0; u < c.u1; ++u) {
             const HostFrame& f = frames[uf[u]];
-            c.uniform = c.uniform && f.width == f0.width && f.height == f0.height && f.row_stride == f0.row_stride;
+            c.uniform = c.uniform && f.width == f0.width && f.height == f0.height && gray_pitch(f) == gray_pitch(f0);
         }
-        const size_t fb = (size_t)f0.height * f0.row_stride;
+        const size_t fb = (size_t)f0.height * gray_pitch(f0);
         if (c.uniform)                          // packed back to back, like one (n, height, row_stride) array
             for (int u = c.u0; u < c.u1; ++u) rec[u].offset = (int64_t)((u - c.u0) * fb);
-        const size_t bytes = (size_t)(rec[c.u1 - 1].offset) + (size_t)frames[uf[c.u1 - 1]].height * frames[uf[c.u1 - 1]].row_stride;
+        const HostFrame& fl = frames[uf[c.u1 - 1]];
+        const size_t gray_bytes = (size_t)(rec[c.u1 - 1].offset) + (size_t)fl.height * gray_pitch(fl);
+        const size_t bgr0 = (gray_bytes + 15) & ~(size_t)15;
+        chunk_job0.push_back((int)jobs.size());
+        for (int u = c.u0; u < c.u1; ++u) {
+            const HostFrame& f = frames[uf[u]];
+            if (f.channels != 3) { src_off[u] = (size_t)rec[u].offset; continue; }
+            src_off[u] += bgr0;
+            jobs.push_back(sd_bgr2gray_job{(int64_t)src_off[u], rec[u].offset, f.width, f.height, f.row_stride, rec[u].row_stride});
+        }
+        const size_t bytes = c.bgr_bytes ? bgr0 + c.bgr_bytes : gray_bytes;
         stage_need = bytes > stage_need ? bytes : stage_need;
     }
+    chunk_job0.push_back((int)jobs.size());
     for (size_t c = 0, k = 0; c < chunks.size(); ++c) {
         chunks[c].f0 = (int)k;
         while (k < (size_t)count && face_u[k] < chunks[c].u1) ++k;
@@ -589,25 +668,29 @@ int detect_host_full(sd_ctx* ctx, const sd_model* m, const HostFrame* frames, co
     }
     int rc = ensure_staging(ctx, stage_need);
     if (rc) return rc;
-    // device tables: landmarks (in, out), frame of every face relative to its chunk, frame records
+    // device tables: landmarks (in, out), frame of every face relative to its chunk, frame records, conversion jobs
     std::vector<int32_t> local(count);
     bool identity = true;                       // one face per frame: no index needed
     for (const Chunk& c : chunks)
         for (int k = c.f0; k < c.f1; ++k) { local[k] = face_u[k] - c.u0; identity = identity && local[k] == k - c.f0; }
     const size_t xbytes = (size_t)count * P * sizeof(float);
     const size_t ibytes = ((size_t)count * sizeof(int32_t) + 15) & ~(size_t)15;
-    unsigned char* tab = (unsigned char*)sd_workspace(ctx, SD_WS_PARTIAL, 2 * xbytes + ibytes + rec.size() * sizeof(sd_frame));
+    const size_t rbytes = rec.size() * sizeof(sd_frame);
+    unsigned char* tab = (unsigned char*)sd_workspace(ctx, SD_WS_PARTIAL, 2 * xbytes + ibytes + rbytes + jobs.size() * sizeof(sd_bgr2gray_job));
     if (!tab) return SD_ERR_CUDA;
     float* d_x = (float*)tab;
     float* d_out = (float*)(tab + xbytes);
     int32_t* d_idx = (int32_t*)(tab + 2 * xbytes);
     sd_frame* d_rec = (sd_frame*)(tab + 2 * xbytes + ibytes);
+    sd_bgr2gray_job* d_jobs = (sd_bgr2gray_job*)(tab + 2 * xbytes + ibytes + rbytes);
     SD_CUDA(ctx, cudaMemcpyAsync(d_x, h_x0, xbytes, cudaMemcpyHostToDevice, ctx->stream));
     if (!identity) SD_CUDA(ctx, cudaMemcpyAsync(d_idx, local.data(), (size_t)count * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
     bool any_mixed = false;
     for (const Chunk& c : chunks) any_mixed = any_mixed || !c.uniform;
-    if (any_mixed) SD_CUDA(ctx, cudaMemcpyAsync(d_rec, rec.data(), rec.size() * sizeof(sd_frame), cudaMemcpyHostToDevice, ctx->stream));
+    if (any_mixed) SD_CUDA(ctx, cudaMemcpyAsync(d_rec, rec.data(), rbytes, cudaMemcpyHostToDevice, ctx->stream));
+    if (!jobs.empty()) SD_CUDA(ctx, cudaMemcpyAsync(d_jobs, jobs.data(), jobs.size() * sizeof(sd_bgr2gray_job), cudaMemcpyHostToDevice, ctx->stream));
     // the copy stream must not run ahead of work already queued on the compute stream that still reads the staging buffers
+    // (the stage_done events also order the table uploads above before the first conversion)
     SD_CUDA(ctx, cudaEventRecord(ctx->stage_done[0], ctx->stream));
     SD_CUDA(ctx, cudaEventRecord(ctx->stage_done[1], ctx->stream));
     int buf = 0;
@@ -621,12 +704,23 @@ int detect_host_full(sd_ctx* ctx, const sd_model* m, const HostFrame* frames, co
             const HostFrame& f = frames[uf[u]];
             const size_t fb = (size_t)f.height * f.row_stride;
             int v = u + 1;
-            while (v < ch.u1 && frames[uf[v]].h == f.h + (v - u) * fb && rec[v].offset == rec[u].offset + (int64_t)((v - u) * fb) &&
-                   frames[uf[v]].row_stride == f.row_stride && frames[uf[v]].height == f.height && frames[uf[v]].width == f.width)
+            while (v < ch.u1 && frames[uf[v]].h == f.h + (v - u) * fb && src_off[v] == src_off[u] + (v - u) * fb &&
+                   frames[uf[v]].row_stride == f.row_stride && frames[uf[v]].height == f.height && frames[uf[v]].width == f.width &&
+                   frames[uf[v]].channels == f.channels)
                 ++v;
-            const size_t bytes = (size_t)(v - u - 1) * fb + (size_t)(f.height - 1) * f.row_stride + f.width;
-            SD_CUDA(ctx, cudaMemcpyAsync(stage + rec[u].offset, f.h, bytes, cudaMemcpyHostToDevice, ctx->copy_stream));
+            const size_t bytes = (size_t)(v - u - 1) * fb + (size_t)(f.height - 1) * f.row_stride + (size_t)f.channels * f.width;
+            SD_CUDA(ctx, cudaMemcpyAsync(stage + src_off[u], f.h, bytes, cudaMemcpyHostToDevice, ctx->copy_stream));
             u = v;
+        }
+        const int j0 = chunk_job0[c], nj = chunk_job0[c + 1] - j0;
+        if (nj > 0) {
+            int64_t max_groups = 0;
+            for (int j = j0; j < j0 + nj; ++j) {
+                const int64_t g = (int64_t)jobs[j].height * ((jobs[j].width + 3) >> 2);
+                max_groups = g > max_groups ? g : max_groups;
+            }
+            rc = sd_bgr2gray_launch(ctx, ctx->copy_stream, stage, stage, sd_bgr2gray_job{}, 0, 0, d_jobs + j0, nj, max_groups);
+            if (rc) return rc;
         }
         SD_CUDA(ctx, cudaEventRecord(ctx->stage_ev[buf], ctx->copy_stream));
         SD_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->stage_ev[buf], 0));
@@ -635,7 +729,7 @@ int detect_host_full(sd_ctx* ctx, const sd_model* m, const HostFrame* frames, co
         ib.count = ch.u1 - ch.u0;
         if (ch.uniform) {
             const HostFrame& f = frames[uf[ch.u0]];
-            ib.width = f.width; ib.height = f.height; ib.row_stride = f.row_stride; ib.image_stride = (int64_t)f.height * f.row_stride;
+            ib.width = f.width; ib.height = f.height; ib.row_stride = gray_pitch(f); ib.image_stride = (int64_t)f.height * gray_pitch(f);
         } else {
             ib.d_frames = d_rec + ch.u0;
         }
@@ -670,7 +764,7 @@ int detect_host_roi(sd_ctx* ctx, const sd_model* m, const HostFrame* frames, con
         const HostFrame& f = frames[fidx[k0]];
         const int g0 = (int)groups.size();
         for (int k = k0; k < k1; ++k) {
-            sd_roi r = face_roi(m, h_x0 + (size_t)k * P, f.width, f.height, f.row_stride);
+            sd_roi r = face_roi(m, h_x0 + (size_t)k * P, f.width, f.height, f.row_stride / f.channels);
             int g = -1;
             for (int j = g0; j < (int)groups.size() && g < 0; ++j) if (roi_intersect(groups[j], r)) g = j;
             if (g < 0) { groups.push_back(r); group_frame.push_back(fidx[k0]); face_group[k] = (int)groups.size() - 1; continue; }
@@ -721,6 +815,7 @@ int detect_host_roi(sd_ctx* ctx, const sd_model* m, const HostFrame* frames, con
     for (int g = 0; g < G; ++g) gface0[g + 1] += gface0[g];
     std::vector<int32_t> local(count);                     // face -> group, relative to the chunk's first group
     std::vector<int> chunk_first;                          // groups
+    std::vector<char> chunk_gray, chunk_colour;            // the chunk holds ROIs of gray / colour frames
     std::vector<RoiSource> srcs(G);
     bool same_size = true;
     size_t used = 0;
@@ -730,10 +825,11 @@ int detect_host_roi(sd_ctx* ctx, const sd_model* m, const HostFrame* frames, con
         const size_t bytes = (size_t)groups[g].row_stride * groups[g].h;
         if (bytes > chunk_cap)                                // a face window larger than a staging buffer: whole-frame route
             return detect_host_full(ctx, m, frames, fidx, h_x0, count, h_out);
-        if (chunk_first.empty() || used + bytes > chunk_cap) { chunk_first.push_back(g); used = 0; }
+        if (chunk_first.empty() || used + bytes > chunk_cap) { chunk_first.push_back(g); chunk_gray.push_back(0); chunk_colour.push_back(0); used = 0; }
         groups[g].offset = (int64_t)used;
         used += bytes;
-        srcs[g] = RoiSource{f.d_alias, (long long)f.row_stride};
+        srcs[g] = RoiSource{f.d_alias, (long long)f.row_stride, f.channels};
+        (f.channels == 3 ? chunk_colour : chunk_gray).back() = 1;
         for (int k = gface0[g]; k < gface0[g + 1]; ++k) local[k] = g - chunk_first.back();
     }
     chunk_first.push_back(G);
@@ -772,8 +868,14 @@ int detect_host_roi(sd_ctx* ctx, const sd_model* m, const HostFrame* frames, con
         const int first = chunk_first[c], n = chunk_first[c + 1] - first;
         SD_CUDA(ctx, cudaStreamWaitEvent(ctx->copy_stream, ctx->stage_done[buf], 0));   // also orders the table uploads before the first gather
         const int blocks = n < 8 * ctx->sm_count ? n : 8 * ctx->sm_count;
-        roi_gather_kernel<<<blocks, 256, 0, ctx->copy_stream>>>(d_src, d_roi, first, n, (uint8_t*)ctx->d_stage[buf]);
-        SD_LAUNCH_CHECK(ctx, "roi_gather_kernel");
+        if (chunk_gray[c]) {
+            roi_gather_kernel<1><<<blocks, 256, 0, ctx->copy_stream>>>(d_src, d_roi, first, n, (uint8_t*)ctx->d_stage[buf]);
+            SD_LAUNCH_CHECK(ctx, "roi_gather_kernel");
+        }
+        if (chunk_colour[c]) {
+            roi_gather_kernel<3><<<blocks, 256, 0, ctx->copy_stream>>>(d_src, d_roi, first, n, (uint8_t*)ctx->d_stage[buf]);
+            SD_LAUNCH_CHECK(ctx, "roi_gather_kernel");
+        }
         SD_CUDA(ctx, cudaEventRecord(ctx->stage_ev[buf], ctx->copy_stream));
         SD_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->stage_ev[buf], 0));
         sd_image_batch ib{};
@@ -806,10 +908,11 @@ int detect_host_roi(sd_ctx* ctx, const sd_model* m, const HostFrame* frames, con
     return SD_OK;
 }
 
-// detect(image, facebox) for count faces; face i in frames[frame_index ? frame_index[i] : i] (indices already validated).
-// Faces are taken frame by frame (stable), their initial landmarks aligned on the host (model.hpp:135).
+// detect(image, facebox) (h_boxes) or detect(image, initialisation) (h_x0, row stride ldx floats) for count faces; face i in
+// frames[frame_index ? frame_index[i] : i] (indices already validated).  Faces are taken frame by frame (stable), their
+// initial landmarks aligned on the host (model.hpp:135) or copied.
 int detect_host(sd_ctx* ctx, const sd_model* m, const std::vector<HostFrame>& frames, const int32_t* frame_index, const int32_t* h_boxes,
-                int count, float* h_landmarks, bool roi)
+                const float* h_x0, int64_t ldx, int count, float* h_landmarks, bool roi)
 {
     const int L = m->num_landmarks, P = 2 * L;
     const int F = (int)frames.size();
@@ -827,8 +930,12 @@ int detect_host(sd_ctx* ctx, const sd_model* m, const std::vector<HostFrame>& fr
     for (int k = 0; k < count && identity; ++k) identity = order[k] == k;
     std::vector<float> x0((size_t)count * P), sorted_out;
     for (int k = 0; k < count; ++k) {
-        const int32_t* b = h_boxes + 4 * (size_t)order[k];
-        sd_align_mean(m->mean.data(), L, b[0], b[1], b[2], b[3], 1.f, 1.f, 0.f, 0.f, &x0[(size_t)k * P]);
+        if (h_boxes) {
+            const int32_t* b = h_boxes + 4 * (size_t)order[k];
+            sd_align_mean(m->mean.data(), L, b[0], b[1], b[2], b[3], 1.f, 1.f, 0.f, 0.f, &x0[(size_t)k * P]);
+        } else {
+            memcpy(&x0[(size_t)k * P], h_x0 + (size_t)order[k] * ldx, P * sizeof(float));
+        }
     }
     float* out = h_landmarks;
     if (!identity) { sorted_out.resize((size_t)count * P); out = sorted_out.data(); }
@@ -848,6 +955,39 @@ const uint8_t* mapped_alias(const void* h)
     return attr.type == cudaMemoryTypeHost ? (const uint8_t*)attr.devicePointer : nullptr;
 }
 
+// the frames of an sd_detect_faces_host(_init) call, checked: every frame index, and the size, pitch and channel count of every
+// referenced frame (frames without faces are never read).  roi: every referenced frame is pinned, device-mapped and aligned.
+int host_frames(sd_ctx* ctx, const char* fn, const sd_host_frame* h_frames, int num_frames, const int32_t* h_frame_index, int count,
+                std::vector<HostFrame>& frames, bool& roi)
+{
+    std::vector<char> used(num_frames, 0);
+    for (int i = 0; i < count; ++i) {
+        if (h_frame_index[i] < 0 || h_frame_index[i] >= num_frames)
+            return sd_fail(ctx, SD_ERR_INVALID, "%s: face %d: frame index %d is not in [0, %d)", fn, i, h_frame_index[i], num_frames);
+        used[h_frame_index[i]] = 1;
+    }
+    frames.assign(num_frames, HostFrame{nullptr, nullptr, 0, 0, 0, 1});
+    for (int f = 0; f < num_frames; ++f) {
+        if (!used[f]) continue;
+        const sd_host_frame& hf = h_frames[f];
+        const int channels = hf.channels == 0 ? 1 : hf.channels;
+        if (channels != 1 && channels != 3)
+            return sd_fail(ctx, SD_ERR_INVALID, "%s: frame %d: %d channels (1 = gray or 3 = B,G,R)", fn, f, hf.channels);
+        if (!hf.h_data || hf.width <= 0 || hf.height <= 0 || (int64_t)hf.row_stride < (int64_t)channels * hf.width)
+            return sd_fail(ctx, SD_ERR_INVALID, "%s: frame %d: bad data pointer or size", fn, f);
+        frames[f] = HostFrame{hf.h_data, nullptr, hf.width, hf.height, hf.row_stride, channels};
+    }
+    // ROI route when the frames are in pinned, device-mapped host memory with 16-byte aligned rows
+    roi = true;
+    for (int f = 0; f < num_frames && roi; ++f) {
+        if (!used[f]) continue;
+        const uint8_t* alias = mapped_alias(frames[f].h);
+        roi = alias && ((reinterpret_cast<uintptr_t>(alias) | (uintptr_t)frames[f].row_stride) & 15) == 0;
+        frames[f].d_alias = alias;
+    }
+    return SD_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -864,8 +1004,8 @@ int sd_detect_batch_host(sd_ctx* ctx, const sd_model* m, const uint8_t* h_images
     const bool aligned = alias && ((reinterpret_cast<uintptr_t>(alias) | (uintptr_t)row_stride | (uintptr_t)frame_bytes) & 15) == 0;
     std::vector<HostFrame> frames(count);
     for (int i = 0; i < count; ++i)
-        frames[i] = HostFrame{h_images + i * frame_bytes, aligned ? alias + i * frame_bytes : nullptr, width, height, row_stride};
-    return detect_host(ctx, m, frames, nullptr, h_boxes, count, h_landmarks, aligned);
+        frames[i] = HostFrame{h_images + i * frame_bytes, aligned ? alias + i * frame_bytes : nullptr, width, height, row_stride, 1};
+    return detect_host(ctx, m, frames, nullptr, h_boxes, nullptr, 0, count, h_landmarks, aligned);
 }
 
 int sd_model_align_boxes(sd_ctx* ctx, const sd_model* m, const int32_t* d_boxes, int count, float* d_x0, int64_t ldx)
@@ -901,25 +1041,26 @@ int sd_detect_faces_host(sd_ctx* ctx, const sd_model* m, const sd_host_frame* h_
     SD_REQUIRE(ctx, m && count >= 0 && num_frames >= 0, "bad argument");
     if (count == 0) return SD_OK;
     SD_REQUIRE(ctx, h_frames && h_frame_index && h_boxes && h_landmarks && num_frames >= 1, "bad argument");
-    std::vector<char> used(num_frames, 0);
-    for (int i = 0; i < count; ++i) {
-        if (h_frame_index[i] < 0 || h_frame_index[i] >= num_frames)
-            return sd_fail(ctx, SD_ERR_INVALID, "%s: face %d: frame index %d is not in [0, %d)", __func__, i, h_frame_index[i], num_frames);
-        used[h_frame_index[i]] = 1;
-    }
-    // frames without faces are never read, so only the referenced ones are checked
-    std::vector<HostFrame> frames(num_frames, HostFrame{nullptr, nullptr, 0, 0, 0});
-    bool roi = true;
-    for (int f = 0; f < num_frames; ++f) {
-        if (!used[f]) continue;
-        const sd_host_frame& hf = h_frames[f];
-        if (!hf.h_data || hf.width <= 0 || hf.height <= 0 || hf.row_stride < hf.width)
-            return sd_fail(ctx, SD_ERR_INVALID, "%s: frame %d: bad data pointer or size", __func__, f);
-        const uint8_t* alias = roi ? mapped_alias(hf.h_data) : nullptr;
-        roi = alias && ((reinterpret_cast<uintptr_t>(alias) | (uintptr_t)hf.row_stride) & 15) == 0;
-        frames[f] = HostFrame{hf.h_data, alias, hf.width, hf.height, hf.row_stride};
-    }
-    return detect_host(ctx, m, frames, h_frame_index, h_boxes, count, h_landmarks, roi);
+    std::vector<HostFrame> frames;
+    bool roi = false;
+    const int rc = host_frames(ctx, __func__, h_frames, num_frames, h_frame_index, count, frames, roi);
+    if (rc) return rc;
+    return detect_host(ctx, m, frames, h_frame_index, h_boxes, nullptr, 0, count, h_landmarks, roi);
+}
+
+int sd_detect_faces_host_init(sd_ctx* ctx, const sd_model* m, const sd_host_frame* h_frames, int num_frames, const int32_t* h_frame_index,
+                              const float* h_x0, int64_t ldx, int count, float* h_landmarks)
+{
+    if (!ctx) return SD_ERR_INVALID;
+    SD_REQUIRE(ctx, m && count >= 0 && num_frames >= 0, "bad argument");
+    if (count == 0) return SD_OK;
+    SD_REQUIRE(ctx, h_frames && h_frame_index && h_x0 && h_landmarks && num_frames >= 1 && ldx >= 2 * (int64_t)m->num_landmarks,
+               "bad argument");
+    std::vector<HostFrame> frames;
+    bool roi = false;
+    const int rc = host_frames(ctx, __func__, h_frames, num_frames, h_frame_index, count, frames, roi);
+    if (rc) return rc;
+    return detect_host(ctx, m, frames, h_frame_index, nullptr, h_x0, ldx, count, h_landmarks, roi);
 }
 
 }  // extern "C"

@@ -1,6 +1,7 @@
 // B200 drop-in for include/rcr/model.hpp: align_mean (:64-76), InterEyeDistanceNormalisation (:84-116),
 // detection_model (:122-183) and load/save_detection_model (:192-219).  detect() runs the whole cascade
-// on the GPU through sd_detect_batch_host; the file format is byte compatible with the reference's
+// on the GPU through sd_detect_batch_host / sd_detect_faces_host(_init), reading host frames in place (8UC1, or 8UC3 B,G,R
+// converted on the device); the file format is byte compatible with the reference's
 // cereal archives (face_landmarks_model_rcr_22.bin loads unchanged).
 #pragma once
 
@@ -100,16 +101,12 @@ public:
     // Run the model from a landmark initialisation, e.g. the previous frame (model.hpp:147-157)
     LandmarkCollection<cv::Vec2f> detect(cv::Mat image, cv::Mat initialisation)
     {
-        sd_ctx* ctx = sd_b200::context();
-        const cv::Mat& gray = image;               // size only; colour frames are converted on the device
-        const size_t frame = static_cast<size_t>(gray.cols) * gray.rows;
-        sd_b200::DeviceBuffer dimg(frame), dx, dout(static_cast<size_t>(initialisation.cols) * sizeof(float)), bgr;
-        upload_gray(ctx, image, dimg.as<unsigned char>(), bgr);
-        sd_b200::upload(initialisation, dx, initialisation.cols);
-        sd_image_batch ib{};
-        ib.d_data = dimg.as<unsigned char>(); ib.width = gray.cols; ib.height = gray.rows; ib.row_stride = gray.cols; ib.image_stride = static_cast<int64_t>(frame); ib.count = 1;
-        sd_b200::check(ctx, sd_detect_batch_device(ctx, handle.get(), &ib, dx.as<float>(), 1, dout.as<float>()), "sd_detect_batch_device");
-        return to_landmark_collection(sd_b200::download(dout.as<float>(), 1, initialisation.cols, initialisation.cols), landmark_ids);
+        const cv::Mat x0 = initialisation.isContinuous() ? initialisation : initialisation.clone();
+        if (x0.rows * x0.cols != 2 * sd_model_num_landmarks(handle.get())) throw std::runtime_error("detect: the initialisation needs 2L values");
+        const std::vector<float> lms = detect_host(std::vector<cv::Mat>{image}, std::vector<int32_t>{0}, nullptr, x0.ptr<float>(0));
+        cv::Mat row(1, static_cast<int>(lms.size()), CV_32FC1);
+        std::memcpy(row.ptr<float>(0), lms.data(), sizeof(float) * lms.size());
+        return to_landmark_collection(row, landmark_ids);
     }
 
     // Batched detect: equally sized frames, one face box each; returns one 1 x 2L row per frame.
@@ -121,39 +118,27 @@ public:
         const int w = images[0].cols, h = images[0].rows;
         const int P = 2 * sd_model_num_landmarks(handle.get());
         bool colour = false;
+        std::vector<int32_t> boxes(static_cast<size_t>(n) * 4);
         for (int i = 0; i < n; ++i) {
             if (images[i].cols != w || images[i].rows != h) throw std::runtime_error("detect: the batched path needs equally sized images");
             colour = colour || images[i].channels() == 3;
-        }
-        if (colour) {
-            // colour frames: upload B,G,R, convert on the device (sd_bgr2gray), start from the aligned mean, stay on the device
-            const size_t frame = static_cast<size_t>(w) * h;
-            sd_b200::DeviceBuffer dimg(frame * n), dx(static_cast<size_t>(n) * P * sizeof(float)), dout(static_cast<size_t>(n) * P * sizeof(float)), bgr;
-            std::vector<float> x0(static_cast<size_t>(n) * P);
-            const cv::Mat mean = get_mean();
-            for (int i = 0; i < n; ++i) {
-                upload_gray(ctx, images[i], dimg.as<unsigned char>() + i * frame, bgr);
-                sd_b200::check(ctx, sd_align_mean(mean.ptr<float>(0), P / 2, faceboxes[i].x, faceboxes[i].y, faceboxes[i].width, faceboxes[i].height,
-                                                  1.f, 1.f, 0.f, 0.f, &x0[static_cast<size_t>(i) * P]), "sd_align_mean");
-            }
-            sd_b200::check(ctx, sd_memcpy_h2d(ctx, dx.as<float>(), x0.data(), x0.size() * sizeof(float)), "detect");
-            sd_image_batch ib{};
-            ib.d_data = dimg.as<unsigned char>(); ib.width = w; ib.height = h; ib.row_stride = w; ib.image_stride = static_cast<int64_t>(frame); ib.count = n;
-            sd_b200::check(ctx, sd_detect_batch_device(ctx, handle.get(), &ib, dx.as<float>(), n, dout.as<float>()), "sd_detect_batch_device");
-            const cv::Mat all = sd_b200::download(dout.as<float>(), n, P, P);
-            std::vector<cv::Mat> rows;
-            for (int i = 0; i < n; ++i) rows.push_back(all.row(i).clone());
-            return rows;
-        }
-        std::vector<unsigned char> frames(static_cast<size_t>(n) * w * h);
-        std::vector<int32_t> boxes(static_cast<size_t>(n) * 4);
-        for (int i = 0; i < n; ++i) {
-            const cv::Mat& g = images[i];
-            for (int y = 0; y < h; ++y) std::memcpy(&frames[(static_cast<size_t>(i) * h + y) * w], g.ptr<unsigned char>(y), w);
             boxes[4 * i] = faceboxes[i].x; boxes[4 * i + 1] = faceboxes[i].y; boxes[4 * i + 2] = faceboxes[i].width; boxes[4 * i + 3] = faceboxes[i].height;
         }
-        std::vector<float> lms(static_cast<size_t>(n) * P);
-        sd_b200::check(ctx, sd_detect_batch_host(ctx, handle.get(), frames.data(), n, w, h, w, boxes.data(), lms.data()), "sd_detect_batch_host");
+        std::vector<float> lms;
+        if (colour) {
+            // colour frames (8UC3 B,G,R) are read in place and converted to gray on the device (sd_detect_faces_host)
+            std::vector<int32_t> index(n);
+            for (int i = 0; i < n; ++i) index[i] = i;
+            lms = detect_host(images, index, boxes.data(), nullptr);
+        } else {
+            std::vector<unsigned char> frames(static_cast<size_t>(n) * w * h);
+            for (int i = 0; i < n; ++i) {
+                const cv::Mat& g = images[i];
+                for (int y = 0; y < h; ++y) std::memcpy(&frames[(static_cast<size_t>(i) * h + y) * w], g.ptr<unsigned char>(y), w);
+            }
+            lms.resize(static_cast<size_t>(n) * P);
+            sd_b200::check(ctx, sd_detect_batch_host(ctx, handle.get(), frames.data(), n, w, h, w, boxes.data(), lms.data()), "sd_detect_batch_host");
+        }
         std::vector<cv::Mat> out;
         for (int i = 0; i < n; ++i) {
             cv::Mat row(1, P, CV_32FC1);
@@ -164,71 +149,36 @@ public:
     }
 
     // Several faces per frame, frames of any sizes (the box list a face detector such as detectMultiScale returns for each
-    // frame): result[i][j] holds the landmarks of faceboxes[i][j] in images[i].  Gray frames are read in place through their
-    // own row pointers (sd_detect_faces_host); if any frame with faces is colour, the frames go to the device, are converted
-    // there (sd_bgr2gray) and the boxes are aligned there (sd_model_align_boxes, sd_detect_faces_device).
+    // frame): result[i][j] holds the landmarks of faceboxes[i][j] in images[i].  Frames, gray or colour (8UC3 B,G,R), are read
+    // in place through their own row pointers (sd_detect_faces_host).
     std::vector<std::vector<LandmarkCollection<cv::Vec2f>>> detect(const std::vector<cv::Mat>& images, const std::vector<std::vector<cv::Rect>>& faceboxes)
     {
         if (images.size() != faceboxes.size()) throw std::runtime_error("detect: images / faceboxes size mismatch");
-        sd_ctx* ctx = sd_b200::context();
-        const int P = 2 * sd_model_num_landmarks(handle.get());
         std::vector<int32_t> index, boxes;
-        bool colour = false;
-        for (size_t i = 0; i < images.size(); ++i) {
-            if (faceboxes[i].empty()) continue;
-            if (images[i].empty()) throw std::runtime_error("detect: empty image with face boxes");
-            colour = colour || images[i].channels() == 3;
+        for (size_t i = 0; i < images.size(); ++i)
             for (const cv::Rect& b : faceboxes[i]) {
                 index.push_back(static_cast<int32_t>(i));
                 boxes.push_back(b.x); boxes.push_back(b.y); boxes.push_back(b.width); boxes.push_back(b.height);
             }
-        }
-        const int count = static_cast<int>(index.size());
-        std::vector<float> lms(static_cast<size_t>(count) * P);
-        if (count > 0 && !colour) {
-            std::vector<sd_host_frame> frames(images.size());
-            for (size_t i = 0; i < images.size(); ++i)
-                if (!faceboxes[i].empty())
-                    frames[i] = sd_host_frame{images[i].ptr<unsigned char>(0), images[i].cols, images[i].rows, static_cast<int32_t>(images[i].step()), 0};
-            sd_b200::check(ctx, sd_detect_faces_host(ctx, handle.get(), frames.data(), static_cast<int>(frames.size()), index.data(), boxes.data(), count,
-                                                     lms.data()), "sd_detect_faces_host");
-        } else if (count > 0) {
-            // the frames with faces, packed on the device as 8UC1 with 16-byte aligned rows, one sd_frame record each
-            std::vector<sd_frame> rec;
-            std::vector<int32_t> local(images.size(), -1);
-            int64_t off = 0;
-            for (size_t i = 0; i < images.size(); ++i) {
-                if (faceboxes[i].empty()) continue;
-                const int w = images[i].cols, h = images[i].rows, stride = (w + 15) / 16 * 16;
-                local[i] = static_cast<int32_t>(rec.size());
-                rec.push_back(sd_frame{w, h, stride, 0, off});
-                off += static_cast<int64_t>(h) * stride;
-            }
-            for (int32_t& f : index) f = local[f];
-            sd_b200::DeviceBuffer dimg(static_cast<size_t>(off)), drec(rec.size() * sizeof(sd_frame)), didx(index.size() * sizeof(int32_t)),
-                dboxes(boxes.size() * sizeof(int32_t)), dx(lms.size() * sizeof(float)), dout(lms.size() * sizeof(float)), bgr;
-            for (size_t i = 0; i < images.size(); ++i)
-                if (local[i] >= 0) upload_gray(ctx, images[i], dimg.as<unsigned char>() + rec[local[i]].offset, bgr, rec[local[i]].row_stride);
-            sd_b200::check(ctx, sd_memcpy_h2d(ctx, drec.as<sd_frame>(), rec.data(), rec.size() * sizeof(sd_frame)), "detect");
-            sd_b200::check(ctx, sd_memcpy_h2d(ctx, didx.as<int32_t>(), index.data(), index.size() * sizeof(int32_t)), "detect");
-            sd_b200::check(ctx, sd_memcpy_h2d(ctx, dboxes.as<int32_t>(), boxes.data(), boxes.size() * sizeof(int32_t)), "detect");
-            sd_b200::check(ctx, sd_model_align_boxes(ctx, handle.get(), dboxes.as<int32_t>(), count, dx.as<float>(), P), "sd_model_align_boxes");
-            sd_image_batch ib{};
-            ib.d_data = dimg.as<unsigned char>(); ib.count = static_cast<int32_t>(rec.size()); ib.d_frames = drec.as<sd_frame>();
-            sd_b200::check(ctx, sd_detect_faces_device(ctx, handle.get(), &ib, didx.as<int32_t>(), dx.as<float>(), count, dout.as<float>()),
-                           "sd_detect_faces_device");
-            const cv::Mat all = sd_b200::download(dout.as<float>(), count, P, P);
-            std::memcpy(lms.data(), all.ptr<float>(0), lms.size() * sizeof(float));
-        }
-        std::vector<std::vector<LandmarkCollection<cv::Vec2f>>> out(images.size());
-        size_t k = 0;
+        return per_frame(images.size(), faceboxes, detect_host(images, index, boxes.data(), nullptr));
+    }
+
+    // Several tracked faces per frame (detect(image, initialisation) for each): result[i][j] holds the landmarks of the face
+    // that starts from initialisations[i][j] (1 x 2L, e.g. its landmarks in the previous frame) in images[i].
+    std::vector<std::vector<LandmarkCollection<cv::Vec2f>>> detect(const std::vector<cv::Mat>& images, const std::vector<std::vector<cv::Mat>>& initialisations)
+    {
+        if (images.size() != initialisations.size()) throw std::runtime_error("detect: images / initialisations size mismatch");
+        const size_t P = 2 * static_cast<size_t>(sd_model_num_landmarks(handle.get()));
+        std::vector<int32_t> index;
+        std::vector<float> x0;
         for (size_t i = 0; i < images.size(); ++i)
-            for (size_t j = 0; j < faceboxes[i].size(); ++j, ++k) {
-                cv::Mat row(1, P, CV_32FC1);
-                std::memcpy(row.ptr<float>(0), &lms[k * P], sizeof(float) * P);
-                out[i].push_back(to_landmark_collection(row, landmark_ids));
+            for (const cv::Mat& init : initialisations[i]) {
+                if (static_cast<size_t>(init.rows) * init.cols != P) throw std::runtime_error("detect: an initialisation needs 2L values");
+                const cv::Mat row = init.isContinuous() ? init : init.clone();
+                index.push_back(static_cast<int32_t>(i));
+                x0.insert(x0.end(), row.ptr<float>(0), row.ptr<float>(0) + P);
             }
-        return out;
+        return per_frame(images.size(), initialisations, detect_host(images, index, nullptr, x0.data()));
     }
 
     cv::Mat get_mean()
@@ -242,23 +192,45 @@ public:
 
 private:
     friend detection_model load_detection_model(std::string filename);
-    // frame -> device as 8UC1 with rows dst_stride bytes apart (0: packed); colour frames go up as B,G,R and are converted
-    // there (cv::cvtColor BGR2GRAY of adaptive_vlhog.hpp:115-117 == sd_bgr2gray)
-    static void upload_gray(sd_ctx* ctx, const cv::Mat& image, unsigned char* d_dst, sd_b200::DeviceBuffer& bgr, int dst_stride = 0)
+    // Every face of `index` (the frame of each face) through sd_detect_faces_host (boxes: 4 per face) or sd_detect_faces_host_init
+    // (x0: 2L per face); returns count x 2L.  Frames are read in place through their own pointer and pitch; colour frames (8UC3
+    // B,G,R) are converted on the device as cv::cvtColor(BGR2GRAY) of adaptive_vlhog.hpp:115-117 would.
+    std::vector<float> detect_host(const std::vector<cv::Mat>& images, const std::vector<int32_t>& index, const int32_t* boxes, const float* x0)
     {
-        const int w = image.cols, h = image.rows;
-        const size_t frame = static_cast<size_t>(w) * h;
-        const size_t ds = dst_stride > 0 ? static_cast<size_t>(dst_stride) : static_cast<size_t>(w);
-        if (image.channels() == 3) {
-            bgr.allocate(3 * frame);
-            for (int y = 0; y < h; ++y)
-                sd_b200::check(ctx, sd_memcpy_h2d(ctx, bgr.as<unsigned char>() + static_cast<size_t>(y) * 3 * w, image.ptr<unsigned char>(y), 3 * static_cast<size_t>(w)), "detect upload");
-            sd_b200::check(ctx, sd_bgr2gray(ctx, bgr.as<unsigned char>(), w, h, 3 * static_cast<int64_t>(w), 3 * static_cast<int64_t>(frame), 1, d_dst,
-                                            static_cast<int64_t>(ds), static_cast<int64_t>(ds * h)), "sd_bgr2gray");
-        } else {
-            for (int y = 0; y < h; ++y)
-                sd_b200::check(ctx, sd_memcpy_h2d(ctx, d_dst + static_cast<size_t>(y) * ds, image.ptr<unsigned char>(y), w), "detect upload");
+        sd_ctx* ctx = sd_b200::context();
+        const int P = 2 * sd_model_num_landmarks(handle.get());
+        const int count = static_cast<int>(index.size());
+        std::vector<float> lms(static_cast<size_t>(count) * P);
+        if (count == 0) return lms;
+        std::vector<sd_host_frame> frames(images.size(), sd_host_frame{nullptr, 0, 0, 0, 0});
+        for (int32_t i : index) {
+            const cv::Mat& im = images[i];
+            if (im.empty()) throw std::runtime_error("detect: empty image with faces");
+            frames[i] = sd_host_frame{im.ptr<unsigned char>(0), im.cols, im.rows, static_cast<int32_t>(im.step()), im.channels()};
         }
+        if (boxes)
+            sd_b200::check(ctx, sd_detect_faces_host(ctx, handle.get(), frames.data(), static_cast<int>(frames.size()), index.data(), boxes, count,
+                                                     lms.data()), "sd_detect_faces_host");
+        else
+            sd_b200::check(ctx, sd_detect_faces_host_init(ctx, handle.get(), frames.data(), static_cast<int>(frames.size()), index.data(), x0, P,
+                                                          count, lms.data()), "sd_detect_faces_host_init");
+        return lms;
+    }
+
+    // count x 2L landmark rows, faces in frame order -> one list of landmark collections per frame
+    template <class PerFrame>
+    std::vector<std::vector<LandmarkCollection<cv::Vec2f>>> per_frame(size_t num_frames, const std::vector<PerFrame>& faces, const std::vector<float>& lms)
+    {
+        const size_t P = 2 * static_cast<size_t>(sd_model_num_landmarks(handle.get()));
+        std::vector<std::vector<LandmarkCollection<cv::Vec2f>>> out(num_frames);
+        size_t k = 0;
+        for (size_t i = 0; i < num_frames; ++i)
+            for (size_t j = 0; j < faces[i].size(); ++j, ++k) {
+                cv::Mat row(1, static_cast<int>(P), CV_32FC1);
+                std::memcpy(row.ptr<float>(0), &lms[k * P], sizeof(float) * P);
+                out[i].push_back(to_landmark_collection(row, landmark_ids));
+            }
+        return out;
     }
 
     std::shared_ptr<sd_model> handle;

@@ -1,11 +1,14 @@
 """Faces/s of detection with several faces per frame (detection_model.detect_faces / detect_faces_device) against the same faces
 through the one-face-per-frame calls on frames duplicated once per face.
 
-    python tools/bench_faces.py [--frames 1024] [--reps 5] [--out DIR]
+    python tools/bench_faces.py [--frames 1024] [--reps 5] [--cases a,b,c,d] [--out DIR]
 
 (a) device-resident 640x480 frames with 1, 4 and 16 faces each: detect_faces_device vs detect_batch_device on duplicated frames
 (b) the same from pinned and from pageable host frames: detect_faces vs detect_batch (sd_detect_batch_host) on duplicated frames
 (c) frames of mixed sizes vs equally sized 640x480 frames with the same number of faces, on each route
+(d) colour 640x480 B,G,R host frames (independent B, G and R planes) with 1, 4 and 16 faces each, pinned and pageable:
+    detect_faces, which converts only each face's neighbourhood (pinned) or each frame once on the device (pageable), against
+    the route without it, built from public calls: bgr2gray of the whole host batch + align_boxes + detect_faces_device
 
 Prints the card's name and power limit first, then one JSON line per measurement; with --out also writes them to DIR/bench_faces.json.
 Every pair of rates is checked to give bit-identical landmarks.
@@ -70,6 +73,7 @@ def main():
     ap.add_argument("--frames", type=int, default=1024)
     ap.add_argument("--reps", type=int, default=5)
     ap.add_argument("--faces", default="1,4,16")
+    ap.add_argument("--cases", default="a,b,c,d")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     if not torch.cuda.is_available():
@@ -88,10 +92,15 @@ def main():
         print(json.dumps(kw), flush=True)
 
     n = args.frames
+    cases = set(args.cases.split(","))
+    if "d" in cases:
+        colour_case(m, sd, n, args, gen, rng, dev, report)
+    if not cases & {"a", "b", "c"}:
+        return finish(args, results)
     frames = torch.stack([smooth_frame(480, 640, gen, dev) for _ in range(n)])
     frames_pinned = frames.cpu().pin_memory()
     frames_np = frames.cpu().numpy()
-    for k in [int(v) for v in args.faces.split(",")]:
+    for k in [int(v) for v in args.faces.split(",")] if cases & {"a", "b"} else []:
         boxes = np.array([b for _ in range(n) for b in grid_boxes(480, 640, k, rng)], dtype=np.int32)
         index = np.repeat(np.arange(n, dtype=np.int32), k)
         faces = len(boxes)
@@ -123,6 +132,8 @@ def main():
         report(case="b", route="pageable", faces_per_frame=k, faces=faces, faces_per_s=faces / t_new, duplicated_faces_per_s=faces / t_dup)
         del dup_np
 
+    if "c" not in cases:
+        return finish(args, results)
     # (c) mixed sizes against equally sized frames, 4 faces per frame
     k = 4
     sizes = [MIXED_SIZES[i % len(MIXED_SIZES)] for i in range(n)]
@@ -167,6 +178,29 @@ def main():
         t_u, _ = timed(fu, args.reps)
         report(case="c", route=route, faces_per_frame=k, faces=len(mboxes), mixed_faces_per_s=len(mboxes) / t_m, uniform_faces_per_s=len(uboxes) / t_u,
                mixed_sizes=sorted({f"{w}x{h}" for h, w in sizes}))
+    finish(args, results)
+
+
+def colour_case(m, sd, n, args, gen, rng, dev, report):
+    """(d): colour host frames through detect_faces against bgr2gray of the whole batch + align_boxes + detect_faces_device."""
+    frames = torch.stack([torch.stack([smooth_frame(480, 640, gen, dev) for _ in range(3)], dim=2) for _ in range(n)])
+    frames_pinned = frames.cpu().pin_memory()
+    frames_np = frames.cpu().numpy()
+    del frames
+    for k in [int(v) for v in args.faces.split(",")]:
+        boxes = np.array([b for _ in range(n) for b in grid_boxes(480, 640, k, rng)], dtype=np.int32)
+        index = np.repeat(np.arange(n, dtype=np.int32), k)
+        for route, host in (("pinned", frames_pinned), ("pageable", frames_np)):
+            fb = m.ctx.roi_fallbacks()
+            t_new, got = timed(lambda: m.detect_faces(host, boxes, index), args.reps)
+            fallbacks = (m.ctx.roi_fallbacks() - fb) / (args.reps + 1)
+            t_old, ref = timed(lambda: m.detect_faces_device(sd.bgr2gray(host, m.ctx), index, m.align_boxes(boxes)).cpu().numpy(), args.reps)
+            assert np.array_equal(got, ref)
+            report(case="d", route=route, faces_per_frame=k, faces=len(boxes), faces_per_s=len(boxes) / t_new,
+                   whole_frame_bgr2gray_faces_per_s=len(boxes) / t_old, roi_fallbacks_per_call=fallbacks)
+
+
+def finish(args, results):
     if args.out:
         os.makedirs(args.out, exist_ok=True)
         with open(os.path.join(args.out, "bench_faces.json"), "w") as f:

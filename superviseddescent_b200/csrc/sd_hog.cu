@@ -2,15 +2,15 @@
 // (reference include/rcr/adaptive_vlhog.hpp:109-185) fused with VLFeat's vl_hog_put_image /
 // vl_hog_extract (reference include/rcr/hog.c:595-728, :857-1062).
 //
-// One CTA per (sample, landmark) patch.  Everything between the 8-bit source image in HBM and the
-// feature row in HBM lives in shared memory:
+// One CTA walks the patches of up to kHogGroup consecutive landmarks of one sample.  Everything between the 8-bit source
+// image in HBM and the feature row in HBM lives in shared memory:
 //   geometry (IED -> half patch size, cvRound centre)            adaptive_vlhog.hpp:123,132-133
 //   zero-padded crop: ONE TMA tile load per patch (3-D tensor map over the frame batch; out-of-frame
 //     bytes are zero-filled by the TMA = copyMakeBorder(BORDER_CONSTANT 0))   adaptive_vlhog.hpp:135-151
 //   cv::resize INTER_LINEAR (fixed point), tables precomputed once per face   adaptive_vlhog.hpp:154-155
-//   gradient, orientation arg-max and modulus from device-generated tables (integer results, bit exact)  hog.c:631-672
+//   gradient, orientation arg-max from a device-generated table (integer result, bit exact), modulus   hog.c:631-672
 //   bilinear spatial vote as two separable passes (rows x cell columns, then cell rows; no atomics)      hog.c:697-724
-//   cell energy, 2x2-block normalisation in double, clamp 0.2    hog.c:875-1053
+//   cell energy, 2x2-block normalisation in double, clamp 0.2, for two patches at once    hog.c:875-1053
 //   per-dimension transpose + landmark concatenation + bias      adaptive_vlhog.hpp:166-183
 //
 // Arithmetic that decides an INTEGER result (crop centre, half size, resize taps, orientation bin)
@@ -29,6 +29,7 @@ namespace {
 constexpr int kHogThreads = 256;
 constexpr int kHogWarps = kHogThreads / 32;
 constexpr int kLutDim = 511;                       // gx, gy in [-255, 255]
+constexpr int kHogGroup = 11;                      // landmarks per CTA (at most; profiles/r05_hog_face.md)
 
 struct HogArgs {
     const uint8_t* images;
@@ -42,10 +43,11 @@ struct HogArgs {
     const float* x;
     long long ldx;
     int N, L;
+    int groups, gsz;            // a CTA walks gsz consecutive landmarks of one sample (the last group of a sample may be shorter)
+    int pair;                   // 1: S4-S8 run once per pair of consecutive patches (two tail slots in shared memory)
     int variant, nc, cs, K, fs, dd;
     const int* half;            // per sample: half patch size (hog_geometry_kernel)
     const int8_t* lut;          // (gy+255)*511 + (gx+255) -> directed orientation bin, -1 for a zero gradient
-    const float* mag_lut;       // gx*gx + gy*gy -> sqrtf of it (the exact integer's correctly rounded root)
     const int* rtab;            // per sample: resize tables [5][fs] (hog_geometry_kernel)
     const float* btab;          // per launch: spatial binning weights [nc][fs], then lo[nc], hi[nc] (hog_bintab_kernel)
     int tma_count;              // number of usable tensor-map size classes (0: the window is staged by load loops)
@@ -136,14 +138,6 @@ __global__ void hog_bintab_kernel(int fs, int nc, int cs, float* __restrict__ bt
     }
 }
 
-// sqrtf of every possible squared gradient modulus of an 8-bit patch (gx, gy in [-255, 255]): hog.c:645 takes sqrtf of the
-// float gx*gx + gy*gy, which is an exactly representable integer here
-__global__ void hog_maglut_kernel(float* __restrict__ lut, int n)
-{
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) lut[i] = __fsqrt_rn((float)i);
-}
-
 // ---- (gx, gy) -> orientation bin table, generated ON THE DEVICE with the reference's float expression
 //      (hog.c:645-672): gradients of an 8-bit patch are integers in [-255, 255], so the arg-max is a pure
 //      function of the pair and can be tabulated exactly. ---------------------------------------------
@@ -184,16 +178,18 @@ struct HogSmem {
 
 __host__ __device__ inline int align_up(int v, int a) { return (v + a - 1) / a * a; }
 
-__host__ __device__ inline HogSmem hog_smem_layout(int fs, int nc, int K, int dd)
+// The feature slice is sized for the larger of the two variants' dimension counts (UoCTTI 3K + 4, Dalal-Triggs 4K), so the
+// layout is a function of (fs, nc, K) and the number of tail slots (1, or 2 when S4-S8 run for pairs of patches) alone: a
+// compile-time constant in the baked schedules.
+__host__ __device__ inline HogSmem hog_smem_layout(int fs, int nc, int K, int slots)
 {
     HogSmem s;
     const int cells = nc * nc;
+    const int dd = 3 * K + 4 > 4 * K ? 3 * K + 4 : 4 * K;
     int o = 0;
     s.patch = o;  o = align_up(o + fs * fs, 128);
     s.bin = o;    o = align_up(o + fs * fs, 16);            // [bin | r1] doubles as the staging area of the source window (128-byte
-    int r1 = fs * fs * 4;                                   //  aligned: TMA destination); r1 = gradient modulus, later the clamped
-    if (cells * K * 32 > r1) r1 = cells * K * 32;           //  hc values (double)
-    s.r1 = o;     o = align_up(o + r1, 16);
+    s.r1 = o;     o = align_up(o + fs * fs * 4, 16);        //  aligned: TMA destination); r1 = gradient modulus
     s.xofs = o;   o += fs * 4;
     s.yofs0 = o;  o += fs * 4;
     s.yofs1 = o;  o += fs * 4;
@@ -202,13 +198,13 @@ __host__ __device__ inline HogSmem hog_smem_layout(int fs, int nc, int K, int dd
     s.wcell = o;  o += nc * fs * 4;                         // weight of pixel t for cell index c (0 if it does not vote)
     s.lo = o;     o += nc * 4;
     s.hi = o;     o += nc * 4;
-    s.hist = o;   o += cells * 2 * K * 4;
-    s.energy = o; o = align_up(o + cells * 4, 16);
-    s.fac = o;    o += cells * 4 * 8;
+    s.hist = o;   o += slots * cells * 2 * K * 4;           // hist, energy, fac, feat: one slot per patch of a pair
+    s.energy = o; o = align_up(o + slots * cells * 4, 16);
+    s.fac = o;    o += slots * cells * 4 * 8;
     s.tpad = align_up((fs - 2) * nc, 32);
     o = align_up(o, 16);
     s.vote = o;   o += 2 * K * s.tpad * 4;                  // horizontal pass of the vote: T[bin][(cell column, row)]
-    s.feat = o;   o += cells * dd * 4;
+    s.feat = o;   o += slots * cells * dd * 4;
     s.mbar = align_up(o, 8); o = s.mbar + 8;
     s.total = align_up(o, 16);
     return s;
@@ -223,8 +219,10 @@ constexpr int kTmaClasses = 8;
 __host__ __device__ constexpr int hog_tma_box(int c) { return c == 0 ? 32 : c == 1 ? 48 : c == 2 ? 64 : c == 3 ? 80 : c == 4 ? 96 : c == 5 ? 112 : c == 6 ? 128 : 160; }
 struct HogMaps { CUtensorMap m[kTmaClasses]; };
 
+// The baked schedules must keep five CTAs resident per SM (<= 51 registers a thread): four measured 21 % slower.  The run-time
+// schedules keep the four (<= 64 registers) they had before.
 template <int KT, int NCT, int CST>
-__global__ void __launch_bounds__(kHogThreads) hog_patch_kernel(const HogArgs a, const __grid_constant__ HogMaps maps)
+__global__ void __launch_bounds__(kHogThreads, NCT > 0 ? 5 : 4) hog_patch_kernel(const HogArgs a, const __grid_constant__ HogMaps maps)
 {
     extern __shared__ __align__(128) unsigned char smem[];
     const int K = KT > 0 ? KT : a.K;
@@ -232,11 +230,11 @@ __global__ void __launch_bounds__(kHogThreads) hog_patch_kernel(const HogArgs a,
     const int fs = (NCT > 0 && CST > 0) ? NCT * CST : a.fs;
     const int dd = a.dd;
     const int cells = nc * nc;
-    const HogSmem lay = hog_smem_layout(fs, nc, K, dd);
+    // both layouts are compile-time constants in the baked schedules
+    const HogSmem lay = a.pair ? hog_smem_layout(fs, nc, K, 2) : hog_smem_layout(fs, nc, K, 1);
     uint8_t* s_patch = smem + lay.patch;
     int8_t* s_bin = reinterpret_cast<int8_t*>(smem + lay.bin);
     float* s_gmag = reinterpret_cast<float*>(smem + lay.r1);
-    double* s_hc = reinterpret_cast<double*>(smem + lay.r1);
     int* s_xofs = reinterpret_cast<int*>(smem + lay.xofs);
     int* s_yofs0 = reinterpret_cast<int*>(smem + lay.yofs0);
     int* s_yofs1 = reinterpret_cast<int*>(smem + lay.yofs1);
@@ -254,22 +252,21 @@ __global__ void __launch_bounds__(kHogThreads) hog_patch_kernel(const HogArgs a,
 
     const int tid = threadIdx.x;
     const int lane = tid & 31, warp = tid >> 5;
-    const long long patch_id = blockIdx.x;
-    const int sample = (int)(patch_id / a.L);
-    const int lm = (int)(patch_id - (long long)sample * a.L);
+    // this CTA's patches: landmarks [lm_begin, lm_end) of one sample
+    const int sample = (int)blockIdx.x / a.groups;
+    const int lm_begin = ((int)blockIdx.x - sample * a.groups) * a.gsz;
+    const int lm_end = min(lm_begin + a.gsz, a.L);
 
-    // ---- S0: geometry: half size from the per-sample pre-pass, centre = cvRound (adaptive_vlhog.hpp:132-133)
+    // ---- S0: per-sample state, once per CTA: half size from the per-sample pre-pass (adaptive_vlhog.hpp:123), the frame
+    //      and the region of it that is resident (the whole frame, or the ROI that sd_detect_batch_host uploaded)
     const float* __restrict__ row = a.x + (long long)sample * a.ldx;
     const int half = __ldg(a.half + sample);
     const int P = 2 * half;
-    const int cx = __float2int_rn(row[lm]);
-    const int cy = __float2int_rn(row[lm + a.L]);
     int img_idx = a.image_index ? a.image_index[sample] : sample;
     if (img_idx < 0 || img_idx >= a.image_count) {
         img_idx = 0;
         if (tid == 0 && a.status) atomicOr(a.status, 2);
     }
-    // resident region of this frame: the whole frame, or the ROI that sd_detect_batch_host uploaded
     int W = a.width, H = a.height, rs = a.row_stride;
     const uint8_t* __restrict__ img = a.images + (long long)img_idx * a.image_stride;
     if (a.frames) {
@@ -283,42 +280,13 @@ __global__ void __launch_bounds__(kHogThreads) hog_patch_kernel(const HogArgs a,
         rx = r.x; ry = r.y; rw = r.w; rh = r.h; rs = r.row_stride;
         img = a.images + r.offset;
     }
-    if (tid == 0 && a.geometry) {
-        a.geometry[patch_id * 3 + 0] = cx;
-        a.geometry[patch_id * 3 + 1] = cy;
-        a.geometry[patch_id * 3 + 2] = half;
-    }
-
-    // ---- S1: zero-padded crop + fixed-point bilinear resize.  The P x P source window is staged in shared memory with its
-    //      zero padding materialised, then resampled from there: one output row per warp pass, lanes along x.
-    const int x0 = cx - half, y0 = cy - half;
-    uint8_t* s_stage = smem + lay.bin;                             // [bin | r1] are dead until S2
-    const int stage_cap = lay.xofs - lay.bin;
-    // TMA route: whole frames resident and describable by a tensor map; the smallest box class that covers the window and
-    // fits the staging area
-    int tma_box = 0;
-    // The TMA wants the box to start on a 16-byte boundary of the innermost dimension (an unaligned start faults with "illegal
-    // instruction"): the box starts at x0 rounded down to a multiple of 16 and the window sits tma_shift bytes into its rows.
-    const int tma_shift = x0 & 15;
-#pragma unroll
-    for (int c = kTmaClasses - 1; c >= 0; --c)
-        if (c < a.tma_count && hog_tma_box(c) >= P + tma_shift && hog_tma_box(c) * hog_tma_box(c) <= stage_cap) tma_box = hog_tma_box(c);
-    if (tma_box > 0 && tid == 0) {
-        // one elected thread: the box lands densely (pitch = box width); bytes outside the frame are zero-filled by the TMA,
-        // which is exactly copyMakeBorder(..., BORDER_CONSTANT, 0) (adaptive_vlhog.hpp:136-147)
-        const uint32_t bar = (uint32_t)__cvta_generic_to_shared(s_mbar);
+    const uint32_t bar = (uint32_t)__cvta_generic_to_shared(s_mbar);
+    if (tid == 0 && a.tma_count > 0) {
         asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar));
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(tma_box * tma_box) : "memory");
-        int cls = 0;
-#pragma unroll
-        for (int c = 0; c < kTmaClasses; ++c) if (hog_tma_box(c) == tma_box) cls = c;
-        asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-                     ::"r"((uint32_t)__cvta_generic_to_shared(s_stage)), "l"(&maps.m[cls]), "r"(bar), "r"(x0 - tma_shift), "r"(y0), "r"(img_idx)
-                     : "memory");
     }
-
-    // tables: cv::resize taps of this sample (hog_geometry_kernel), spatial binning weights of this launch (hog_bintab_kernel)
+    // tables shared by every patch of the CTA: cv::resize taps of this sample (hog_geometry_kernel), spatial binning weights
+    // of this launch (hog_bintab_kernel).  They are visible after the first patch's staging barrier.
     {
         const int* __restrict__ rt = a.rtab + (long long)sample * 5 * fs;
         for (int t = tid; t < fs; t += kHogThreads) {
@@ -332,295 +300,364 @@ __global__ void __launch_bounds__(kHogThreads) hog_patch_kernel(const HogArgs a,
         for (int i = tid; i < nc * fs; i += kHogThreads) s_wcell[i] = __ldg(a.btab + i);
         const int* __restrict__ lohi = reinterpret_cast<const int*>(a.btab + nc * fs);
         if (tid < nc) { s_lo[tid] = __ldg(lohi + tid); s_hi[tid] = __ldg(lohi + nc + tid); }
-        float4* T4 = reinterpret_cast<float4*>(s_T);
-        for (int i = tid; i < K * lay.tpad / 2; i += kHogThreads) T4[i] = make_float4(0.f, 0.f, 0.f, 0.f);     // 2K * tpad floats
     }
-    {
-        const bool resident = x0 >= rx && y0 >= ry && x0 + P <= rx + rw && y0 + P <= ry + rh && x0 >= 0 && y0 >= 0 && x0 + P <= W && y0 + P <= H;
-        const uintptr_t align_bits = reinterpret_cast<uintptr_t>(img) | (uintptr_t)rs;
-        const bool vec16 = !tma_box && resident && (align_bits & 15) == 0;      // rows can be fetched as aligned 16-byte vectors
-        const bool words = !tma_box && resident && (align_bits & 3) == 0;
-        // column c of the staged window sits at byte shiftb + c of its row
-        const int shiftb = tma_box ? tma_shift : (vec16 ? ((x0 - rx) & 15) : (words ? ((x0 - rx) & 3) : 0));
-        const int pitch = tma_box ? tma_box : ((P + 15 + 15) & ~15);
-        const bool staged = pitch * P <= stage_cap;
-        bool miss = false;
-        if (staged) {
-            if (tma_box) {
-                // nothing to do: the tile is in flight
-            } else if (vec16) {
-                // 8 / 16 / 32 lanes per source row, one aligned uint4 each: ~P * nvec / 32 warp loads in total
-                const int nvec = (shiftb + P + 15) >> 4;
-                const int gs = nvec <= 8 ? 3 : (nvec <= 16 ? 4 : 5);
-                const int lv = lane & ((1 << gs) - 1), lr = lane >> gs, rows_per_pass = 32 >> gs;
-                const uint8_t* wrow = img + (long long)(y0 - ry) * rs + (x0 - rx - shiftb);
-                for (int r = warp * rows_per_pass + lr; r < P; r += kHogWarps * rows_per_pass)
-                    for (int v = lv; v < nvec; v += (1 << gs))
-                        reinterpret_cast<uint4*>(s_stage + r * pitch)[v] = __ldg(reinterpret_cast<const uint4*>(wrow + (long long)r * rs) + v);
-            } else if (words) {
-                const int nwords = (shiftb + P + 3) >> 2;
-                const uint8_t* wrow = img + (long long)(y0 - ry) * rs + (x0 - rx - shiftb);
-                for (int r = warp; r < P; r += kHogWarps) {
-                    const uint32_t* src = reinterpret_cast<const uint32_t*>(wrow + (long long)r * rs);
-                    uint32_t* dst = reinterpret_cast<uint32_t*>(s_stage + r * pitch);
-                    for (int w = lane; w < nwords; w += 32) dst[w] = __ldg(src + w);
-                }
-            } else {
-                for (int r = warp; r < P; r += kHogWarps) {
-                    const int iy = y0 + r;
-                    const bool rowin = (unsigned)iy < (unsigned)H;
-                    const bool rowres = iy >= ry && iy < ry + rh;
-                    for (int c = lane; c < P; c += 32) {
-                        const int ix = x0 + c;
-                        int v = 0;
-                        if (rowin && (unsigned)ix < (unsigned)W) {
-                            if (rowres && ix >= rx && ix < rx + rw) v = __ldg(img + (long long)(iy - ry) * rs + (ix - rx));
-                            else miss = true;                      // a frame pixel that was not uploaded
+    uint8_t* s_stage = smem + lay.bin;                                 // [bin | r1]: dead between S8 and the next S2
+    const int stage_cap = lay.xofs - lay.bin;
+    uint32_t tma_phase = 0;                                            // parity of the mbarrier phase the next TMA completes
+
+    // Shared-memory regions live in each phase of one patch (the loop's barriers separate consecutive patches):
+    //   S1  stage = [bin | r1] (window), patch (written), tables, T (zeroed)
+    //   S2  patch (read), bin + gmag (r1) written
+    //   S3  bin, gmag, tables, T -> hist
+    //   S4-S7  hist, energy, fac, feat (once per pair of patches)
+    //   S8  feat
+    for (int lm = lm_begin; lm < lm_end; ++lm) {
+        const int slot = a.pair ? (lm - lm_begin) & 1 : 0;             // hist / feat slot of this patch in its pair
+        const int patch_id = sample * a.L + lm;                        // < 2^31: launch_hog checks N * L
+        const int cx = __float2int_rn(row[lm]);                        // centre = cvRound (adaptive_vlhog.hpp:132-133)
+        const int cy = __float2int_rn(row[lm + a.L]);
+        if (tid == 0 && a.geometry) {
+            a.geometry[patch_id * 3 + 0] = cx;
+            a.geometry[patch_id * 3 + 1] = cy;
+            a.geometry[patch_id * 3 + 2] = half;
+        }
+
+        // ---- S1: zero-padded crop + fixed-point bilinear resize.  The P x P source window is staged in shared memory with
+        //      its zero padding materialised, then resampled from there: one output row per warp pass, lanes along x.
+        const int x0 = cx - half, y0 = cy - half;
+        // TMA route: whole frames resident and describable by a tensor map; the smallest box class that covers the window and
+        // fits the staging area
+        int tma_box = 0;
+        // The TMA wants the box to start on a 16-byte boundary of the innermost dimension (an unaligned start faults with
+        // "illegal instruction"): the box starts at x0 rounded down to a multiple of 16 and the window sits tma_shift bytes
+        // into its rows.
+        const int tma_shift = x0 & 15;
+#pragma unroll
+        for (int c = kTmaClasses - 1; c >= 0; --c)
+            if (c < a.tma_count && hog_tma_box(c) >= P + tma_shift && hog_tma_box(c) * hog_tma_box(c) <= stage_cap) tma_box = hog_tma_box(c);
+        if (tma_box > 0 && tid == 0) {
+            // one elected thread: the box lands densely (pitch = box width); bytes outside the frame are zero-filled by the
+            // TMA, which is exactly copyMakeBorder(..., BORDER_CONSTANT, 0) (adaptive_vlhog.hpp:136-147).  The previous
+            // patch's generic-proxy writes to the staging area were fenced before the barrier that ended it.
+            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(tma_box * tma_box) : "memory");
+            int cls = 0;
+#pragma unroll
+            for (int c = 0; c < kTmaClasses; ++c) if (hog_tma_box(c) == tma_box) cls = c;
+            asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
+                         ::"r"((uint32_t)__cvta_generic_to_shared(s_stage)), "l"(&maps.m[cls]), "r"(bar), "r"(x0 - tma_shift), "r"(y0), "r"(img_idx)
+                         : "memory");
+        }
+        {
+            float4* T4 = reinterpret_cast<float4*>(s_T);
+            for (int i = tid; i < K * lay.tpad / 2; i += kHogThreads) T4[i] = make_float4(0.f, 0.f, 0.f, 0.f);     // 2K * tpad floats
+        }
+        {
+            const bool resident = x0 >= rx && y0 >= ry && x0 + P <= rx + rw && y0 + P <= ry + rh && x0 >= 0 && y0 >= 0 && x0 + P <= W && y0 + P <= H;
+            const uintptr_t align_bits = reinterpret_cast<uintptr_t>(img) | (uintptr_t)rs;
+            const bool vec16 = !tma_box && resident && (align_bits & 15) == 0;      // rows can be fetched as aligned 16-byte vectors
+            const bool words = !tma_box && resident && (align_bits & 3) == 0;
+            // column c of the staged window sits at byte shiftb + c of its row
+            const int shiftb = tma_box ? tma_shift : (vec16 ? ((x0 - rx) & 15) : (words ? ((x0 - rx) & 3) : 0));
+            const int pitch = tma_box ? tma_box : ((P + 15 + 15) & ~15);
+            const bool staged = pitch * P <= stage_cap;
+            bool miss = false;
+            if (staged) {
+                if (tma_box) {
+                    // nothing to do: the tile is in flight
+                } else if (vec16) {
+                    // 8 / 16 / 32 lanes per source row, one aligned uint4 each: ~P * nvec / 32 warp loads in total
+                    const int nvec = (shiftb + P + 15) >> 4;
+                    const int gs = nvec <= 8 ? 3 : (nvec <= 16 ? 4 : 5);
+                    const int lv = lane & ((1 << gs) - 1), lr = lane >> gs, rows_per_pass = 32 >> gs;
+                    const uint8_t* wrow = img + (long long)(y0 - ry) * rs + (x0 - rx - shiftb);
+                    for (int r = warp * rows_per_pass + lr; r < P; r += kHogWarps * rows_per_pass)
+                        for (int v = lv; v < nvec; v += (1 << gs))
+                            reinterpret_cast<uint4*>(s_stage + r * pitch)[v] = __ldg(reinterpret_cast<const uint4*>(wrow + (long long)r * rs) + v);
+                } else if (words) {
+                    const int nwords = (shiftb + P + 3) >> 2;
+                    const uint8_t* wrow = img + (long long)(y0 - ry) * rs + (x0 - rx - shiftb);
+                    for (int r = warp; r < P; r += kHogWarps) {
+                        const uint32_t* src = reinterpret_cast<const uint32_t*>(wrow + (long long)r * rs);
+                        uint32_t* dst = reinterpret_cast<uint32_t*>(s_stage + r * pitch);
+                        for (int w = lane; w < nwords; w += 32) dst[w] = __ldg(src + w);
+                    }
+                } else {
+                    for (int r = warp; r < P; r += kHogWarps) {
+                        const int iy = y0 + r;
+                        const bool rowin = (unsigned)iy < (unsigned)H;
+                        const bool rowres = iy >= ry && iy < ry + rh;
+                        for (int c = lane; c < P; c += 32) {
+                            const int ix = x0 + c;
+                            int v = 0;
+                            if (rowin && (unsigned)ix < (unsigned)W) {
+                                if (rowres && ix >= rx && ix < rx + rw) v = __ldg(img + (long long)(iy - ry) * rs + (ix - rx));
+                                else miss = true;                      // a frame pixel that was not uploaded
+                            }
+                            s_stage[r * pitch + c] = (uint8_t)v;
                         }
-                        s_stage[r * pitch + c] = (uint8_t)v;
                     }
                 }
-            }
-            __syncthreads();                                       // tables (and the load loops' stores) visible
-            if (tma_box) {
-                const uint32_t bar = (uint32_t)__cvta_generic_to_shared(s_mbar);
-                uint32_t ok = 0;
-                const long long t0 = clock64();
-                while (!ok) {                                      // bounded: a protocol bug must trap, never hang the GPU
-                    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], 0;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                                 : "=r"(ok) : "r"(bar) : "memory");
-                    if (!ok && clock64() - t0 > 4000000000LL) __trap();
+                __syncthreads();                                       // tables (and the load loops' stores) visible
+                if (tma_box) {
+                    uint32_t ok = 0;
+                    const long long t0 = clock64();
+                    while (!ok) {                                      // bounded: a protocol bug must trap, never hang the GPU
+                        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
+                                     : "=r"(ok) : "r"(bar), "r"(tma_phase) : "memory");
+                        if (!ok && clock64() - t0 > 4000000000LL) __trap();
+                    }
+                    tma_phase ^= 1;
                 }
-            }
-            if (fs <= 64) {
-                // a thread keeps ONE output column (its two source taps and weights stay in registers) and walks down the rows
-                const int dx = tid & 63, g = tid >> 6;
-                if (dx < fs) {
-                    const int sx = s_xofs[dx];
-                    const int sx1 = min(sx + 1, P - 1);            // clamped tap has zero weight
-                    const int ax = s_xa[dx].x, bx = s_xa[dx].y;
-                    const uint8_t* base = s_stage + shiftb;
+                if (fs <= 64) {
+                    // a thread keeps ONE output column (its two source taps and weights stay in registers) and walks down the rows
+                    const int dx = tid & 63, g = tid >> 6;
+                    if (dx < fs) {
+                        const int sx = s_xofs[dx];
+                        const int sx1 = min(sx + 1, P - 1);            // clamped tap has zero weight
+                        const int ax = s_xa[dx].x, bx = s_xa[dx].y;
+                        const uint8_t* base = s_stage + shiftb;
 #pragma unroll 4
-                    for (int dy = g; dy < fs; dy += kHogThreads / 64) {
+                        for (int dy = g; dy < fs; dy += kHogThreads / 64) {
+                            const short2 yb = s_yb[dy];
+                            const uint8_t* r0 = base + s_yofs0[dy] * pitch;
+                            const uint8_t* r1 = base + s_yofs1[dy] * pitch;
+                            const int t0 = (int)r0[sx] * ax + (int)r0[sx1] * bx;
+                            const int t1 = (int)r1[sx] * ax + (int)r1[sx1] * bx;
+                            const int v = ((((int)yb.x * (t0 >> 4)) >> 16) + (((int)yb.y * (t1 >> 4)) >> 16) + 2) >> 2;
+                            s_patch[dy * fs + dx] = (uint8_t)v;        // s_patch precedes the staging area: no overlap
+                        }
+                    }
+                } else {
+                    for (int dy = warp; dy < fs; dy += kHogWarps) {
                         const short2 yb = s_yb[dy];
-                        const uint8_t* r0 = base + s_yofs0[dy] * pitch;
-                        const uint8_t* r1 = base + s_yofs1[dy] * pitch;
-                        const int t0 = (int)r0[sx] * ax + (int)r0[sx1] * bx;
-                        const int t1 = (int)r1[sx] * ax + (int)r1[sx1] * bx;
-                        const int v = ((((int)yb.x * (t0 >> 4)) >> 16) + (((int)yb.y * (t1 >> 4)) >> 16) + 2) >> 2;
-                        s_patch[dy * fs + dx] = (uint8_t)v;        // s_patch precedes the staging area: no overlap
+                        const uint8_t* r0 = s_stage + s_yofs0[dy] * pitch + shiftb;
+                        const uint8_t* r1 = s_stage + s_yofs1[dy] * pitch + shiftb;
+                        for (int dx = lane; dx < fs; dx += 32) {
+                            const int sx = s_xofs[dx];
+                            const int sx1 = min(sx + 1, P - 1);
+                            const short2 xa = s_xa[dx];
+                            const int t0 = (int)r0[sx] * xa.x + (int)r0[sx1] * xa.y;
+                            const int t1 = (int)r1[sx] * xa.x + (int)r1[sx1] * xa.y;
+                            const int v = ((((int)yb.x * (t0 >> 4)) >> 16) + (((int)yb.y * (t1 >> 4)) >> 16) + 2) >> 2;
+                            s_patch[dy * fs + dx] = (uint8_t)v;
+                        }
                     }
                 }
             } else {
+                // window too large for the staging area: sample straight from global memory with full checks
+                __syncthreads();                                       // tables visible
                 for (int dy = warp; dy < fs; dy += kHogWarps) {
                     const short2 yb = s_yb[dy];
-                    const uint8_t* r0 = s_stage + s_yofs0[dy] * pitch + shiftb;
-                    const uint8_t* r1 = s_stage + s_yofs1[dy] * pitch + shiftb;
+                    const int iy0 = y0 + s_yofs0[dy], iy1 = y0 + s_yofs1[dy];
                     for (int dx = lane; dx < fs; dx += 32) {
                         const int sx = s_xofs[dx];
-                        const int sx1 = min(sx + 1, P - 1);
                         const short2 xa = s_xa[dx];
-                        const int t0 = (int)r0[sx] * xa.x + (int)r0[sx1] * xa.y;
-                        const int t1 = (int)r1[sx] * xa.x + (int)r1[sx1] * xa.y;
+                        int p[4];
+#pragma unroll
+                        for (int q = 0; q < 4; ++q) {
+                            const int ix = x0 + sx + (q & 1), iy = (q & 2) ? iy1 : iy0;
+                            int v = 0;
+                            if ((q & 1) && xa.y == 0) { p[q] = 0; continue; }
+                            if ((unsigned)ix < (unsigned)W && (unsigned)iy < (unsigned)H) {
+                                if (ix >= rx && ix < rx + rw && iy >= ry && iy < ry + rh) v = __ldg(img + (long long)(iy - ry) * rs + (ix - rx));
+                                else miss = true;
+                            }
+                            p[q] = v;
+                        }
+                        const int t0 = p[0] * xa.x + p[1] * xa.y;
+                        const int t1 = p[2] * xa.x + p[3] * xa.y;
                         const int v = ((((int)yb.x * (t0 >> 4)) >> 16) + (((int)yb.y * (t1 >> 4)) >> 16) + 2) >> 2;
                         s_patch[dy * fs + dx] = (uint8_t)v;
                     }
                 }
             }
-        } else {
-            // window too large for the staging area: sample straight from global memory with full checks
-            __syncthreads();                                       // tables visible
-            for (int dy = warp; dy < fs; dy += kHogWarps) {
-                const short2 yb = s_yb[dy];
-                const int iy0 = y0 + s_yofs0[dy], iy1 = y0 + s_yofs1[dy];
-                for (int dx = lane; dx < fs; dx += 32) {
-                    const int sx = s_xofs[dx];
-                    const short2 xa = s_xa[dx];
-                    int p[4];
+            if (miss && a.roi_miss) a.roi_miss[img_idx] = 1;
+            if (a.patches) {
+                __syncthreads();
+                for (int i = tid; i < fs * fs; i += kHogThreads) a.patches[(long long)patch_id * fs * fs + i] = s_patch[i];
+            }
+        }
+        __syncthreads();
+
+        // ---- S2: gradient + orientation arg-max per interior pixel (hog.c:631-672): the arg-max comes from the
+        //      device-generated table (the gradient of an 8-bit patch is a pair of integers in [-255, 255]); the modulus is
+        //      sqrtf of the exactly representable integer gx*gx + gy*gy (hog.c:645), computed in registers
+        {
+            // linear index over the interior pixels (all lanes busy); four pixels per thread in flight so that the four table
+            // look-ups overlap (the phase was bound by their latency: profiles/r02_summary.md)
+            const int iw = fs - 2, npix = iw * iw;
+            for (int i0 = tid; i0 < npix; i0 += 4 * kHogThreads) {
+                int idx[4], gxs[4], gys[4];
 #pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        const int ix = x0 + sx + (q & 1), iy = (q & 2) ? iy1 : iy0;
-                        int v = 0;
-                        if ((q & 1) && xa.y == 0) { p[q] = 0; continue; }
-                        if ((unsigned)ix < (unsigned)W && (unsigned)iy < (unsigned)H) {
-                            if (ix >= rx && ix < rx + rw && iy >= ry && iy < ry + rh) v = __ldg(img + (long long)(iy - ry) * rs + (ix - rx));
-                            else miss = true;
-                        }
-                        p[q] = v;
+                for (int k = 0; k < 4; ++k) {
+                    const int i = i0 + k * kHogThreads;
+                    const int y = i / iw, x = i - y * iw;
+                    idx[k] = (y + 1) * fs + (x + 1);
+                    if (i < npix) {
+                        gxs[k] = (int)s_patch[idx[k] + 1] - (int)s_patch[idx[k] - 1];
+                        gys[k] = (int)s_patch[idx[k] + fs] - (int)s_patch[idx[k] - fs];
+                    } else { gxs[k] = 0; gys[k] = 0; }
+                }
+                int8_t bn[4];
+#pragma unroll
+                for (int k = 0; k < 4; ++k) bn[k] = __ldg(a.lut + (gys[k] + 255) * kLutDim + (gxs[k] + 255));
+#pragma unroll
+                for (int k = 0; k < 4; ++k)
+                    if (i0 + k * kHogThreads < npix) {
+                        s_bin[idx[k]] = bn[k];
+                        s_gmag[idx[k]] = __fsqrt_rn((float)(gxs[k] * gxs[k] + gys[k] * gys[k]));
                     }
-                    const int t0 = p[0] * xa.x + p[1] * xa.y;
-                    const int t1 = p[2] * xa.x + p[3] * xa.y;
-                    const int v = ((((int)yb.x * (t0 >> 4)) >> 16) + (((int)yb.y * (t1 >> 4)) >> 16) + 2) >> 2;
-                    s_patch[dy * fs + dx] = (uint8_t)v;
+            }
+        }
+        if (a.bins) {
+            __syncthreads();
+            for (int idx = tid; idx < fs * fs; idx += kHogThreads) {
+                const int y = idx / fs, x = idx - y * fs;
+                const bool interior = x >= 1 && x <= fs - 2 && y >= 1 && y <= fs - 2;
+                a.bins[(long long)patch_id * fs * fs + idx] = interior ? s_bin[idx] : (int8_t)-1;
+            }
+        }
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // bin / gmag writes before the next patch's TMA
+        __syncthreads();
+
+        // ---- S3: bilinear spatial vote (hog.c:697-724), separable:  hist[b][cj][ci] = sum_y wy[cj][y] * ( sum_x wx[ci][x] * g[y][x] * [bin[y][x] == b] ).
+        //      Pass 1: one thread per (cell column ci, interior row y) walks the <= 2*cs pixels of that row that vote into ci and adds
+        //      g * wx into ITS OWN column of T[bin][task] (bank == task mod 32: conflict free, no atomics, fixed order).
+        //      Pass 2: one thread per (bin, cell) folds the rows with wy.  The reference adds (g * wx) * wy per pixel in raster
+        //      order; this is the same sum associated differently (~1e-7 relative), deterministic.
+        {
+            const int nrow = fs - 2, ntask = nrow * nc, tpad = lay.tpad;
+            for (int task = tid; task < ntask; task += kHogThreads) {
+                const int ci = task / nrow, y = 1 + task - ci * nrow;
+                const int xlo = s_lo[ci], xhi = s_hi[ci];
+                const int8_t* bp = s_bin + y * fs + xlo;
+                const float* gp = s_gmag + y * fs + xlo;
+                const float* wp = s_wcell + ci * fs + xlo;
+                float* T = s_T + task;
+#pragma unroll 2
+                for (int x = xlo; x <= xhi; ++x) {
+                    const int b = max((int)*bp++, 0);                     // zero gradient: bin -1, modulus 0 -> adds +0 to bin 0
+                    float* q = T + b * tpad;
+                    *q = __fadd_rn(*q, __fmul_rn(*gp++, *wp++));
                 }
             }
-        }
-        if (miss && a.roi_miss) a.roi_miss[img_idx] = 1;
-        if (a.patches) {
             __syncthreads();
-            for (int i = tid; i < fs * fs; i += kHogThreads) a.patches[patch_id * fs * fs + i] = s_patch[i];
-        }
-    }
-    __syncthreads();
-
-    // ---- S2: gradient + orientation arg-max per interior pixel (hog.c:631-672): arg-max and modulus come from the
-    //      device-generated tables (the gradient of an 8-bit patch is a pair of integers in [-255, 255]) ---------
-    {
-        // linear index over the interior pixels (all lanes busy); four pixels per thread in flight so that the eight table
-        // look-ups overlap (the phase was bound by their latency: profiles/r02_summary.md)
-        const int iw = fs - 2, npix = iw * iw;
-        for (int i0 = tid; i0 < npix; i0 += 4 * kHogThreads) {
-            int idx[4], gxs[4], gys[4];
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                const int i = i0 + k * kHogThreads;
-                const int y = i / iw, x = i - y * iw;
-                idx[k] = (y + 1) * fs + (x + 1);
-                if (i < npix) {
-                    gxs[k] = (int)s_patch[idx[k] + 1] - (int)s_patch[idx[k] - 1];
-                    gys[k] = (int)s_patch[idx[k] + fs] - (int)s_patch[idx[k] - fs];
-                } else { gxs[k] = 0; gys[k] = 0; }
-            }
-            int8_t bn[4];
-            float mg[4];
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                bn[k] = __ldg(a.lut + (gys[k] + 255) * kLutDim + (gxs[k] + 255));
-                mg[k] = __ldg(a.mag_lut + (gxs[k] * gxs[k] + gys[k] * gys[k]));
-            }
-#pragma unroll
-            for (int k = 0; k < 4; ++k)
-                if (i0 + k * kHogThreads < npix) { s_bin[idx[k]] = bn[k]; s_gmag[idx[k]] = mg[k]; }
-        }
-    }
-    if (a.bins) {
-        __syncthreads();
-        for (int idx = tid; idx < fs * fs; idx += kHogThreads) {
-            const int y = idx / fs, x = idx - y * fs;
-            const bool interior = x >= 1 && x <= fs - 2 && y >= 1 && y <= fs - 2;
-            a.bins[patch_id * fs * fs + idx] = interior ? s_bin[idx] : (int8_t)-1;
-        }
-    }
-    __syncthreads();
-
-    // ---- S3: bilinear spatial vote (hog.c:697-724), separable:  hist[b][cj][ci] = sum_y wy[cj][y] * ( sum_x wx[ci][x] * g[y][x] * [bin[y][x] == b] ).
-    //      Pass 1: one thread per (cell column ci, interior row y) walks the <= 2*cs pixels of that row that vote into ci and adds
-    //      g * wx into ITS OWN column of T[bin][task] (bank == task mod 32: conflict free, no atomics, fixed order).
-    //      Pass 2: one thread per (bin, cell) folds the rows with wy.  The reference adds (g * wx) * wy per pixel in raster
-    //      order; this is the same sum associated differently (~1e-7 relative), deterministic.
-    {
-        const int nrow = fs - 2, ntask = nrow * nc, tpad = lay.tpad;
-        for (int task = tid; task < ntask; task += kHogThreads) {
-            const int ci = task / nrow, y = 1 + task - ci * nrow;
-            const int xlo = s_lo[ci], xhi = s_hi[ci];
-            const int8_t* bp = s_bin + y * fs + xlo;
-            const float* gp = s_gmag + y * fs + xlo;
-            const float* wp = s_wcell + ci * fs + xlo;
-            float* T = s_T + task;
-#pragma unroll 2
-            for (int x = xlo; x <= xhi; ++x) {
-                const int b = max((int)*bp++, 0);                     // zero gradient: bin -1, modulus 0 -> adds +0 to bin 0
-                float* q = T + b * tpad;
-                *q = __fadd_rn(*q, __fmul_rn(*gp++, *wp++));
+            for (int i = tid; i < 2 * K * cells; i += kHogThreads) {
+                const int b = i / cells, c = i - b * cells;
+                const int cj = c / nc, ci = c - cj * nc;                  // cell row (y), cell column (x)
+                const int ylo = s_lo[cj], yhi = s_hi[cj];
+                const float* Tp = s_T + b * tpad + ci * nrow + (ylo - 1);
+                const float* wy = s_wcell + cj * fs + ylo;
+                float acc = 0.f;
+                for (int y = ylo; y <= yhi; ++y) acc = __fadd_rn(acc, __fmul_rn(*Tp++, *wy++));
+                s_hist[slot * 2 * K * cells + b * cells + c] = acc;
             }
         }
         __syncthreads();
-        for (int i = tid; i < 2 * K * cells; i += kHogThreads) {
-            const int b = i / cells, c = i - b * cells;
-            const int cj = c / nc, ci = c - cj * nc;                  // cell row (y), cell column (x)
-            const int ylo = s_lo[cj], yhi = s_hi[cj];
-            const float* Tp = s_T + b * tpad + ci * nrow + (ylo - 1);
-            const float* wy = s_wcell + cj * fs + ylo;
-            float acc = 0.f;
-            for (int y = ylo; y <= yhi; ++y) acc = __fadd_rn(acc, __fmul_rn(*Tp++, *wy++));
-            s_hist[b * cells + c] = acc;
-        }
-    }
-    __syncthreads();
 
-    // ---- S4: undirected cell energy (hog.c:875-890) -------------------------------------------
-    for (int c = tid; c < cells; c += kHogThreads) {
-        float e = 0.f;
-        for (int k = 0; k < K; ++k) {
-            const float h = __fadd_rn(s_hist[k * cells + c], s_hist[(k + K) * cells + c]);
-            e = __fadd_rn(e, __fmul_rn(h, h));
-        }
-        s_energy[c] = e;
-    }
-    __syncthreads();
+        // ---- S4-S8 run once per pair of consecutive patches (or for the last patch alone): twice the threads per phase, half
+        //      the barriers per patch.  Slot p of the pair is patch lm_first + p.
+        if (slot == 1 || lm + 1 == lm_end || !a.pair) {
+            const int npair = slot + 1, lm_first = lm - slot;
 
-    // ---- S5: the four block factors of each cell, in double (hog.c:930-982) ------------------
-    for (int i = tid; i < cells * 4; i += kHogThreads) {
-        const int c = i >> 2, f = i & 3;
-        const int y = c / nc, x = c - y * nc;
-        const int xm = max(x - 1, 0), xp = min(x + 1, nc - 1);
-        const int ym = max(y - 1, 0), yp = min(y + 1, nc - 1);
-        // factor1: n1+n2+n4+n5, factor2: n2+n3+n5+n6, factor3: n4+n5+n7+n8, factor4: n5+n6+n8+n9
-        const int xa = (f & 1) ? x : xm, xb = (f & 1) ? xp : x;
-        const int ya = (f & 2) ? y : ym, yb = (f & 2) ? yp : y;
-        double s = (double)s_energy[xa + ya * nc];
-        s = __dadd_rn(s, (double)s_energy[xb + ya * nc]);
-        s = __dadd_rn(s, (double)s_energy[xa + yb * nc]);
-        s = __dadd_rn(s, (double)s_energy[xb + yb * nc]);
-        s = __dadd_rn(s, 1e-4);
-        s_fac[i] = __ddiv_rn(1.0, sqrt(s));
-    }
-    __syncthreads();
+            // ---- S4: undirected cell energy (hog.c:875-890) -------------------------------------------
+            for (int i = tid; i < npair * cells; i += kHogThreads) {
+                const int p = i >= cells ? 1 : 0, c = i - p * cells;
+                const float* hist = s_hist + p * 2 * K * cells;
+                float e = 0.f;
+                for (int k = 0; k < K; ++k) {
+                    const float h = __fadd_rn(hist[k * cells + c], hist[(k + K) * cells + c]);
+                    e = __fadd_rn(e, __fmul_rn(h, h));
+                }
+                s_energy[i] = e;
+            }
+            __syncthreads();
 
-    // ---- S6: normalise, clamp at 0.2, project (hog.c:985-1044); s_gmag is dead, reuse as s_hc -
-    for (int i = tid; i < cells * K; i += kHogThreads) {
-        const int k = i / cells, c = i - k * cells;
-        const int cj = c / nc, ci = c - cj * nc;
-        const int oc = ci * nc + cj;                        // per-dimension transpose, adaptive_vlhog.hpp:168-174
-        const double ha = (double)s_hist[k * cells + c];
-        const double hb = (double)s_hist[(k + K) * cells + c];
-        double sa = 0.0, sb = 0.0, sc = 0.0;
-        double hcv[4];
+            // ---- S5: the four block factors of each cell, in double (hog.c:930-982) ------------------
+            for (int i = tid; i < npair * cells * 4; i += kHogThreads) {
+                const int p = i >= cells * 4 ? 1 : 0, ii = i - p * cells * 4;
+                const int c = ii >> 2, f = ii & 3;
+                const int y = c / nc, x = c - y * nc;
+                const int xm = max(x - 1, 0), xp = min(x + 1, nc - 1);
+                const int ym = max(y - 1, 0), yp = min(y + 1, nc - 1);
+                // factor1: n1+n2+n4+n5, factor2: n2+n3+n5+n6, factor3: n4+n5+n7+n8, factor4: n5+n6+n8+n9
+                const int xa = (f & 1) ? x : xm, xb = (f & 1) ? xp : x;
+                const int ya = (f & 2) ? y : ym, yb = (f & 2) ? yp : y;
+                const float* energy = s_energy + p * cells;
+                double e = (double)energy[xa + ya * nc];
+                e = __dadd_rn(e, (double)energy[xb + ya * nc]);
+                e = __dadd_rn(e, (double)energy[xa + yb * nc]);
+                e = __dadd_rn(e, (double)energy[xb + yb * nc]);
+                e = __dadd_rn(e, 1e-4);
+                s_fac[i] = __ddiv_rn(1.0, sqrt(e));
+            }
+            __syncthreads();
+
+            // ---- S6: normalise, clamp at 0.2, project (hog.c:985-1044) ------------------------------
+            for (int i = tid; i < npair * cells * K; i += kHogThreads) {
+                const int p = i >= cells * K ? 1 : 0, ii = i - p * cells * K;
+                const int k = ii / cells, c = ii - k * cells;
+                const int cj = c / nc, ci = c - cj * nc;
+                const int oc = ci * nc + cj;                        // per-dimension transpose, adaptive_vlhog.hpp:168-174
+                const float* hist = s_hist + p * 2 * K * cells;
+                const double* fac4 = s_fac + p * cells * 4 + c * 4;
+                float* feat = s_feat + p * cells * dd;
+                const double ha = (double)hist[k * cells + c];
+                const double hb = (double)hist[(k + K) * cells + c];
+                double sa = 0.0, sb = 0.0, sc = 0.0;
+                double hcv[4];
 #pragma unroll
-        for (int f = 0; f < 4; ++f) {
-            const double fac = s_fac[c * 4 + f];
-            double haf = __dmul_rn(fac, ha);
-            double hbf = __dmul_rn(fac, hb);
-            double hcf = __dadd_rn(haf, hbf);
-            haf = (0.2 < haf) ? 0.2 : haf;
-            hbf = (0.2 < hbf) ? 0.2 : hbf;
-            hcf = (0.2 < hcf) ? 0.2 : hcf;
-            hcv[f] = hcf;
-            sa = (f == 0) ? haf : __dadd_rn(sa, haf);
-            sb = (f == 0) ? hbf : __dadd_rn(sb, hbf);
-            sc = (f == 0) ? hcf : __dadd_rn(sc, hcf);
-            s_hc[(c * K + k) * 4 + f] = hcf;
-        }
-        if (a.variant == 1) {                               // UoCTTI
-            s_feat[k * cells + oc] = (float)__dmul_rn(0.5, sa);
-            s_feat[(k + K) * cells + oc] = (float)__dmul_rn(0.5, sb);
-            s_feat[(k + 2 * K) * cells + oc] = (float)__dmul_rn(0.5, sc);
-        } else {                                            // Dalal-Triggs
+                for (int f = 0; f < 4; ++f) {
+                    const double fac = fac4[f];
+                    double haf = __dmul_rn(fac, ha);
+                    double hbf = __dmul_rn(fac, hb);
+                    double hcf = __dadd_rn(haf, hbf);
+                    haf = (0.2 < haf) ? 0.2 : haf;
+                    hbf = (0.2 < hbf) ? 0.2 : hbf;
+                    hcf = (0.2 < hcf) ? 0.2 : hcf;
+                    hcv[f] = hcf;
+                    sa = (f == 0) ? haf : __dadd_rn(sa, haf);
+                    sb = (f == 0) ? hbf : __dadd_rn(sb, hbf);
+                    sc = (f == 0) ? hcf : __dadd_rn(sc, hcf);
+                }
+                if (a.variant == 1) {                               // UoCTTI
+                    feat[k * cells + oc] = (float)__dmul_rn(0.5, sa);
+                    feat[(k + K) * cells + oc] = (float)__dmul_rn(0.5, sb);
+                    feat[(k + 2 * K) * cells + oc] = (float)__dmul_rn(0.5, sc);
+                } else {                                            // Dalal-Triggs
 #pragma unroll
-            for (int f = 0; f < 4; ++f) s_feat[(k + f * K) * cells + oc] = (float)hcv[f];
-        }
-    }
-    __syncthreads();
+                    for (int f = 0; f < 4; ++f) feat[(k + f * K) * cells + oc] = (float)hcv[f];
+                }
+            }
 
-    // ---- S7: texture dims = 1/sqrt(18) * sum_k hc_f, summed in ascending k (hog.c:1046-1053) -
-    if (a.variant == 1) {
-        for (int i = tid; i < cells * 4; i += kHogThreads) {
-            const int c = i >> 2, f = i & 3;
-            const int cj = c / nc, ci = c - cj * nc;
-            double t = 0.0;
-            for (int k = 0; k < K; ++k) t = __dadd_rn(t, s_hc[(c * K + k) * 4 + f]);
-            const float c18 = __fdiv_rn(1.0f, __fsqrt_rn(18.0f));
-            s_feat[(3 * K + f) * cells + ci * nc + cj] = (float)__dmul_rn((double)c18, t);
-        }
-        __syncthreads();
-    }
+            // ---- S7: texture dims = 1/sqrt(18) * sum_k hc_f, summed in ascending k (hog.c:1046-1053).  A thread recomputes the
+            //      clamped hc_f of its cell from hist and fac with S6's operations (same bits), so S7 needs no barrier after S6.
+            if (a.variant == 1) {
+                for (int i = tid; i < npair * cells * 4; i += kHogThreads) {
+                    const int p = i >= cells * 4 ? 1 : 0, ii = i - p * cells * 4;
+                    const int c = ii >> 2, f = ii & 3;
+                    const int cj = c / nc, ci = c - cj * nc;
+                    const float* hist = s_hist + p * 2 * K * cells;
+                    const double fac = s_fac[i];
+                    double t = 0.0;
+                    for (int k = 0; k < K; ++k) {
+                        const double hcf = __dadd_rn(__dmul_rn(fac, (double)hist[k * cells + c]), __dmul_rn(fac, (double)hist[(k + K) * cells + c]));
+                        t = __dadd_rn(t, (0.2 < hcf) ? 0.2 : hcf);
+                    }
+                    const float c18 = __fdiv_rn(1.0f, __fsqrt_rn(18.0f));
+                    s_feat[p * cells * dd + (3 * K + f) * cells + ci * nc + cj] = (float)__dmul_rn((double)c18, t);
+                }
+            }
+            __syncthreads();
 
-    // ---- S8: coalesced write of this landmark's slice of the feature row ---------------------
-    if (a.A) {
-        const int per_lm = cells * dd;
-        float* __restrict__ out = a.A + (long long)sample * a.ld + (long long)lm * per_lm;
-        for (int i = tid; i < per_lm; i += kHogThreads) out[i] = s_feat[i];
-        if (lm == 0 && tid == 0) a.A[(long long)sample * a.ld + (long long)a.L * per_lm] = 1.0f;   // bias, :182-183
+            // ---- S8: coalesced write of the pair's slices of the feature row (consecutive landmarks are adjacent) ----------
+            if (a.A) {
+                const int per_lm = cells * dd;
+                float* __restrict__ out = a.A + (long long)sample * a.ld + (long long)lm_first * per_lm;
+                for (int i = tid; i < npair * per_lm; i += kHogThreads) out[i] = s_feat[i];
+                if (lm_first == 0 && tid == 0) a.A[(long long)sample * a.ld + (long long)a.L * per_lm] = 1.0f;   // bias, :182-183
+            }
+        }
     }
 }
 
@@ -705,15 +742,6 @@ int launch_hog(sd_ctx* ctx, const sd_image_batch* images, const int32_t* d_image
         ctx->hog_lut[a.K] = lut;
     }
     a.lut = (const int8_t*)ctx->hog_lut[a.K];
-    if (!ctx->hog_lut[0]) {              // slot 0 (K >= 1 always): modulus table, shared by every K
-        const int n = 2 * 255 * 255 + 1;
-        void* lut = nullptr;
-        SD_CUDA(ctx, cudaMalloc(&lut, (size_t)n * sizeof(float)));
-        hog_maglut_kernel<<<sd_div_up(n, 256), 256, 0, ctx->stream>>>((float*)lut, n);
-        SD_LAUNCH_CHECK(ctx, "hog_maglut_kernel");
-        ctx->hog_lut[0] = lut;
-    }
-    a.mag_lut = (const float*)ctx->hog_lut[0];
 
     // per-sample tables (half size, cv::resize taps) and the per-launch spatial binning table
     const size_t geom_bytes = (size_t)N * sizeof(int) + (size_t)N * 5 * fs * sizeof(int) + (size_t)(a.nc * fs + 2 * a.nc) * sizeof(float);
@@ -753,10 +781,15 @@ int launch_hog(sd_ctx* ctx, const sd_image_batch* images, const int32_t* d_image
         }
     }
 
-    const HogSmem lay = hog_smem_layout(fs, a.nc, a.K, a.dd);
-    SD_REQUIRE(ctx, lay.total <= 227 * 1024, "HOG configuration needs more than 227 KB of shared memory");
-    const long long blocks = (long long)N * L;
-    SD_REQUIRE(ctx, blocks < 2147483647LL, "too many patches for one launch");
+    const HogSmem lay1 = hog_smem_layout(fs, a.nc, a.K, 1), lay2 = hog_smem_layout(fs, a.nc, a.K, 2);
+    SD_REQUIRE(ctx, lay1.total <= 227 * 1024, "HOG configuration needs more than 227 KB of shared memory");
+    SD_REQUIRE(ctx, (long long)N * L < 2147483647LL, "too many patches for one launch");
+    // A CTA walks the patches of kHogGroup consecutive landmarks of one sample and pays the per-sample work (image and ROI
+    // look-up, resize taps, binning weights, mbarrier set-up) once for all of them.  The landmarks of a sample are split
+    // into groups of equal size up to one.
+    a.groups = sd_div_up(L, kHogGroup);
+    a.gsz = sd_div_up(L, a.groups);
+    const long long blocks = (long long)N * a.groups;
     auto kern = hog_patch_kernel<0, 0, 0>;
     if (a.K == 4) kern = hog_patch_kernel<4, 0, 0>;
     else if (a.K == 9) kern = hog_patch_kernel<9, 0, 0>;
@@ -766,9 +799,20 @@ int launch_hog(sd_ctx* ctx, const sd_image_batch* images, const int32_t* d_image
         SD_HOG_PICK(9, 11) SD_HOG_PICK(9, 10) SD_HOG_PICK(9, 8) SD_HOG_PICK(9, 6)
 #undef SD_HOG_PICK
     }
+    // Pairs of patches share the tail unless the second slot costs resident CTAs (with K = 9 at cs = 10 it would take the
+    // kernel from five to four CTAs per SM).
+    a.pair = 0;
+    if (lay2.total <= 227 * 1024) {
+        int occ1 = 0, occ2 = 0;
+        SD_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, lay2.total));
+        SD_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ1, kern, kHogThreads, lay1.total));
+        SD_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ2, kern, kHogThreads, lay2.total));
+        a.pair = occ2 >= occ1 ? 1 : 0;
+    }
+    const HogSmem lay = a.pair ? lay2 : lay1;
     SD_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, lay.total));
     // (Measured, profiles/r02_summary.md: forcing six resident CTAs per SM with the whole shared-memory carve-out is SLOWER than
-    // five with the default split -- the orientation / modulus tables live in L1, which the larger carve-out takes away.)
+    // five with the default split -- the orientation table lives in L1, which the larger carve-out takes away.)
     kern<<<(unsigned)blocks, kHogThreads, lay.total, ctx->stream>>>(a, maps);
     SD_LAUNCH_CHECK(ctx, "hog_patch_kernel");
     return SD_OK;

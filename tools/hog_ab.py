@@ -1,12 +1,21 @@
 """Times the HOG launch of every cascade level and the whole device-resident detect step (development helper for comparing
-two builds of the library): python tools/hog_ab.py [batch]"""
+two builds of the library): python tools/hog_ab.py [batch] [--dump DIR]
+
+--dump DIR also writes each level's descriptors as DIR/hog_level<i>.npy, so that two builds can be compared bit for bit."""
 import ctypes as C, os, sys
 import numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import bench
 from superviseddescent_b200 import api as sd, _capi
-B = int(sys.argv[1]) if len(sys.argv) > 1 else 4096
+args = sys.argv[1:]
+DUMP = None
+if "--dump" in args:
+    i = args.index("--dump")
+    DUMP = args[i + 1]
+    del args[i:i + 2]
+    os.makedirs(DUMP, exist_ok=True)
+B = int(args[0]) if args else 4096
 dev = torch.device("cuda", 0)
 ctx = sd.Context(0)
 model = sd.load_detection_model(bench.MODEL, ctx)
@@ -31,6 +40,8 @@ for level in range(model.num_levels):
     for _ in range(10): hog()
     e1.record(); torch.cuda.synchronize()
     out.append(round(e0.elapsed_time(e1) / 10, 4))
+    if DUMP:
+        np.save(os.path.join(DUMP, f"hog_level{level}.npy"), A[:, :D].cpu().numpy())
 for _ in range(3): model.detect_batch_device(frames, x0)
 torch.cuda.synchronize(); e0.record()
 for _ in range(5): model.detect_batch_device(frames, x0)
